@@ -45,6 +45,8 @@ METRIC = "admm_inner_iter_per_s"
 UNIT = "inner ADMM iterations/s"
 SWEEP_RATES = (1.5, 2.0, 3.0, 4.0)
 SWEEP_BITS = (3, 4, 6, 8)
+DUMP_LIMIT_BYTES = 64 * 10**6     # --dump-outputs: all files of one run together
+DUMP_WHOLE_ELEMENTS = 4096        # arrays up to this size are never sampled
 
 
 def parse_args():
@@ -69,10 +71,15 @@ def parse_args():
     ap.add_argument("--concurrency", default="prop", choices=["off", "prop"],
                     help="off: layers run one after the other on every SM; prop: every layer gets a share of the SMs "
                          "proportional to its cost and all layers run concurrently on their own streams")
-    ap.add_argument("--min-ctas", type=int, default=2)
-    ap.add_argument("--balance", default="model", choices=["model", "prop"],
-                    help="re-balancing of the SM budgets during warm-up: 'model' = wave model of the tensor-core product "
-                         "fitted to the reported phase times (source/workloads.py), 'prop' = proportional to time x CTAs")
+    ap.add_argument("--min-ctas", type=int, default=2,
+                    help="--full, and the first warm-up step of --balance model / prop: SMs at least per unit")
+    ap.add_argument("--balance", default="cost", choices=["cost", "model", "prop"],
+                    help="SM budgets of the concurrent units: 'cost' (default) = proportional to the cost model and fixed, "
+                         "so that runs with the same arguments compute the same numbers; re-balanced during warm-up from "
+                         "measured times: 'model' = wave model of the tensor-core product fitted to the reported phase "
+                         "times (source/workloads.py), 'prop' = proportional to time x CTAs.  The loop kernel a factor runs "
+                         "on depends on its budget, so with measured budgets the results differ from run to run in the "
+                         "last bits, which the solver amplifies")
     ap.add_argument("--budgets", default=None,
                     help="experiment knob: comma-separated SM budgets, one per layer in workload order; fixes the budgets "
                          "(no re-balancing during warm-up; single GPU)")
@@ -93,6 +100,11 @@ def parse_args():
                          "factorize time (init + ADMM) instead of the per-sweep throughput")
     ap.add_argument("--init", default="random", choices=["random", "parafac-epc"], help="--full: factor initialisation")
     ap.add_argument("--max-iter-als", type=int, default=1000, help="--full: sweep budget per unit")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last step computed for every unit (factors, quantized "
+                         "factors, the two reconstruction errors) as DIR/<unit>.<array>.npy, so that two builds can be "
+                         f"compared output for output; above {DUMP_LIMIT_BYTES // 10**6} MB in all, every large array is "
+                         "replaced by the same seeded sample of its elements")
     return ap.parse_args()
 
 
@@ -373,6 +385,32 @@ def allocate_ctas(costs, sm_count, min_ctas):
     return out
 
 
+def dump_outputs(out_dir, units, world):
+    """Write what the last timed step computed for every unit of this rank - factors, quantized factors and the two
+    reconstruction errors - as out_dir/<unit>.<array>.npy (float32; the errors float64).  The ranks of a job share
+    DUMP_LIMIT_BYTES.  When a rank's arrays need more, every array of more than DUMP_WHOLE_ELEMENTS elements is replaced
+    by the same fraction of its elements, at positions drawn with a fixed seed, so that runs with the same arguments
+    sample the same positions.  units: [(key, factors, factors_q, rec_error, quant_rec_error)]."""
+    import numpy as np
+    arrays = {}
+    for key, factors, factors_q, err, errq in units:
+        name = key.replace("/", "_")
+        arrays[f"{name}.rec_error"] = np.array([err, errq], dtype=np.float64)
+        for m, (f, q) in enumerate(zip(factors, factors_q)):
+            arrays[f"{name}.factor{m}"] = f.float().cpu().numpy()
+            arrays[f"{name}.factor{m}_quantized"] = q.float().cpu().numpy()
+    room = DUMP_LIMIT_BYTES // world - 256 * len(arrays)     # 256 B per file covers the .npy header
+    whole = sum(a.nbytes for a in arrays.values() if a.size <= DUMP_WHOLE_ELEMENTS)
+    big = sum(a.nbytes for a in arrays.values()) - whole
+    keep = min(1.0, max(room - whole, 0) / big) if big else 1.0
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if keep < 1.0 and a.size > DUMP_WHOLE_ELEMENTS:
+            pos = np.random.default_rng(0).choice(a.size, int(a.size * keep), replace=False)
+            a = a.reshape(-1)[np.sort(pos)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------ native arm
 class Rank:
     """Process-group plumbing of one rank."""
@@ -467,8 +505,9 @@ def run_native(args):
         problems.append((key, W, rnk, wl.random_init(W.shape, rnk, init_seed), bits))
     host, solvers = [], []   # pinned host state for the end-to-end leg
     concurrent = args.concurrency == "prop" and len(problems) > 0
+    # fixed budgets give the small units one SM each, where the re-balancing from measured times always ends
     budgets = allocate_ctas([wl.solve_cost(W.shape, rnk) for _, W, rnk, _, _ in problems], sm_count - args.reserve_sms,
-                            args.min_ctas) if concurrent else [0] * len(problems)
+                            1 if args.balance == "cost" else args.min_ctas) if concurrent else [0] * len(problems)
     if args.budgets and concurrent and world == 1:
         budgets = [int(x) for x in args.budgets.split(",")]
         assert len(budgets) == len(problems) and sum(budgets) <= sm_count, (len(problems), sum(budgets), sm_count)
@@ -545,7 +584,7 @@ def run_native(args):
         w1.record()
         torch.cuda.synchronize()
         tried.append((w0.elapsed_time(w1), [s.max_ctas for s in solvers]))
-        if streams is not None and w < args.warmup - 1 and not args.budgets and len(solvers) > 1:
+        if streams is not None and w < args.warmup - 1 and args.balance != "cost" and not args.budgets and len(solvers) > 1:
             # re-balance the SM budgets from what was just measured: per unit the sweep time and, per factor, the
             # phase times its persistent kernel reported, through the wave model of source/workloads.py
             fitted = []
@@ -600,6 +639,9 @@ def run_native(args):
     total_ms = rk.reduce(sum(step_ms), "MAX")
     done_all = rk.reduce(done_total, "SUM")
     value = done_all / (total_ms / 1e3)
+    if args.dump_outputs and (rank == 0 or not args.seed_replicas):   # seed replicas: every rank has the same units
+        dump_outputs(args.dump_outputs, [(p[0], s.factors, s.factors_q, *e) for p, s, e in zip(problems, solvers, errs)],
+                     1 if args.seed_replicas else world)
 
     # ---- the dominant kernel (persistent ADMM loop), timed with CUDA events on its own stream.  In concurrent mode a
     # launch holds only its share g of the SMs, so its duration is weighted by g / SMs: the sum is the time the whole
@@ -760,7 +802,7 @@ def run_native(args):
                 "warmup": args.warmup, "ms_per_step": total_ms / args.steps, "higher_is_better": True,
                 "scaling": "weak" if args.seed_replicas else "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
                 "config": config_dict(args, desc, {"l2": "flushed between timed steps (256 MiB write)",
-                                                   "concurrency": args.concurrency,
+                                                   "concurrency": args.concurrency, "balance": args.balance,
                                                    "units_per_rank": [len(pr["units"]) for pr in per_rank],
                                                    "ctas_per_unit": {k: v for pr in per_rank for k, v in pr["ctas"].items()},
                                                    "parallelism": par,
@@ -840,6 +882,7 @@ def run_sweep256(args, rk, units, owner, mine, desc, sm_count):
             out = _native.factorize_batch(rd)
             for j, (hist, histq, n, fq) in zip(rd, out):
                 errs[j["key"]] = hist[-1]
+                j["last"] = (fq, hist[-1], histq[-1])
                 if e2e:
                     for dst, src in zip(j["host"]["factors"] + j["host"]["duals"] + j["host"]["factors_q"],
                                         j["factors"] + j["duals"] + fq):
@@ -873,6 +916,8 @@ def run_sweep256(args, rk, units, owner, mine, desc, sm_count):
     # layers leave early in later sweeps, so this is an upper bound of the executed iterations by a few per cent)
     inner_all = rk.reduce(inner_nominal * args.steps, "SUM")
     value = inner_all / (total_ms / 1e3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [(j["key"], j["factors"], *j["last"]) for j in jobs], world)
     e2e = None
     if not args.no_e2e:
         step(e2e=True)
@@ -1002,6 +1047,9 @@ def run_full(args, rk, units, owner, mine, desc, sm_count):
     wall = time.perf_counter() - t_job
     job_s = rk.reduce(wall, "MAX")
     inner_all = rk.reduce(inner, "SUM")
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [(p[0], s.factors, s.factors_q, s.loss_hist[-1], s.loss_quant_hist[-1])
+                                         for p, s in zip(problems, solvers)], world)
     gather_ms, _ = rk.gather_factors([f for s in solvers for f in s.factors])
     per_rank = rk.gather_objects({"init_s": {k: round(v, 3) for k, v in init_s.items()},
                                   "admm_s": {k: round(v, 3) for k, v in admm_s.items()}, "sweeps": sweeps,
@@ -1031,6 +1079,8 @@ def main():
     args = parse_args()
     if args.steps < 1 or args.warmup < 0:
         raise SystemExit("--steps >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        raise SystemExit("--dump-outputs: the reference arm times samples, not the workload's outputs")
     sys.exit(run_reference(args) if args.impl == "reference" else run_native(args))
 
 

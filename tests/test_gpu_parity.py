@@ -850,19 +850,18 @@ def test_factorize_cli_writes_the_reference_file_set(tmp_path, monkeypatch):
     with pytest.raises(SystemExit):
         fz.parse_args(["--model-name", "resnet18"])                       # required flags (:38-102)
     # the reference loads the PRETRAINED model: that is the default, and without network / cache it fails loudly instead
-    # of factorizing random weights under the reference's file names
+    # of factorizing random weights under the reference's file names.  The checkpoint fetch is replaced by one that
+    # fails the way it does offline, so the test neither reads the user's download cache nor reaches the network.
     base = ["--model-name", "resnet18", "--method", "admm", "--layer", "layer1.0.conv1", "--reduction-rate", "2", "--bits", "4",
             "--qscheme", MSE, "--seed", "42"]
     assert fz.parse_args(base).weights == "pretrained"
-    try:
-        import torchvision
-        torchvision.models.resnet18(weights="DEFAULT")
-        have_checkpoint = True
-    except Exception:  # noqa: BLE001
-        have_checkpoint = False
-    if not have_checkpoint:
-        with pytest.raises(RuntimeError, match="pretrained"):
-            fz.main(base + ["--max_iter_als", "1", "--max_iter_admm", "5"])
+    import torchvision.models._api
+
+    def offline(url, *_a, **_k):
+        raise OSError(f"no network and no cached checkpoint for {url}")
+    monkeypatch.setattr(torchvision.models._api, "load_state_dict_from_url", offline)
+    with pytest.raises(RuntimeError, match="pretrained"):
+        fz.main(base + ["--max_iter_als", "1", "--max_iter_admm", "5"])
     acc = load("calibrate").main(["--bits", "4", "--qscheme", MSE, "--seed", "42", "--layers", "layer1.0.conv1",
                                   "--eval-batches", "2", "--batch-size", "16", "--calibration-samples", "32"])
     assert 0.0 <= acc <= 100.0

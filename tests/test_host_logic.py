@@ -118,6 +118,42 @@ def test_cli_argument_contract():
     assert fz.run_name(fz.parse_args(base + ["--rank", "134"])) == "admm_l=layer1.0.conv1_r=134_b=4_s=42_i=random_tensor_mseminmax_symmetric"
 
 
+def test_bench_output_dump_whole_under_the_limit_and_a_fixed_sample_above(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: every array of every unit is written whole while they fit the size limit; above it each
+    large array is replaced by a sample at the same seeded positions in every run, and the files stay within the limit."""
+    import importlib.util
+    # bench.py sets this at import for the processes it runs; keep it out of the test process
+    monkeypatch.setenv("CUDA_DEVICE_MAX_CONNECTIONS", os.environ.get("CUDA_DEVICE_MAX_CONNECTIONS", "32"))
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(REPO, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    g = torch.Generator().manual_seed(0)
+    fac = [torch.randn(d, 40, generator=g) for d in (300, 200, 9)]
+    units = [("layer1.0.conv1/rr2.0/b4", fac, [f.round() for f in fac], 0.5, 0.25)]
+    name = "layer1.0.conv1_rr2.0_b4"
+    bench.dump_outputs(str(tmp_path / "whole"), units, 1)
+    whole = {p.name: np.load(p) for p in (tmp_path / "whole").iterdir()}
+    assert sorted(whole) == sorted([f"{name}.rec_error.npy"] + [f"{name}.factor{m}{q}.npy" for m in range(3)
+                                                                for q in ("", "_quantized")])
+    assert whole[f"{name}.rec_error.npy"].dtype == np.float64 and whole[f"{name}.rec_error.npy"].tolist() == [0.5, 0.25]
+    for m in range(3):
+        assert whole[f"{name}.factor{m}.npy"].dtype == np.float32
+        assert np.array_equal(whole[f"{name}.factor{m}.npy"], fac[m].numpy())
+        assert np.array_equal(whole[f"{name}.factor{m}_quantized.npy"], fac[m].round().numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 100_000)
+    runs = []
+    for k in range(2):
+        d = tmp_path / f"sampled{k}"
+        bench.dump_outputs(str(d), units, 1)
+        assert sum(p.stat().st_size for p in d.iterdir()) <= 100_000
+        runs.append({p.name: np.load(p) for p in d.iterdir()})
+    assert sorted(runs[0]) == sorted(whole) and sorted(runs[1]) == sorted(whole)
+    sample = runs[0][f"{name}.factor0.npy"]
+    assert 0 < sample.size < fac[0].numel() and np.isin(sample, fac[0].numpy()).all()
+    assert np.array_equal(runs[0][f"{name}.factor2.npy"], fac[2].numpy())     # small arrays stay whole
+    assert all(np.array_equal(runs[0][n], runs[1][n]) for n in runs[0])
+
+
 def _gather_worker(rank, world, port, out):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
     sys.path[:0] = [REPO, PKG]

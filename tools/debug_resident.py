@@ -1,5 +1,6 @@
-import sys
-sys.path[:0]=['/root/repo','/root/repo/admm-quantization_b200']
+import os, sys
+REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path[:0] = [REPO, os.path.join(REPO, "admm-quantization_b200")]
 import torch
 from oracle import admm_oracle as orc
 from source import _native as nat
