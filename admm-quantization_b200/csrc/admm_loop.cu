@@ -1051,16 +1051,60 @@ static int check_loop_args(const char* who, const void* H, const void* U, const 
   return ADMMQ_OK;
 }
 
+// The loop kernel of a call: one decision for launch_loop and admmq_admm_loop_kernel (include/admmq.h lists the ids).
+static int select_loop_kernel(int I, int R, int num_attempts, int precision, int grid) {
+  const int Rp = (R + 3) / 4 * 4;
+  static const bool no_resident = getenv("ADMMQ_NO_RESIDENT") != nullptr;  // diagnostics: force the general kernel
+  static const bool no_cluster = getenv("ADMMQ_NO_CLUSTER") != nullptr;    // diagnostics: never take the cluster kernel
+  static const bool no_tap = getenv("ADMMQ_NO_TAP") != nullptr;            // diagnostics: never take the tap-factor cluster kernel
+  const int ccl = (precision != 0 && !no_resident && !no_cluster && grid >= 4) ? cluster_ctas_for(I, R, Rp, num_attempts, grid) : 0;
+  if ((grid == 1 || ccl >= 4) && precision != 0 && !no_resident && resident_fits(I, R, Rp, num_attempts)) {
+    // a small factor: the shared-memory-resident loop on one CTA (admm_loop_resident.cuh) or, with a budget of at
+    // least four CTAs, on a thread-block cluster that splits rows and clip candidates (admm_loop_cluster.cuh)
+    if (ccl == 8) return ADMMQ_LOOP_CLUSTER8;
+    if (ccl == 4) return ADMMQ_LOOP_CLUSTER4;
+    return ADMMQ_LOOP_RESIDENT;
+  }
+  // the tap factor of a wide convolution (9 x R): one cluster of 8 CTAs, columns and clip candidates split (admm_loop_tap.cuh)
+  if (precision != 0 && !no_tap && !no_cluster && tap_cluster_fits(I, R, Rp, num_attempts, grid)) return ADMMQ_LOOP_TAP;
+  if (precision == 0)  // parity mode: float64-accumulating tiles against the float64 inverse
+    return pick_tile(I, R, grid) == 0 ? ADMMQ_LOOP_F64_64 : ADMMQ_LOOP_F64_32;
+  if (I <= 16 && (long long)I * Rp <= SkinnySmem<16>::kRhsFloats) return I <= 9 ? ADMMQ_LOOP_SKINNY9 : ADMMQ_LOOP_SKINNY16;
+  // tensor-core P1 only pays off when the factor has enough rows to fill a good part of a 128-row tile
+  if (precision == 1 && I >= 64 && R >= 32) {
+    const int tilesM = (I + tc::kTileM - 1) / tc::kTileM;
+    // tile width (multiple of 16): a tile costs a fixed part (fill, drain, epilogue set-up) plus bn columns of
+    // tensor-core work; minimise waves * (kTileFixed + bn), ties go to the wider tile.  Widths above 128 (one
+    // accumulator, shallower raw ring: ~5 % dearer per column) exist for the wave structure: 4 x 8 tiles of width 144
+    // cover 512 x 1141 in ONE wave on 32 .. 35 CTAs where 4 x 9 of width 128 need two
+    int tcbn = kLoopPS ? 128 : 64;
+    long long best = -1;
+    for (int bn = (kLoopPS ? 160 : 64); bn >= 16; bn -= 16) {
+      const long long tiles = (long long)tilesM * ((R + bn - 1) / bn);
+      const long long cost = ((tiles + grid - 1) / grid) * (kTileFixed + bn) * (bn > 128 ? 105 : 100);
+      if (best < 0 || cost < best) {
+        best = cost;
+        tcbn = bn;
+      }
+    }
+    static const int force_bn = getenv("ADMMQ_LOOP_BN") ? atoi(getenv("ADMMQ_LOOP_BN")) : 0;   // experiment knob
+    if (force_bn >= 16 && force_bn <= (kLoopPS ? 160 : 64) && (force_bn & 15) == 0) tcbn = force_bn;
+    return ADMMQ_LOOP_TC + tcbn;
+  }
+  switch (pick_tile(I, R, grid)) {
+    case 0: return ADMMQ_LOOP_FFMA64;
+    case 1: return ADMMQ_LOOP_FFMA32;
+    default: return ADMMQ_LOOP_FFMA16;
+  }
+}
+
 static int launch_loop(float* H, float* U, const float* F, const float* Minv, const double* Minv64, const float* rho,
                        const int* inv_status, int I, int R, int max_iter, float eps, int bits, int qscheme, int num_attempts, int precision,
                        int8_t* codes, admmq_loop_report* report, char* ws, int grid, cudaStream_t stream) {
   const LoopLayout l = loop_layout(I, R, grid);
-  static const bool no_resident = getenv("ADMMQ_NO_RESIDENT") != nullptr;  // diagnostics: force the general kernel
-  static const bool no_cluster = getenv("ADMMQ_NO_CLUSTER") != nullptr;    // diagnostics: never take the cluster kernel
-  const int ccl = (precision != 0 && !no_resident && !no_cluster && grid >= 4) ? cluster_ctas_for(I, R, l.Rp, num_attempts, grid) : 0;
-  if ((grid == 1 || ccl >= 4) && precision != 0 && !no_resident && resident_fits(I, R, l.Rp, num_attempts)) {
-    // a small factor: the shared-memory-resident loop on one CTA (admm_loop_resident.cuh) or, with a budget of at
-    // least two CTAs, on a thread-block cluster that splits rows and clip candidates (admm_loop_cluster.cuh)
+  const int kid = select_loop_kernel(I, R, num_attempts, precision, grid);
+  if (kid == ADMMQ_LOOP_RESIDENT || kid == ADMMQ_LOOP_CLUSTER4 || kid == ADMMQ_LOOP_CLUSTER8) {
+    const int ccl = kid == ADMMQ_LOOP_CLUSTER8 ? 8 : kid == ADMMQ_LOOP_CLUSTER4 ? 4 : 0;
     ResidentParams rp;
     rp.H = H;
     rp.U = U;
@@ -1103,9 +1147,7 @@ static int launch_loop(float* H, float* U, const float* F, const float* Minv, co
     count_launches(1);
     return ADMMQ_OK;
   }
-  static const bool no_tap = getenv("ADMMQ_NO_TAP") != nullptr;   // diagnostics: never take the tap-factor cluster kernel
-  if (precision != 0 && !no_tap && !no_cluster && tap_cluster_fits(I, R, l.Rp, num_attempts, grid)) {
-    // the tap factor of a wide convolution (9 x R): one cluster of 8 CTAs, columns and clip candidates split (admm_loop_tap.cuh)
+  if (kid == ADMMQ_LOOP_TAP) {
     ResidentParams rp;
     rp.H = H;
     rp.U = U;
@@ -1178,79 +1220,41 @@ static int launch_loop(float* H, float* U, const float* F, const float* Minv, co
   void* args[] = {&p};
   const void* fn = nullptr;
   size_t smem = 0;
-  // tensor-core P1 only pays off when the factor has enough rows to fill a good part of a 128-row tile
-  const bool use_tc = precision == 1 && I >= 64 && R >= 32;
-  const bool use_skinny = precision != 0 && I <= 16 && (long long)I * l.Rp <= SkinnySmem<16>::kRhsFloats;
-  if (precision == 0) {  // parity mode: float64-accumulating tiles against the float64 inverse
+  if (kid < ADMMQ_LOOP_TC) {
     memset(&p.tm_rhs, 0, sizeof(CUtensorMap));
     memset(&p.tm_minv_hi, 0, sizeof(CUtensorMap));
     memset(&p.tm_minv_lo, 0, sizeof(CUtensorMap));
-    if (pick_tile(I, R, grid) == 0) {
-      fn = (const void*)k_admm_loop<64, 64, 4, 4, kF64P1>;
-      smem = sizeof(LoopSmem<64, 64, kF64P1>);
-    } else {
-      fn = (const void*)k_admm_loop<32, 32, 2, 2, kF64P1>;
-      smem = sizeof(LoopSmem<32, 32, kF64P1>);
-    }
-  } else if (use_skinny) {
-    memset(&p.tm_rhs, 0, sizeof(CUtensorMap));
-    memset(&p.tm_minv_hi, 0, sizeof(CUtensorMap));
-    memset(&p.tm_minv_lo, 0, sizeof(CUtensorMap));
-    if (I <= 9) {
-      fn = (const void*)k_admm_loop<16, 32, 1, 2, -9>;
-      smem = sizeof(LoopSmem<16, 32, -9>);
-    } else {
-      fn = (const void*)k_admm_loop<16, 32, 1, 2, -16>;
-      smem = sizeof(LoopSmem<16, 32, -16>);
-    }
-  } else if (use_tc) {
-    const int tilesM = (I + tc::kTileM - 1) / tc::kTileM;
-    // tile width (multiple of 16): a tile costs a fixed part (fill, drain, epilogue set-up) plus bn columns of
-    // tensor-core work; minimise waves * (kTileFixed + bn), ties go to the wider tile
-    int tcbn = kLoopPS ? 128 : 64;
-    {
-      // widths above 128 (one accumulator, shallower raw ring: ~5 % dearer per column) exist for the wave structure:
-      // 4 x 8 tiles of width 144 cover 512 x 1141 in ONE wave on 32 .. 35 CTAs where 4 x 9 of width 128 need two
-      long long best = -1;
-      for (int bn = (kLoopPS ? 160 : 64); bn >= 16; bn -= 16) {
-        const long long tiles = (long long)tilesM * ((R + bn - 1) / bn);
-        const long long cost = ((tiles + grid - 1) / grid) * (kTileFixed + bn) * (bn > 128 ? 105 : 100);
-        if (best < 0 || cost < best) {
-          best = cost;
-          tcbn = bn;
-        }
+  }
+  switch (kid) {
+    case ADMMQ_LOOP_F64_64: fn = (const void*)k_admm_loop<64, 64, 4, 4, kF64P1>; smem = sizeof(LoopSmem<64, 64, kF64P1>); break;
+    case ADMMQ_LOOP_F64_32: fn = (const void*)k_admm_loop<32, 32, 2, 2, kF64P1>; smem = sizeof(LoopSmem<32, 32, kF64P1>); break;
+    case ADMMQ_LOOP_SKINNY9: fn = (const void*)k_admm_loop<16, 32, 1, 2, -9>; smem = sizeof(LoopSmem<16, 32, -9>); break;
+    case ADMMQ_LOOP_SKINNY16: fn = (const void*)k_admm_loop<16, 32, 1, 2, -16>; smem = sizeof(LoopSmem<16, 32, -16>); break;
+    case ADMMQ_LOOP_FFMA64: fn = (const void*)k_admm_loop<64, 64, 4, 4, 0>; smem = sizeof(LoopSmem<64, 64, 0>); break;
+    case ADMMQ_LOOP_FFMA32: fn = (const void*)k_admm_loop<32, 32, 2, 2, 0>; smem = sizeof(LoopSmem<32, 32, 0>); break;
+    case ADMMQ_LOOP_FFMA16: fn = (const void*)k_admm_loop<16, 32, 1, 2, 0>; smem = sizeof(LoopSmem<16, 32, 0>); break;
+    default: {  // ADMMQ_LOOP_TC + tile width
+      const int tcbn = kid - ADMMQ_LOOP_TC;
+      p.tc_bn = tcbn;
+      if (int e = tc::make_operand_tmap(&p.tm_rhs, p.RHS, I, R, l.Rp, tc::kTileM)) return e;
+      if (int e = tc::make_operand_tmap(&p.tm_minv_hi, kLoopPS ? p.MinvHi : Minv, R, R, l.Rp, tcbn)) return e;
+      if (int e = tc::make_operand_tmap(&p.tm_minv_lo, kLoopPS ? p.MinvLo : Minv, R, R, l.Rp, tcbn)) return e;
+      if (tcbn > 128) {
+        fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 160 : 64)>;
+        smem = sizeof(LoopSmem<16, 32, (kLoopPS ? 160 : 64)>);
+      } else if (tcbn > 64) {
+        fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 128 : 64)>;
+        smem = sizeof(LoopSmem<16, 32, (kLoopPS ? 128 : 64)>);
+      } else if (tcbn > 32) {
+        fn = (const void*)k_admm_loop<16, 32, 1, 2, 64>;
+        smem = sizeof(LoopSmem<16, 32, 64>);
+      } else if (tcbn > 16) {
+        fn = (const void*)k_admm_loop<16, 32, 1, 2, 32>;
+        smem = sizeof(LoopSmem<16, 32, 32>);
+      } else {
+        fn = (const void*)k_admm_loop<16, 32, 1, 2, 16>;
+        smem = sizeof(LoopSmem<16, 32, 16>);
       }
-      static const int force_bn = getenv("ADMMQ_LOOP_BN") ? atoi(getenv("ADMMQ_LOOP_BN")) : 0;   // experiment knob
-      if (force_bn >= 16 && force_bn <= (kLoopPS ? 160 : 64) && (force_bn & 15) == 0) tcbn = force_bn;
-    }
-    p.tc_bn = tcbn;
-    if (int e = tc::make_operand_tmap(&p.tm_rhs, p.RHS, I, R, l.Rp, tc::kTileM)) return e;
-    if (int e = tc::make_operand_tmap(&p.tm_minv_hi, kLoopPS ? p.MinvHi : Minv, R, R, l.Rp, tcbn)) return e;
-    if (int e = tc::make_operand_tmap(&p.tm_minv_lo, kLoopPS ? p.MinvLo : Minv, R, R, l.Rp, tcbn)) return e;
-    if (tcbn > 128) {
-      fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 160 : 64)>;
-      smem = sizeof(LoopSmem<16, 32, (kLoopPS ? 160 : 64)>);
-    } else if (tcbn > 64) {
-      fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 128 : 64)>;
-      smem = sizeof(LoopSmem<16, 32, (kLoopPS ? 128 : 64)>);
-    } else if (tcbn > 32) {
-      fn = (const void*)k_admm_loop<16, 32, 1, 2, 64>;
-      smem = sizeof(LoopSmem<16, 32, 64>);
-    } else if (tcbn > 16) {
-      fn = (const void*)k_admm_loop<16, 32, 1, 2, 32>;
-      smem = sizeof(LoopSmem<16, 32, 32>);
-    } else {
-      fn = (const void*)k_admm_loop<16, 32, 1, 2, 16>;
-      smem = sizeof(LoopSmem<16, 32, 16>);
-    }
-  } else {
-    memset(&p.tm_rhs, 0, sizeof(CUtensorMap));
-    memset(&p.tm_minv_hi, 0, sizeof(CUtensorMap));
-    memset(&p.tm_minv_lo, 0, sizeof(CUtensorMap));
-    switch (pick_tile(I, R, grid)) {
-      case 0: fn = (const void*)k_admm_loop<64, 64, 4, 4, 0>; smem = sizeof(LoopSmem<64, 64, 0>); break;
-      case 1: fn = (const void*)k_admm_loop<32, 32, 2, 2, 0>; smem = sizeof(LoopSmem<32, 32, 0>); break;
-      default: fn = (const void*)k_admm_loop<16, 32, 1, 2, 0>; smem = sizeof(LoopSmem<16, 32, 0>); break;
     }
   }
   ADMMQ_CUDA_OK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1286,6 +1290,12 @@ extern "C" int admmq_spd_inverse(const float* G, int R, float* Minv, double* Min
   double* Lw = (double*)(ws + 256);
   double* Xw = (double*)(ws + 256 + spd_scratch_bytes(R) / 2);
   return launch_spd_inverse(G, R, Minv, Minv64, admmq_padded_ld(R), rho_out, status, (unsigned int*)ws, Lw, Xw, coop_grid(dp, max_ctas), stream);
+}
+
+extern "C" int admmq_admm_loop_kernel(int I, int R, int num_attempts, int precision, int grid) {
+  if (I <= 0 || R <= 0 || grid <= 0 || precision < 0 || precision > 2)
+    return fail(ADMMQ_E_BADARG, "admmq_admm_loop_kernel: bad argument");
+  return select_loop_kernel(I, R, num_attempts, precision, grid);
 }
 
 extern "C" size_t admmq_admm_loop_workspace_bytes(int I, int R, int num_attempts) {

@@ -73,6 +73,7 @@ def _load():
         "admmq_padded_ld": (c_int, [c_int]),
         "admmq_spd_inverse_workspace_bytes": (c_sz, [c_int]),
         "admmq_spd_inverse": (c_int, [vp, c_int, vp, vp, vp, vp, c_int, vp, c_sz, vp]),
+        "admmq_admm_loop_kernel": (c_int, [c_int, c_int, c_int, c_int, c_int]),
         "admmq_admm_loop_workspace_bytes": (c_sz, [c_int, c_int, c_int]),
         "admmq_admm_loop": (c_int, [vp, vp, vp, vp, vp, vp, vp, c_int, c_int, c_int, c_f, c_int, c_int, c_int, c_int, c_int,
                                     vp, vp, vp, c_sz, vp]),
@@ -97,7 +98,7 @@ def _load():
 
 lib = _load()
 EXPORTS = ("admmq_version admmq_last_error admmq_device_info admmq_launch_count admmq_project_workspace_bytes "
-           "admmq_project admmq_clip_search_sums admmq_admm_loop_workspace_bytes admmq_admm_loop admmq_gemm_nt "
+           "admmq_project admmq_clip_search_sums admmq_admm_loop_kernel admmq_admm_loop_workspace_bytes admmq_admm_loop admmq_gemm_nt "
            "admmq_gram_hadamard admmq_unfold3 admmq_mttkrp_workspace_bytes admmq_mttkrp admmq_permute_myx "
            "admmq_mttkrp_tc_workspace_bytes admmq_mttkrp_tc admmq_mttkrp_f64_workspace_bytes admmq_mttkrp_f64 "
            "admmq_gram_hadamard_f64 admmq_normalize_columns_f64 "
@@ -428,6 +429,13 @@ def admm_iteration_inplace(H, U, F, G, max_iter, eps, bits, qscheme, num_attempt
                                    qscheme_id(qscheme), int(num_attempts), int(precision), int(max_ctas), ptr(codes),
                                    ptr(report), ptr(ws), ws.numel(), stream_ptr(H.device))
     return report
+
+
+def loop_kernel(I, R, num_attempts, precision, grid):
+    """Id of the loop kernel (include/admmq.h ADMMQ_LOOP_*) a call on a cooperative grid of `grid` CTAs runs."""
+    rc = int(lib.admmq_admm_loop_kernel(int(I), int(R), int(num_attempts), int(precision), int(grid)))
+    check(min(rc, 0))
+    return rc
 
 
 def admm_loop_workspace_bytes(I, R, num_attempts=200):

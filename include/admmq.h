@@ -198,6 +198,22 @@ typedef struct admmq_loop_report {
  *   Minv  R x admmq_padded_ld(R) float32, rho / inv_status device scalars written by admmq_spd_inverse
  *         (inv_status may be NULL; a non-zero value makes the loop return it in report->status untouched).
  *   Minv64  the float64 inverse (same shape) - required for precision 0, NULL otherwise. */
+/* The kernel a loop call with this factor shape, precision and grid size runs (grid = the cooperative grid: max_ctas,
+ * or the SM count when max_ctas is 0 or larger).  Pure host logic: needs no device, honours the ADMMQ_NO_RESIDENT /
+ * ADMMQ_NO_CLUSTER / ADMMQ_NO_TAP switches and ADMMQ_LOOP_BN.  Returns one of the ids below, or ADMMQ_E_BADARG. */
+#define ADMMQ_LOOP_RESIDENT 1  /* one CTA, the whole loop state in shared memory (admm_loop_resident.cuh) */
+#define ADMMQ_LOOP_CLUSTER4 2  /* thread-block cluster of 4 CTAs, rows split (admm_loop_cluster.cuh) */
+#define ADMMQ_LOOP_CLUSTER8 3  /* the same on 8 CTAs */
+#define ADMMQ_LOOP_TAP 4       /* cluster of 8 CTAs for <= 9 rows, columns split (admm_loop_tap.cuh) */
+#define ADMMQ_LOOP_SKINNY9 5   /* cooperative grid, column strips for <= 9 rows */
+#define ADMMQ_LOOP_SKINNY16 6  /* cooperative grid, column strips for 10 .. 16 rows */
+#define ADMMQ_LOOP_FFMA64 7    /* cooperative grid, float32 FFMA tiles of 64 x 64 */
+#define ADMMQ_LOOP_FFMA32 8    /* ... of 32 x 32 */
+#define ADMMQ_LOOP_FFMA16 9    /* ... of 16 x 32 */
+#define ADMMQ_LOOP_F64_64 10   /* cooperative grid, float64 parity tiles (precision 0) of 64 x 64 */
+#define ADMMQ_LOOP_F64_32 11   /* ... of 32 x 32 */
+#define ADMMQ_LOOP_TC 1000     /* + tile width (16 .. 160, multiple of 16): cooperative grid, 3xTF32 tcgen05 product */
+ADMMQ_API int admmq_admm_loop_kernel(int I, int R, int num_attempts, int precision, int grid);
 ADMMQ_API size_t admmq_admm_loop_workspace_bytes(int I, int R, int num_attempts);
 ADMMQ_API int admmq_admm_loop(float* H, float* U, const float* F, const float* Minv, const double* Minv64,
                     const float* rho, const int* inv_status, int I, int R, int max_iter, float eps, int bits, int qscheme,
