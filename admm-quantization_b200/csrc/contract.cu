@@ -263,13 +263,7 @@ __global__ void __launch_bounds__(kCT) k_sum_pairs(const double* __restrict__ ct
   }
 }
 
-static int mttkrp_splits(int M, long long P, int R, int bm, int sms) {
-  const long long tiles = (long long)((M + bm - 1) / bm) * ((R + 63) / 64);
-  long long want = (2LL * sms + tiles - 1) / tiles;            // aim for ~2 waves
-  const long long max_by_depth = std::max<long long>(1, P / 256);  // keep >= 256 deep slices
-  want = std::max<long long>(1, std::min(want, max_by_depth));
-  return (int)std::min<long long>(want, 64);
-}
+int select_mttkrp_kernel(int M, int nx, int ny, int R, int precision, int sms, int* grid, int* splits);  // tc_gemm.cu
 
 template <typename TI, typename TO>
 static int launch_mttkrp_f64(const TI* Wn, int M, const TI* X, int nx, const TI* Y, int ny, int R, TO* F, void* workspace,
@@ -277,12 +271,11 @@ static int launch_mttkrp_f64(const TI* Wn, int M, const TI* X, int nx, const TI*
   DeviceProps dp;
   if (int e = device_props(&dp)) return e;
   const long long P = (long long)nx * ny;
-  const int bm = (M <= 16) ? 16 : 64;
-  int splits = mttkrp_splits(M, P, R, bm, dp.sm_count);
+  int splits;
+  const int bm = select_mttkrp_kernel(M, nx, ny, R, 0, dp.sm_count, nullptr, &splits) == ADMMQ_MTTKRP_F64_16 ? 16 : 64;
+  // without room for the partials (admmq_mttkrp_workspace_bytes) the sum over p runs in one slice
   if (splits > 1 && (workspace == nullptr || workspace_bytes < (size_t)splits * M * R * sizeof(double))) splits = 1;
-  long long per = (P + splits - 1) / splits;
-  per = (per + kBK - 1) / kBK * kBK;
-  splits = (int)((P + per - 1) / per);
+  const long long per = ((P + splits - 1) / splits + kBK - 1) / kBK * kBK;
   dim3 grid((R + 63) / 64, (M + bm - 1) / bm, splits);
   if (bm == 16) k_mttkrp_f64<16, TI, TO><<<grid, kCT, 0, stream>>>(Wn, M, P, X, Y, ny, R, per, (double*)workspace, F);
   else k_mttkrp_f64<64, TI, TO><<<grid, kCT, 0, stream>>>(Wn, M, P, X, Y, ny, R, per, (double*)workspace, F);
@@ -363,8 +356,8 @@ extern "C" size_t admmq_mttkrp_workspace_bytes(int M, int nx, int ny, int R, int
   if (precision == 1) return mttkrp_tc_workspace_bytes(M, nx, ny, R);
   DeviceProps dp;
   const int sms = (device_props(&dp) == ADMMQ_OK) ? dp.sm_count : 148;
-  const int bm = (M <= 16) ? 16 : 64;
-  const int splits = mttkrp_splits(M, (long long)nx * std::max(ny, 1), R, bm, sms);
+  int splits;
+  select_mttkrp_kernel(M, nx, std::max(ny, 1), R, 0, sms, nullptr, &splits);
   return align_up((size_t)splits * M * R * sizeof(double), 256);  // split-K partials
 }
 

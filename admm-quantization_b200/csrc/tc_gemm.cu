@@ -200,6 +200,85 @@ __global__ void __launch_bounds__(256) k_fold_partials(const double* __restrict_
   }
 }
 
+// ---------------------------------------------------------------------------- launch choices
+// Tile widths come from a wave model: a tile costs a fixed part plus bn columns of tensor-core work, and the width
+// minimises waves * (fixed + bn); ties go to the wider tile (the candidates are tried widest first).
+static long long wave_cost(long long tilesM, int N, int w, int sms, int fixed) {
+  const long long tiles = tilesM * ((N + w - 1) / w);
+  return ((tiles + sms - 1) / sms) * (fixed + w);
+}
+
+// gemm_nt: measured 3.3 + 0.225 bn us at K = 1141, i.e. a fixed part of 16 columns; 128-wide tiles need the pre-split
+// B operand
+static int gemm_tile_width(int M, int N, int sms, bool presplit) {
+  const long long tilesM = (M + tc::kTileM - 1) / tc::kTileM;
+  int bn = 16;
+  long long best = -1;
+  for (const int w : {128, 64, 32, 16}) {
+    if (w == 128 && !presplit) continue;
+    const long long cost = wave_cost(tilesM, N, w, sms, 16);
+    if (best < 0 || cost < best) {
+      best = cost;
+      bn = w;
+    }
+  }
+  return bn;
+}
+
+// The float64 MTTKRP splits its sum over p into slices of at least 256 (aim: ~2 waves of tiles, at most 64 slices);
+// a slice is a whole number of 16-deep slabs, so rounding can leave fewer slices than asked for
+static int mttkrp_f64_splits(int M, long long P, int R, int bm, int sms) {
+  const long long tiles = (long long)((M + bm - 1) / bm) * ((R + 63) / 64);
+  long long want = (2LL * sms + tiles - 1) / tiles;
+  const long long max_by_depth = std::max<long long>(1, P / 256);
+  want = std::min<long long>(std::max<long long>(1, std::min(want, max_by_depth)), 64);
+  const long long per = ((P + want - 1) / want + 15) / 16 * 16;
+  return (int)((P + per - 1) / per);
+}
+
+// The kernel an MTTKRP call runs: one decision for the launchers (launch_mttkrp_f64, mttkrp_fold_gemm,
+// mttkrp_foldlong_gemm, and gemm_nt through gemm_tile_width) and admmq_mttkrp_kernel.  precision 1 is the
+// permuted-operand call admmq_mttkrp_tc.  grid: CTAs of the contraction kernel; splits: slices of the float64 sum
+// (1 on the tensor cores).  Honours ADMMQ_FOLD_BN.
+int select_mttkrp_kernel(int M, int nx, int ny, int R, int precision, int sms, int* grid, int* splits) {
+  int kid, g, s = 1;
+  if (precision == 0) {
+    const int bm = (M <= 16) ? 16 : 64;
+    s = mttkrp_f64_splits(M, (long long)nx * ny, R, bm, sms);
+    g = ((R + 63) / 64) * ((M + bm - 1) / bm) * s;
+    kid = bm == 16 ? ADMMQ_MTTKRP_F64_16 : ADMMQ_MTTKRP_F64_64;
+  } else if (ny == 1) {  // matrix: F = W . X
+    const int bn = gemm_tile_width(M, R, sms, true);
+    g = (int)std::min<long long>((long long)((M + tc::kTileM - 1) / tc::kTileM) * ((R + bn - 1) / bn), sms);
+    kid = ADMMQ_MTTKRP_GEMM + bn;
+  } else {
+    // fold: a tile takes mg = 128 / ny whole m, any multiple of 16 up to 128 wide; long fold (ny > 128): 128-row tiles,
+    // 80 .. 128 wide (one thread per column of a 128-wide staging tile).  The fixed part of a tile (pipeline fill,
+    // epilogue, fold) is worth ~40 columns at K = 512.
+    const bool longf = ny > tc::kTileM;
+    const long long tilesM = longf ? ((long long)M * ny + tc::kTileM - 1) / tc::kTileM
+                                   : (M + tc::kTileM / ny - 1) / (tc::kTileM / ny);
+    int bn = 128;
+    long long best = -1;
+    for (int w = 128; w >= (longf ? 80 : 16); w -= 16) {
+      const long long cost = wave_cost(tilesM, R, w, sms, 40);
+      if (best < 0 || cost < best) {
+        best = cost;
+        bn = w;
+      }
+    }
+    if (const char* force = longf ? nullptr : getenv("ADMMQ_FOLD_BN")) {  // experiment knob, read per call
+      const int w = atoi(force);
+      if (w >= 16 && w <= 128 && (w & 15) == 0) bn = w;
+    }
+    g = (int)std::min<long long>(tilesM * ((R + bn - 1) / bn), sms);
+    kid = (longf ? ADMMQ_MTTKRP_FOLDLONG : ADMMQ_MTTKRP_FOLD) + bn;
+  }
+  if (grid != nullptr) *grid = g;
+  if (splits != nullptr) *splits = s;
+  return kid;
+}
+
 template <int BN, bool PS>
 static int launch_gemm(const GemmMaps& maps, int M, int N, int K, float* C, int ldc, int grid, cudaStream_t stream) {
   const int smem = tc::TileSmem<BN, PS>::kBytes;
@@ -220,21 +299,7 @@ int gemm_nt(const float* A, int lda, int M, const float* B, const float* Blo, in
   if (int e = device_props(&dp)) return e;
   if (dp.cc_major != 10) return fail(ADMMQ_E_UNSUPPORTED, "admmq_gemm_nt needs an sm_100 device (tcgen05)");
   const int tilesM = (M + tc::kTileM - 1) / tc::kTileM;
-  // tile width: a tile costs a fixed part plus bn columns of tensor-core work (measured 3.3 + 0.225 bn us at K = 1141);
-  // minimise waves * (16 + bn), ties go to the wider tile (128-wide tiles need the pre-split B operand)
-  int bn = 16;
-  {
-    long long best = -1;
-    const int widths[4] = {128, 64, 32, 16};
-    for (int w = (Blo != nullptr ? 0 : 1); w < 4; ++w) {
-      const long long tiles_w = (long long)tilesM * ((N + widths[w] - 1) / widths[w]);
-      const long long cost = ((tiles_w + dp.sm_count - 1) / dp.sm_count) * (16 + widths[w]);
-      if (best < 0 || cost < best) {
-        best = cost;
-        bn = widths[w];
-      }
-    }
-  }
+  const int bn = gemm_tile_width(M, N, dp.sm_count, Blo != nullptr);
   const int tiles = tilesM * ((N + bn - 1) / bn);
   const int grid = std::min(tiles, dp.sm_count);
   GemmMaps maps;
@@ -265,29 +330,8 @@ int mttkrp_fold_gemm(const float* V, int ldv, int Mout, int ny, const float* B, 
   DeviceProps dp;
   if (int e = device_props(&dp)) return e;
   if (dp.cc_major != 10) return fail(ADMMQ_E_UNSUPPORTED, "the tensor-core MTTKRP needs an sm_100 device (tcgen05)");
-  const int mg = tc::kTileM / ny;
-  const long long tilesM = (Mout + mg - 1) / mg;
-  // tile width: any multiple of 16 up to 128; a tile costs a fixed part (pipeline fill, epilogue, fold) worth ~40
-  // columns at K = 512 plus bn columns of tensor-core work: minimise waves * (kFoldFixed + bn), ties to the wider tile
-  constexpr int kFoldFixed = 40;
-  int bn = 64;
-  {
-    long long best = -1;
-    for (int w = 128; w >= 16; w -= 16) {
-      const long long tiles_w = tilesM * ((N + w - 1) / w);
-      const long long cost = ((tiles_w + dp.sm_count - 1) / dp.sm_count) * (kFoldFixed + w);
-      if (best < 0 || cost < best) {
-        best = cost;
-        bn = w;
-      }
-    }
-  }
-  if (const char* force = getenv("ADMMQ_FOLD_BN")) {  // experiment knob
-    const int w = atoi(force);
-    if (w >= 16 && w <= 128 && (w & 15) == 0) bn = w;
-  }
-  const long long tiles = tilesM * ((N + bn - 1) / bn);
-  const int grid = (int)std::min<long long>(tiles, dp.sm_count);
+  int grid;
+  const int bn = select_mttkrp_kernel(Mout, K, ny, N, 1, dp.sm_count, &grid, nullptr) - ADMMQ_MTTKRP_FOLD;
   GemmMaps maps;
   if (int e = tc::make_operand_tmap(&maps.a, V, Mout * ny, K, ldv, tc::kTileM)) return e;
   if (int e = tc::make_operand_tmap(&maps.b, B, N, K, ldb, bn)) return e;
@@ -320,22 +364,8 @@ int mttkrp_foldlong_gemm(const float* V, int ldv, int Mout, int ny, const float*
   if (int e = device_props(&dp)) return e;
   if (dp.cc_major != 10) return fail(ADMMQ_E_UNSUPPORTED, "the tensor-core MTTKRP needs an sm_100 device (tcgen05)");
   const int rows = Mout * ny;
-  const long long tilesM = (rows + tc::kTileM - 1) / tc::kTileM;
-  constexpr int kFoldFixed = 40;
-  int bn = 128;
-  {
-    long long best = -1;
-    for (int w = 128; w >= 80; w -= 16) {   // the fold maps one thread to one column of a 128-wide staging tile
-      const long long tiles_w = tilesM * ((N + w - 1) / w);
-      const long long cost = ((tiles_w + dp.sm_count - 1) / dp.sm_count) * (kFoldFixed + w);
-      if (best < 0 || cost < best) {
-        best = cost;
-        bn = w;
-      }
-    }
-  }
-  const long long tiles = tilesM * ((N + bn - 1) / bn);
-  const int grid = (int)std::min<long long>(tiles, dp.sm_count);
+  int grid;
+  const int bn = select_mttkrp_kernel(Mout, K, ny, N, 1, dp.sm_count, &grid, nullptr) - ADMMQ_MTTKRP_FOLDLONG;
   GemmMaps maps;
   if (int e = tc::make_operand_tmap(&maps.a, V, rows, K, ldv, tc::kTileM)) return e;
   if (int e = tc::make_operand_tmap(&maps.b, B, N, K, ldb, bn)) return e;
@@ -357,4 +387,10 @@ using namespace admmq;
 extern "C" int admmq_gemm_nt(const float* A, int lda, int M, const float* B, int ldb, int N, int K, float* C, int ldc,
                              void* stream_) {
   return gemm_nt(A, lda, M, B, nullptr, ldb, N, K, C, ldc, (cudaStream_t)stream_);
+}
+
+extern "C" int admmq_mttkrp_kernel(int M, int nx, int ny, int R, int precision, int sm_count, int* grid, int* splits) {
+  if (M <= 0 || nx <= 0 || ny <= 0 || R <= 0 || sm_count <= 0 || precision < 0 || precision > 1)
+    return fail(ADMMQ_E_BADARG, "admmq_mttkrp_kernel: bad argument");
+  return select_mttkrp_kernel(M, nx, ny, R, precision, sm_count, grid, splits);
 }

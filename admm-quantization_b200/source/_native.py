@@ -63,6 +63,8 @@ def _load():
         "admmq_permute_myx": (c_int, [vp, c_int, c_int, c_int, vp, vp]),
         "admmq_mttkrp_tc_workspace_bytes": (c_sz, [c_int, c_int, c_int, c_int]),
         "admmq_mttkrp_tc": (c_int, [vp, c_int, vp, c_int, vp, c_int, c_int, vp, vp, c_sz, vp]),
+        "admmq_mttkrp_kernel": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_int),
+                                        ctypes.POINTER(c_int)]),
         "admmq_mttkrp_f64_workspace_bytes": (c_sz, [c_int, c_int, c_int, c_int]),
         "admmq_mttkrp_f64": (c_int, [vp, c_int, vp, c_int, vp, c_int, c_int, vp, vp, c_sz, vp]),
         "admmq_gram_hadamard_f64": (c_int, [vp, c_int, vp, c_int, c_int, vp, vp]),
@@ -100,7 +102,8 @@ lib = _load()
 EXPORTS = ("admmq_version admmq_last_error admmq_device_info admmq_launch_count admmq_project_workspace_bytes "
            "admmq_project admmq_clip_search_sums admmq_admm_loop_kernel admmq_admm_loop_workspace_bytes admmq_admm_loop admmq_gemm_nt "
            "admmq_gram_hadamard admmq_unfold3 admmq_mttkrp_workspace_bytes admmq_mttkrp admmq_permute_myx "
-           "admmq_mttkrp_tc_workspace_bytes admmq_mttkrp_tc admmq_mttkrp_f64_workspace_bytes admmq_mttkrp_f64 "
+           "admmq_mttkrp_tc_workspace_bytes admmq_mttkrp_tc admmq_mttkrp_kernel admmq_mttkrp_f64_workspace_bytes "
+           "admmq_mttkrp_f64 "
            "admmq_gram_hadamard_f64 admmq_normalize_columns_f64 "
            "admmq_recon_error_workspace_bytes admmq_recon_error admmq_padded_ld admmq_spd_inverse_workspace_bytes "
            "admmq_spd_inverse admmq_admm_iteration_workspace_bytes admmq_admm_iteration "
@@ -305,6 +308,16 @@ def mttkrp_tc(V, M, X, Y=None, out=None, ws=None):
     ws = _ws(mttkrp_tc_workspace_bytes(M, nx, ny, R), V.device, ws)
     call(V.device, lib.admmq_mttkrp_tc, ptr(V), int(M), ptr(X), nx, ptr(Y), ny, R, ptr(F), ptr(ws), ws.numel(), stream_ptr(V.device))
     return F
+
+
+def mttkrp_kernel(M, nx, ny, R, precision, sm_count):
+    """(id, grid, splits) of the MTTKRP kernel (include/admmq.h ADMMQ_MTTKRP_*) a call runs on `sm_count` SMs;
+    precision 1 = mttkrp_tc, ny = 1 for a matrix."""
+    grid, splits = ctypes.c_int(0), ctypes.c_int(0)
+    rc = int(lib.admmq_mttkrp_kernel(int(M), int(nx), int(ny), int(R), int(precision), int(sm_count),
+                                     ctypes.byref(grid), ctypes.byref(splits)))
+    check(min(rc, 0))
+    return rc, grid.value, splits.value
 
 
 # ---- float64 pieces of the ALS + EPC initialisation (source/parafac_epc.py)

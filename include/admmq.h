@@ -114,6 +114,19 @@ ADMMQ_API size_t admmq_mttkrp_tc_workspace_bytes(int M, int nx, int ny, int R);
 ADMMQ_API int admmq_mttkrp_tc(const float* V, int M, const float* X, int nx, const float* Y, int ny, int R, float* F,
                     void* workspace, size_t workspace_bytes, void* stream);
 
+/* The kernel an MTTKRP call runs on a device with sm_count SMs: precision 0 is admmq_mttkrp(..., 0, ...), precision 1
+ * the permuted-operand call admmq_mttkrp_tc; ny = 1 for a matrix.  Pure host logic: needs no device, honours
+ * ADMMQ_FOLD_BN (a forced width of the fold, read per call).  Returns one of the ids below, or ADMMQ_E_BADARG.
+ *   grid    (or NULL) CTAs of the contraction kernel
+ *   splits  (or NULL) slices of the float64 sum over p (precision 0, with the workspace that
+ *           admmq_mttkrp_workspace_bytes asks for; a smaller one makes it 1); 1 on the tensor cores */
+#define ADMMQ_MTTKRP_F64_16 1       /* float64-accumulating CUDA-core tiles of 16 x 64 (M <= 16) */
+#define ADMMQ_MTTKRP_F64_64 2       /* ... of 64 x 64 */
+#define ADMMQ_MTTKRP_GEMM 1000      /* + tile width (16, 32, 64, 128): matrix, 3xTF32 tcgen05 product F = W . X */
+#define ADMMQ_MTTKRP_FOLD 2000      /* + tile width (16 .. 128, multiple of 16): 2 <= ny <= 128, y folded in the epilogue */
+#define ADMMQ_MTTKRP_FOLDLONG 3000  /* + tile width (80 .. 128, multiple of 16): ny > 128, two float64 partials per tile */
+ADMMQ_API int admmq_mttkrp_kernel(int M, int nx, int ny, int R, int precision, int sm_count, int* grid, int* splits);
+
 /* Reconstruction error pieces for squared_relative_diff  source/admm.py:14-15 with the einsum of
  * scripts/factorize.py:246-253 (3-D) / :296-297 (2-D):  out2 (device double[2]) = { sum (W - [[A,X,Y]])^2, sum W^2 }.
  *   W0 (M x P) mode-0 unfolding, A (M x R), X (nx x R), Y (ny x R) or NULL.  The reconstruction is never stored. */
