@@ -21,6 +21,7 @@
 #include <cstdlib>
 #include <cstring>
 #include "search.cuh"
+#include "admm_loop_common.cuh"
 #include "spd_inverse.cuh"
 #include "tc_gemm.cuh"
 #include "admm_loop_resident.cuh"
@@ -509,26 +510,6 @@ union LoopSmem {
   SkinnySmem<(TCBN < 0 && TCBN != kDiagP1 && TCBN != kF64P1 ? -TCBN : 1)> skinny;
 };
 
-// sum over the CTA of four per-thread doubles, result valid in every thread
-__device__ __forceinline__ void cta_sum4(double v[4], ResidualSmem& rs) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int q = 0; q < 4; ++q) v[q] = warp_sum(v[q]);
-  __syncthreads();
-  if (lane == 0) {
-#pragma unroll
-    for (int q = 0; q < 4; ++q) rs.red[q][warp] = v[q];
-  }
-  __syncthreads();
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    double s = 0.0;
-#pragma unroll
-    for (int w = 0; w < kWarps; ++w) s += rs.red[q][w];
-    v[q] = s;
-  }
-}
-
 // Totals of the per-CTA residual slots, formed redundantly by every warp: lane c takes the CTAs c, c + 32, ... in
 // order, then a xor butterfly (the same association in every lane, warp and CTA, so every thread of the grid holds
 // bit-identical totals) - no shared memory and no CTA barrier on the path of the exit test.
@@ -721,8 +702,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop(const __grid_constant
         bar.sync();
         lap(1);
         // ---------------- P3
-        rep.best_index = cta_best_candidate(cand, p.Nc, absmax, (double)N, sm.search.direct);
-        qp.scale = scale_of(clip_candidate(make_clip_grid(absmax, p.Nc), rep.best_index), L);
+        rep.best_index = cta_best_candidate<true>(cand, p.Nc, absmax, (double)N, sm.search.direct.key);
+        qp.scale = clip_scale(absmax, p.Nc, rep.best_index, L);
       }
     } else {
       degenerate = (absmax != absmax) || isinf(absmax);
@@ -1098,13 +1079,33 @@ static int select_loop_kernel(int I, int R, int num_attempts, int precision, int
   }
 }
 
+// one launch of a shared-memory loop kernel on a thread-block cluster of `ctas` CTAs (the whole grid)
+static int launch_cluster(void (*kernel)(ResidentParams), int ctas, size_t smem, const ResidentParams& rp, cudaStream_t stream) {
+  ADMMQ_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  cudaLaunchConfig_t cfg;
+  memset(&cfg, 0, sizeof(cfg));
+  cfg.gridDim = dim3(ctas);
+  cfg.blockDim = dim3(kThreads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = ctas;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  ADMMQ_CUDA_OK(cudaLaunchKernelEx(&cfg, kernel, rp));
+  count_launches(1);
+  return ADMMQ_OK;
+}
+
 static int launch_loop(float* H, float* U, const float* F, const float* Minv, const double* Minv64, const float* rho,
                        const int* inv_status, int I, int R, int max_iter, float eps, int bits, int qscheme, int num_attempts, int precision,
                        int8_t* codes, admmq_loop_report* report, char* ws, int grid, cudaStream_t stream) {
   const LoopLayout l = loop_layout(I, R, grid);
   const int kid = select_loop_kernel(I, R, num_attempts, precision, grid);
-  if (kid == ADMMQ_LOOP_RESIDENT || kid == ADMMQ_LOOP_CLUSTER4 || kid == ADMMQ_LOOP_CLUSTER8) {
-    const int ccl = kid == ADMMQ_LOOP_CLUSTER8 ? 8 : kid == ADMMQ_LOOP_CLUSTER4 ? 4 : 0;
+  if (kid == ADMMQ_LOOP_RESIDENT || kid == ADMMQ_LOOP_CLUSTER4 || kid == ADMMQ_LOOP_CLUSTER8 || kid == ADMMQ_LOOP_TAP) {
     ResidentParams rp;
     rp.H = H;
     rp.U = U;
@@ -1122,64 +1123,12 @@ static int launch_loop(float* H, float* U, const float* F, const float* Minv, co
     rp.Nc = (qscheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) ? num_attempts : 0;
     rp.codes = codes;
     rp.report = report;
-    if (ccl >= 4) {
-      ADMMQ_CUDA_OK(cudaFuncSetAttribute(k_admm_loop_cluster, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ClusterSmem)));
-      cudaLaunchConfig_t cfg;
-      memset(&cfg, 0, sizeof(cfg));
-      cfg.gridDim = dim3(ccl);
-      cfg.blockDim = dim3(kThreads);
-      cfg.dynamicSmemBytes = sizeof(ClusterSmem);
-      cfg.stream = stream;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = ccl;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      ADMMQ_CUDA_OK(cudaLaunchKernelEx(&cfg, k_admm_loop_cluster, rp));
-      count_launches(1);
-      return ADMMQ_OK;
-    }
+    if (kid == ADMMQ_LOOP_TAP) return launch_cluster(k_admm_loop_tap<kTapMaxRows>, kTapCtas, sizeof(TapSmem), rp, stream);
+    if (kid != ADMMQ_LOOP_RESIDENT)
+      return launch_cluster(k_admm_loop_cluster, kid == ADMMQ_LOOP_CLUSTER8 ? 8 : 4, sizeof(ClusterSmem), rp, stream);
     ADMMQ_CUDA_OK(cudaFuncSetAttribute(k_admm_loop_resident, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ResidentSmem)));
     k_admm_loop_resident<<<1, kThreads, sizeof(ResidentSmem), stream>>>(rp);
     ADMMQ_CUDA_OK(cudaGetLastError());
-    count_launches(1);
-    return ADMMQ_OK;
-  }
-  if (kid == ADMMQ_LOOP_TAP) {
-    ResidentParams rp;
-    rp.H = H;
-    rp.U = U;
-    rp.F = F;
-    rp.Minv = Minv;
-    rp.rho = rho;
-    rp.inv_status = inv_status;
-    rp.I = I;
-    rp.R = R;
-    rp.Rp = l.Rp;
-    rp.max_iter = max_iter;
-    rp.eps = eps;
-    rp.bits = bits;
-    rp.scheme = qscheme;
-    rp.Nc = (qscheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) ? num_attempts : 0;
-    rp.codes = codes;
-    rp.report = report;
-    ADMMQ_CUDA_OK(cudaFuncSetAttribute(k_admm_loop_tap<kTapMaxRows>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TapSmem)));
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(kTapCtas);
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = sizeof(TapSmem);
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = kTapCtas;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    ADMMQ_CUDA_OK(cudaLaunchKernelEx(&cfg, k_admm_loop_tap<kTapMaxRows>, rp));
     count_launches(1);
     return ADMMQ_OK;
   }

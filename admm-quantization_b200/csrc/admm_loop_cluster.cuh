@@ -22,6 +22,7 @@
 // of 2, 4 and 8 CTAs; against the single-CTA kernel (float32 FMAs) they differ by the rounding of the product only
 // (tests/test_gpu_parity_r2.py).
 #pragma once
+#include "admm_loop_common.cuh"
 #include "admm_loop_resident.cuh"
 
 namespace admmq {
@@ -84,195 +85,19 @@ __device__ __forceinline__ void cl_store(unsigned int addr, double v) {
   asm volatile("st.shared::cluster.f64 [%0], %1;" ::"r"(addr), "d"(v) : "memory");
 }
 
-// sum over the CTA of four per-thread doubles (fixed order), result valid in every thread
-template <class Smem>
-__device__ __forceinline__ void cl_sum4(double v[4], Smem& sm) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int q = 0; q < 4; ++q) v[q] = warp_sum(v[q]);
-  __syncthreads();
-  if (lane == 0) {
-#pragma unroll
-    for (int q = 0; q < 4; ++q) sm.red[q][warp] = v[q];
-  }
-  __syncthreads();
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    double s = 0.0;
-#pragma unroll
-    for (int w = 0; w < kWarps; ++w) s += sm.red[q][w];
-    v[q] = s;
-  }
-}
-
-// Fixed-point sums of squared errors of the n elements of sm.Vall for candidates [c0, c1) into sm.acc (threshold form,
-// the same recipe - element order, fixed-point units, float64 terms - as res_candidate_sums of the resident kernel).
-template <class Smem>
-__device__ inline void cl_candidate_sums(Smem& sm, int n, float absmax, int Nc, int c0, int c1, const Levels L, int bits) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const ClipGrid g = make_clip_grid(absmax, Nc);
-  const double unit_inv = fixed_point_unit_inv((double)n, absmax);
-  const FixX fx = make_fix_x(absmax);
-  const float bmul = div_rn((float)(kResBins / 2), absmax);
-  const int nthr = (1 << bits) - 1;
-  const int ncand = c1 - c0;
-  const int npairs = ncand * nthr;
-  for (int c = c0 + tid; c < c1; c += kThreads) {
-    sm.scale[c] = scale_of(clip_candidate(g, c), L);
-    sm.acc[c] = 0ull;
-  }
-  float* sorted = sm.X;
-  for (int b = tid; b < kResBins; b += kThreads) {
-    sm.cnt[b] = 0u;
-    sm.slo[b] = 0u;
-    sm.shi[b] = 0u;
-  }
-  __syncthreads();
-  // pass 1: histogram (count + 64-bit fixed-point sum per bin) and the sum of squares
-  double x2 = 0.0;
-  for (int e = tid; e < n; e += kThreads) {
-    const float x = sm.Vall[e];
-    const int b = res_bin_of(x, bmul);
-    atomicAdd(&sm.cnt[b], 1u);
-    const long long f = fix_x(x, fx);
-    const unsigned int lo = (unsigned int)f, hi = (unsigned int)((unsigned long long)f >> 32);
-    const unsigned int old = atomicAdd(&sm.slo[b], lo);
-    atomicAdd(&sm.shi[b], hi + ((old + lo < old) ? 1u : 0u));
-    const double xd = (double)x;
-    x2 = fma(xd, xd, x2);
-  }
-  __syncthreads();
-  // exclusive scan over the bins: thread t owns kResBins / kThreads consecutive bins
-  {
-    constexpr int kPer = kResBins / kThreads;
-    const int b0 = tid * kPer;
-    unsigned int c[kPer], lo[kPer], hi[kPer];
-#pragma unroll
-    for (int i = 0; i < kPer; ++i) {
-      c[i] = sm.cnt[b0 + i];
-      lo[i] = sm.slo[b0 + i];
-      hi[i] = sm.shi[b0 + i];
-    }
-    unsigned int ct = 0u;
-    unsigned long long st = 0ull;
-#pragma unroll
-    for (int i = 0; i < kPer; ++i) {
-      ct += c[i];
-      st += ((unsigned long long)hi[i] << 32) | lo[i];
-    }
-    unsigned int ci = ct;
-    unsigned long long si = st;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const unsigned int nc = __shfl_up_sync(0xffffffffu, ci, o);
-      const unsigned long long ns = __shfl_up_sync(0xffffffffu, si, o);
-      if (lane >= o) {
-        ci += nc;
-        si += ns;
-      }
-    }
-    if (lane == 31) {
-      sm.wcnt[warp] = ci;
-      sm.wsum[warp] = si;
-    }
-    __syncthreads();
-    unsigned int rc = ci - ct;
-    unsigned long long rs = si - st;
-    for (int w = 0; w < warp; ++w) {
-      rc += sm.wcnt[w];
-      rs += sm.wsum[w];
-    }
-#pragma unroll
-    for (int i = 0; i < kPer; ++i) {
-      const unsigned int cc = c[i];
-      const unsigned long long ss = ((unsigned long long)hi[i] << 32) | lo[i];
-      sm.cnt[b0 + i] = rc;
-      sm.slo[b0 + i] = (unsigned int)rs;
-      sm.shi[b0 + i] = (unsigned int)(rs >> 32);
-      rc += cc;
-      rs += ss;
-    }
-  }
-  __syncthreads();
-  // pass 2: counting-sort scatter into X (cnt[b] runs from the start to the end of bin b)
-  for (int e = tid; e < n; e += kThreads) {
-    const float x = sm.Vall[e];
-    const unsigned int pos = atomicAdd(&sm.cnt[res_bin_of(x, bmul)], 1u);
-    sorted[pos] = x;
-  }
-  __syncthreads();
-  // pass 3: one (candidate, threshold) pair per thread, own candidates only
-  {
-    long long ptot = 0ll;
-    for (int w = 0; w < kWarps; ++w) ptot += (long long)sm.wsum[w];
-    for (int p = tid; p < npairs; p += kThreads) {
-      const int j = p / ncand, c = c0 + (p - j * ncand);
-      const float s = sm.scale[c];
-      const float level = L.lo + (float)j;
-      const float theta = code_threshold(s, level);
-      const int b = res_bin_of(theta, bmul);
-      const unsigned int beg = b ? sm.cnt[b - 1] : 0u, end = sm.cnt[b];
-      long long ps = (long long)(((unsigned long long)sm.shi[b] << 32) | sm.slo[b]);
-      long long cn = (long long)beg;
-      for (unsigned int i = beg; i < end; ++i) {
-        const float x = sorted[i];
-        if (x < theta) {
-          ++cn;
-          ps += fix_x(x, fx);
-        }
-      }
-      double term = threshold_term(s, level, cn, ps, fx.unit);
-      if (j == nthr - 1) term += closing_term(s, L.hi, (long long)n, ptot, fx.unit);
-      atomicAdd(&sm.acc[c], (unsigned long long)__double2ll_rn(term * unit_inv));
-    }
-  }
-  // sum of squares, fixed order
-  x2 = warp_sum(x2);
-  __syncthreads();
-  if (lane == 0) sm.red[0][warp] = x2;
-  __syncthreads();
-  double tot = 0.0;
-#pragma unroll
-  for (int w = 0; w < kWarps; ++w) tot += sm.red[0][w];
-  const long long x2f = __double2ll_rn(tot * unit_inv);
-  for (int c = c0 + tid; c < c1; c += kThreads) {
-    const long long f = (long long)sm.acc[c] + x2f;
-    sm.acc[c] = (unsigned long long)max(f, 0ll);
-  }
-  __syncthreads();
-}
-
 __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_cluster(const ResidentParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   ClusterSmem& sm = *reinterpret_cast<ClusterSmem*>(smem_raw);
   const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
   const int I = p.I, R = p.R, Rp = p.Rp, n = I * R;
   const int rank = (int)cl_rank(), C = (int)cl_size();
-  admmq_loop_report rep;
-  rep.iterations = 0;
-  rep.status = 0;
-  rep.rho = *p.rho;
-  rep.scale = 0.0f;
-  rep.r = 0.0f;
-  rep.s = 0.0f;
-  rep.best_index = -1;
-  rep.absmax = 0.0f;
-  rep.phase_ns[0] = rep.phase_ns[1] = rep.phase_ns[2] = rep.phase_ns[3] = 0ull;
-  if (p.inv_status != nullptr && *p.inv_status != 0) {  // uniform over the cluster: nobody reaches a barrier
-    rep.status = *p.inv_status;
-    if (rank == 0 && t == 0) *p.report = rep;
-    return;
-  }
-  const unsigned long long t_begin = global_ns();
-  unsigned long long t_mark = t_begin;
-  auto lap = [&](int phase) {
-    const unsigned long long now = global_ns();
-    rep.phase_ns[phase] += now - t_mark;
-    t_mark = now;
-  };
+  LoopReport rb;
+  admmq_loop_report& rep = rb.rep;
+  // inv_status is uniform over the cluster: nobody reaches a barrier
+  if (!rb.begin(p.rho, p.inv_status, p.report, rank == 0 && t == 0)) return;
+  rb.start();
   const float rho = rep.rho;
   const Levels L = make_levels(p.bits);
-  const float qnan = __int_as_float(0x7fc00000);
   // own rows [i0, i1) and own candidates [c0, c1)
   const int rows_per = (I + C - 1) / C;
   const int i0 = min(I, rank * rows_per), i1 = min(I, i0 + rows_per);
@@ -287,7 +112,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_cluster(const Residen
     const int il = e / R, c = e - il * R;
     const float u = p.U[e_base + e];
     sm.U[e] = u;
-    rhs[il * Rp + c] = (double)add_rn(p.F[e_base + e], mul_rn(rho, add_rn(p.H[e_base + e], u)));
+    rhs[il * Rp + c] = (double)rhs_of(p.F[e_base + e], rho, p.H[e_base + e], u);
   }
   cl_sync();   // every CTA of the cluster is running (remote shared memory may be written from here on)
   const int row_groups = (own_rows + 3) / 4;
@@ -341,18 +166,11 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_cluster(const Residen
       cl_store(cl_map(&sm.keys[rank][t & 1], (unsigned int)(t >> 1)), k);
     }
     cl_sync();   // ---- barrier 1: V, keys (and the previous iteration's residual sums) are everywhere
-    if (pending) {   // exit test of iteration j - 1 (:62-65), evaluated identically by every CTA
-      double tot[4] = {0.0, 0.0, 0.0, 0.0};
-      for (int rk = 0; rk < C; ++rk)
-#pragma unroll
-        for (int q = 0; q < 4; ++q) tot[q] += sm.slots[rk][q];
-      rep.r = div_rn((float)tot[0], (float)tot[1]);
-      rep.s = div_rn((float)tot[2], (float)tot[3]);
-      if (rep.r < p.eps && rep.s < p.eps) {   // the speculative P1 above touched neither H, U nor RHS
-        rep.status |= ADMMQ_ST_CONVERGED;
-        pending = false;
-        break;
-      }
+    // exit test of iteration j - 1 (:62-65); the speculative P1 above touched neither H, U nor RHS
+    if (pending && cluster_converged(sm.slots, C, p.eps, rep)) {
+      rep.status |= ADMMQ_ST_CONVERGED;
+      pending = false;
+      break;
     }
     kmax = 0u;
     kinv = 0u;
@@ -360,131 +178,56 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_cluster(const Residen
       kmax = max(kmax, sm.keys[rk][0]);
       kinv = max(kinv, sm.keys[rk][1]);
     }
-    lap(0);
+    rb.lap(0);
     // ---------------- P2
-    const float tmax = key_float(kmax), tmin = key_float(~kinv);
-    float absmax = fmaxf(fabsf(tmin), fabsf(tmax));
-    if (tmin != tmin || tmax != tmax) absmax = qnan;
-    rep.absmax = absmax;
+    const Projection pj = projection_from_keys(kmax, kinv, p.scheme, p.bits, L);
+    rep.absmax = pj.absmax;
     rep.iterations = j;
     done = j;
-    QParams qp;
-    qp.scheme = p.scheme;
-    qp.bits = p.bits;
-    qp.aux = 0.0f;
-    qp.n = 0.0f;
-    qp.scale = 0.0f;
-    bool degenerate = false;
-    if (p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) {
-      degenerate = !(absmax > 0.0f) || isinf(absmax);
-      if (!degenerate) {
-        if (binned_range_ok(absmax)) {
-          cl_candidate_sums(sm, n, absmax, p.Nc, c0, c1, L, p.bits);
-        } else {
-          // extreme magnitudes (outside [2^-40, 2^40]): plain evaluation of every (element, candidate) pair
-          const ClipGrid g = make_clip_grid(absmax, p.Nc);
-          const double unit_inv = fixed_point_unit_inv((double)n, absmax);
-          for (int c = c0 + t; c < c1; c += kThreads) {
-            const float s = scale_of(clip_candidate(g, c), L);
-            double tot = 0.0;
-            for (int e = 0; e < n; ++e) tot += (double)sqerr_exact(sm.Vall[e], s, L);
-            sm.acc[c] = (unsigned long long)__double2ll_rn(tot * unit_inv);
-          }
-          __syncthreads();
-        }
-        for (int c = c0 + t; c < c1; c += kThreads) {
-          const unsigned long long v = sm.acc[c];
-          for (int rk = 0; rk < C; ++rk) cl_store(cl_map(&sm.cand[c], (unsigned int)rk), v);
-        }
+    QParams qp = pj.qp;
+    const bool search = p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC && !pj.degenerate;
+    if (search) {
+      smem_candidate_sums(sm, n, [&](int e) { return sm.Vall[e]; }, pj.absmax, p.Nc, c0, c1, L, p.bits);
+      for (int c = c0 + t; c < c1; c += kThreads) {
+        const unsigned long long v = sm.acc[c];
+        for (int rk = 0; rk < C; ++rk) cl_store(cl_map(&sm.cand[c], (unsigned int)rk), v);
       }
-    } else {
-      degenerate = (absmax != absmax) || isinf(absmax);
-      qp = params_from_minmax(p.scheme, p.bits, tmin, tmax, L);
     }
     cl_sync();   // ---- barrier 2: every candidate's sum is everywhere (and nobody reads V / the sorted array any more)
-    if (p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC && !degenerate) {
-      // first index of the smallest MSE (torch.argmin)
-      const double unit = fixed_point_unit((double)n, absmax);
-      const float nf = (float)n;
-      unsigned long long best = ~0ull;
-      for (int c = t; c < p.Nc; c += kThreads) {
-        const float mse = mse_from_fixed((long long)sm.cand[c], unit, nf);
-        best = min(best, ((unsigned long long)float_key(mse) << 32) | (unsigned int)c);
-      }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) best = min(best, __shfl_xor_sync(0xffffffffu, best, o));
-      if (lane == 0) sm.best[warp] = best;
-      __syncthreads();
-      unsigned long long b = sm.best[0];
-#pragma unroll
-      for (int w = 1; w < kWarps; ++w) b = min(b, sm.best[w]);
-      rep.best_index = (int)(b & 0xffffffffu);
-      qp.scale = scale_of(clip_candidate(make_clip_grid(absmax, p.Nc), rep.best_index), L);
+    if (search) {
+      rep.best_index = cta_best_candidate<false>(sm.cand, p.Nc, pj.absmax, (double)n, sm.best);
+      qp.scale = clip_scale(pj.absmax, p.Nc, rep.best_index, L);
     }
     rep.scale = qp.scale;
-    lap(1);
+    rb.lap(1);
     // ---------------- P3: H = Q(V), U += H - H_ls, residual sums, next RHS - own rows
-    float f0 = 0.0f, f1 = 0.0f, f2 = 0.0f, f3 = 0.0f;
-    double sums[4] = {0.0, 0.0, 0.0, 0.0};
-    int cnt = 0;
+    ResidualSums res;
     for (int e = t; e < own; e += kThreads) {
       const int il = e / R, c = e - il * R;
       const float hp = p.H[e_base + e];
       const float fv = __ldg(p.F + e_base + e);
-      const float hls = sm.Hls[e], u = sm.U[e];
-      const float v = sub_rn(hls, u);
-      float code = 0.0f;
-      const float hq = degenerate ? qnan : quantize_value(v, qp, L, code);   // H = Q(H_ls - U)   (:59)
-      const float d1 = sub_rn(hq, hls);
-      const float un = add_rn(u, d1);                                        // U += H - H_ls     (:60)
-      const float d2 = sub_rn(hq, hp);
-      f0 = fmaf(d1, d1, f0);  // sum (H - H_ls)^2     (:62)
-      f1 = fmaf(hq, hq, f1);  // sum H^2
-      f2 = fmaf(d2, d2, f2);  // sum (H - H_prev)^2   (:63)
-      f3 = fmaf(un, un, f3);  // sum U^2
-      p.H[e_base + e] = hq;
-      sm.U[e] = un;
-      rhs[il * Rp + c] = (double)add_rn(fv, mul_rn(rho, add_rn(hq, un)));
-      if (p.codes != nullptr) p.codes[e_base + e] = (int8_t)code;
-      if (++cnt == 16) {
-        sums[0] += (double)f0;
-        sums[1] += (double)f1;
-        sums[2] += (double)f2;
-        sums[3] += (double)f3;
-        f0 = f1 = f2 = f3 = 0.0f;
-        cnt = 0;
-      }
+      const ElementStep o = p3_element(sm.Hls[e], sm.U[e], hp, fv, rho, qp, L, pj.degenerate, res);
+      p.H[e_base + e] = o.hq;
+      sm.U[e] = o.un;
+      rhs[il * Rp + c] = (double)o.rhs_next;
+      if (p.codes != nullptr) p.codes[e_base + e] = (int8_t)o.code;
     }
-    sums[0] += (double)f0;
-    sums[1] += (double)f1;
-    sums[2] += (double)f2;
-    sums[3] += (double)f3;
-    if (degenerate) {  // uniform: the reference would carry NaN through every remaining iteration
-      rep.status |= ADMMQ_ST_NONFINITE;
-      rep.r = qnan;
-      rep.s = qnan;
+    res.flush();
+    if (pj.degenerate) {  // uniform
+      rb.nonfinite();
       pending = false;
       break;
     }
-    cl_sum4(sums, sm);  // (contains the barriers that publish U and X for the next iteration)
-    if (t < 4 * C) cl_store(cl_map(&sm.slots[rank][t & 3], (unsigned int)(t >> 2)), sums[t & 3]);
+    cta_sum4(res.sums, sm);  // (contains the barriers that publish U and X for the next iteration)
+    if (t < 4 * C) cl_store(cl_map(&sm.slots[rank][t & 3], (unsigned int)(t >> 2)), res.total(t & 3));
     pending = true;
-    lap(2);
+    rb.lap(2);
   }
   cl_sync();   // the last residual sums are everywhere; no CTA leaves while its shared memory may still be written
-  if (pending) {
-    double tot[4] = {0.0, 0.0, 0.0, 0.0};
-    for (int rk = 0; rk < C; ++rk)
-#pragma unroll
-      for (int q = 0; q < 4; ++q) tot[q] += sm.slots[rk][q];
-    rep.r = div_rn((float)tot[0], (float)tot[1]);
-    rep.s = div_rn((float)tot[2], (float)tot[3]);
-    if (rep.r < p.eps && rep.s < p.eps) rep.status |= ADMMQ_ST_CONVERGED;
-  }
+  if (pending && cluster_converged(sm.slots, C, p.eps, rep)) rep.status |= ADMMQ_ST_CONVERGED;
   rep.iterations = done;
   for (int e = t; e < own; e += kThreads) p.U[e_base + e] = sm.U[e];
-  rep.phase_ns[3] = global_ns() - t_begin;
-  if (rank == 0 && t == 0) *p.report = rep;
+  rb.finish(p.report, rank == 0 && t == 0);
 }
 
 // Size of the cluster for a factor: the largest power of two in {8, 4} within the budget for which a CTA's own rows fit

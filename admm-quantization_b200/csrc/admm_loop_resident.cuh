@@ -12,13 +12,12 @@
 // Results follow the same float32 recipe as the general kernel's parity mode (precision 0) up to the summation order
 // of the ridge product.
 #pragma once
-#include "search.cuh"
+#include "admm_loop_common.cuh"
 
 namespace admmq {
 
 constexpr int kResMaxElems = 8704;        // I * R  (64 x 136)
 constexpr int kResMaxMinv = 136 * 136;    // R * Rp
-constexpr int kResBins = 2048;
 
 struct ResidentParams {
   float* H;
@@ -52,208 +51,23 @@ struct __align__(16) ResidentSmem {
   unsigned long long best[kWarps];
 };
 
-__device__ __forceinline__ int res_bin_of(float x, float bmul) {
-  const float t = fma_rn(x, bmul, 12582912.0f + (float)(kResBins / 2));
-  const int b = (int)__float_as_uint(t) - 0x4B400000;
-  return min(max(b, 0), kResBins - 1);
-}
-
-// sum over the CTA of four per-thread doubles (fixed order), result valid in every thread
-__device__ __forceinline__ void res_sum4(double v[4], ResidentSmem& sm) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int q = 0; q < 4; ++q) v[q] = warp_sum(v[q]);
-  __syncthreads();
-  if (lane == 0) {
-#pragma unroll
-    for (int q = 0; q < 4; ++q) sm.red[q][warp] = v[q];
-  }
-  __syncthreads();
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    double s = 0.0;
-#pragma unroll
-    for (int w = 0; w < kWarps; ++w) s += sm.red[q][w];
-    v[q] = s;
-  }
-}
-
-// Per-candidate sums of squared errors of V = Hls - U (n elements) in the threshold form, into sm.acc (fixed point).
-__device__ inline void res_candidate_sums(ResidentSmem& sm, int n, float absmax, int Nc, const Levels L, int bits) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const ClipGrid g = make_clip_grid(absmax, Nc);
-  const double unit_inv = fixed_point_unit_inv((double)n, absmax);
-  const FixX fx = make_fix_x(absmax);
-  const float bmul = div_rn((float)(kResBins / 2), absmax);
-  const int nthr = (1 << bits) - 1;
-  const int npairs = Nc * nthr;
-  for (int c = tid; c < Nc; c += kThreads) {
-    sm.scale[c] = scale_of(clip_candidate(g, c), L);
-    sm.acc[c] = 0ull;
-  }
-  for (int b = tid; b < kResBins; b += kThreads) {
-    sm.cnt[b] = 0u;
-    sm.slo[b] = 0u;
-    sm.shi[b] = 0u;
-  }
-  __syncthreads();
-  // pass 1: histogram (count + 64-bit fixed-point sum per bin) and the sum of squares
-  double x2 = 0.0;
-  for (int e = tid; e < n; e += kThreads) {
-    const float x = sub_rn(sm.Hls[e], sm.U[e]);
-    const int b = res_bin_of(x, bmul);
-    atomicAdd(&sm.cnt[b], 1u);
-    const long long f = fix_x(x, fx);
-    const unsigned int lo = (unsigned int)f, hi = (unsigned int)((unsigned long long)f >> 32);
-    const unsigned int old = atomicAdd(&sm.slo[b], lo);
-    atomicAdd(&sm.shi[b], hi + ((old + lo < old) ? 1u : 0u));
-    const double xd = (double)x;
-    x2 = fma(xd, xd, x2);
-  }
-  __syncthreads();
-  // exclusive scan over the bins: thread t owns kResBins / kThreads consecutive bins
-  {
-    constexpr int kPer = kResBins / kThreads;
-    const int b0 = tid * kPer;
-    unsigned int c[kPer], lo[kPer], hi[kPer];
-#pragma unroll
-    for (int i = 0; i < kPer; ++i) {
-      c[i] = sm.cnt[b0 + i];
-      lo[i] = sm.slo[b0 + i];
-      hi[i] = sm.shi[b0 + i];
-    }
-    unsigned int ct = 0u;
-    unsigned long long st = 0ull;
-#pragma unroll
-    for (int i = 0; i < kPer; ++i) {
-      ct += c[i];
-      st += ((unsigned long long)hi[i] << 32) | lo[i];
-    }
-    unsigned int ci = ct;
-    unsigned long long si = st;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const unsigned int nc = __shfl_up_sync(0xffffffffu, ci, o);
-      const unsigned long long ns = __shfl_up_sync(0xffffffffu, si, o);
-      if (lane >= o) {
-        ci += nc;
-        si += ns;
-      }
-    }
-    if (lane == 31) {
-      sm.wcnt[warp] = ci;
-      sm.wsum[warp] = si;
-    }
-    __syncthreads();
-    unsigned int rc = ci - ct;
-    unsigned long long rs = si - st;
-    for (int w = 0; w < warp; ++w) {
-      rc += sm.wcnt[w];
-      rs += sm.wsum[w];
-    }
-#pragma unroll
-    for (int i = 0; i < kPer; ++i) {
-      const unsigned int cc = c[i];
-      const unsigned long long ss = ((unsigned long long)hi[i] << 32) | lo[i];
-      sm.cnt[b0 + i] = rc;
-      sm.slo[b0 + i] = (unsigned int)rs;
-      sm.shi[b0 + i] = (unsigned int)(rs >> 32);
-      rc += cc;
-      rs += ss;
-    }
-  }
-  __syncthreads();
-  // pass 2: counting-sort scatter into X (cnt[b] runs from the start to the end of bin b)
-  for (int e = tid; e < n; e += kThreads) {
-    const float x = sub_rn(sm.Hls[e], sm.U[e]);
-    const unsigned int pos = atomicAdd(&sm.cnt[res_bin_of(x, bmul)], 1u);
-    sm.X[pos] = x;
-  }
-  __syncthreads();
-  // pass 3: one (candidate, threshold) pair per thread
-  {
-    long long ptot = 0ll;
-    for (int w = 0; w < kWarps; ++w) ptot += (long long)sm.wsum[w];
-    int j = tid / Nc, c = tid - j * Nc;
-    const int dj = kThreads / Nc, dc = kThreads - dj * Nc;
-    for (int p = tid; p < npairs; p += kThreads) {
-      const float s = sm.scale[c];
-      const float level = L.lo + (float)j;
-      const float theta = code_threshold(s, level);
-      const int b = res_bin_of(theta, bmul);
-      const unsigned int beg = b ? sm.cnt[b - 1] : 0u, end = sm.cnt[b];
-      long long ps = (long long)(((unsigned long long)sm.shi[b] << 32) | sm.slo[b]);
-      long long cn = (long long)beg;
-      for (unsigned int i = beg; i < end; ++i) {
-        const float x = sm.X[i];
-        if (x < theta) {
-          ++cn;
-          ps += fix_x(x, fx);
-        }
-      }
-      double term = threshold_term(s, level, cn, ps, fx.unit);
-      if (j == nthr - 1) term += closing_term(s, L.hi, (long long)n, ptot, fx.unit);
-      atomicAdd(&sm.acc[c], (unsigned long long)__double2ll_rn(term * unit_inv));
-      j += dj;
-      c += dc;
-      if (c >= Nc) {
-        c -= Nc;
-        ++j;
-      }
-    }
-  }
-  // sum of squares, fixed order
-  x2 = warp_sum(x2);
-  __syncthreads();
-  if (lane == 0) sm.red[0][warp] = x2;
-  __syncthreads();
-  double tot = 0.0;
-#pragma unroll
-  for (int w = 0; w < kWarps; ++w) tot += sm.red[0][w];
-  const long long x2f = __double2ll_rn(tot * unit_inv);
-  for (int c = tid; c < Nc; c += kThreads) {
-    const long long f = (long long)sm.acc[c] + x2f;
-    sm.acc[c] = (unsigned long long)max(f, 0ll);
-  }
-  __syncthreads();
-}
-
 __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_resident(const ResidentParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   ResidentSmem& sm = *reinterpret_cast<ResidentSmem*>(smem_raw);
   const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
   const int I = p.I, R = p.R, Rp = p.Rp, n = I * R;
-  admmq_loop_report rep;
-  rep.iterations = 0;
-  rep.status = 0;
-  rep.rho = *p.rho;
-  rep.scale = 0.0f;
-  rep.r = 0.0f;
-  rep.s = 0.0f;
-  rep.best_index = -1;
-  rep.absmax = 0.0f;
-  rep.phase_ns[0] = rep.phase_ns[1] = rep.phase_ns[2] = rep.phase_ns[3] = 0ull;
-  if (p.inv_status != nullptr && *p.inv_status != 0) {
-    rep.status = *p.inv_status;
-    if (t == 0) *p.report = rep;
-    return;
-  }
-  const unsigned long long t_begin = global_ns();
-  unsigned long long t_mark = t_begin;
-  auto lap = [&](int phase) {
-    const unsigned long long now = global_ns();
-    rep.phase_ns[phase] += now - t_mark;
-    t_mark = now;
-  };
+  LoopReport rb;
+  admmq_loop_report& rep = rb.rep;
+  if (!rb.begin(p.rho, p.inv_status, p.report, t == 0)) return;
+  rb.start();
   const float rho = rep.rho;
   const Levels L = make_levels(p.bits);
-  const float qnan = __int_as_float(0x7fc00000);
   // ---- state into shared memory; RHS = F + rho (H + U) for the first iteration (:56)
   for (int e = t; e < R * Rp; e += kThreads) sm.Minv[e] = p.Minv[e];
   for (int e = t; e < n; e += kThreads) {
     const float u = p.U[e];
     sm.U[e] = u;
-    sm.X[e] = add_rn(p.F[e], mul_rn(rho, add_rn(p.H[e], u)));
+    sm.X[e] = rhs_of(p.F[e], rho, p.H[e], u);
   }
   __syncthreads();
   // P1 mapping: 4 rows x 5 columns per thread
@@ -315,66 +129,22 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_resident(const Reside
       kmax = max(kmax, sm.wkey[0][w]);
       kinv = max(kinv, sm.wkey[1][w]);
     }
-    lap(0);
+    rb.lap(0);
     // ---------------- P2
-    const float tmax = key_float(kmax), tmin = key_float(~kinv);
-    float absmax = fmaxf(fabsf(tmin), fabsf(tmax));
-    if (tmin != tmin || tmax != tmax) absmax = qnan;
-    rep.absmax = absmax;
+    const Projection pj = projection_from_keys(kmax, kinv, p.scheme, p.bits, L);
+    rep.absmax = pj.absmax;
     rep.iterations = j;
-    QParams qp;
-    qp.scheme = p.scheme;
-    qp.bits = p.bits;
-    qp.aux = 0.0f;
-    qp.n = 0.0f;
-    qp.scale = 0.0f;
-    bool degenerate = false;
-    if (p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) {
-      degenerate = !(absmax > 0.0f) || isinf(absmax);
-      if (!degenerate) {
-        if (binned_range_ok(absmax)) {
-          res_candidate_sums(sm, n, absmax, p.Nc, L, p.bits);
-        } else {
-          // extreme magnitudes (outside [2^-40, 2^40]): plain evaluation of every (element, candidate) pair
-          const ClipGrid g = make_clip_grid(absmax, p.Nc);
-          const double unit_inv = fixed_point_unit_inv((double)n, absmax);
-          for (int c = t; c < p.Nc; c += kThreads) {
-            const float s = scale_of(clip_candidate(g, c), L);
-            double tot = 0.0;
-            for (int e = 0; e < n; ++e) tot += (double)sqerr_exact(sub_rn(sm.Hls[e], sm.U[e]), s, L);
-            sm.acc[c] = (unsigned long long)__double2ll_rn(tot * unit_inv);
-          }
-          __syncthreads();
-        }
-        // first index of the smallest MSE (torch.argmin)
-        const double unit = fixed_point_unit((double)n, absmax);
-        const float nf = (float)n;
-        unsigned long long best = ~0ull;
-        for (int c = t; c < p.Nc; c += kThreads) {
-          const float mse = mse_from_fixed((long long)sm.acc[c], unit, nf);
-          best = min(best, ((unsigned long long)float_key(mse) << 32) | (unsigned int)c);
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) best = min(best, __shfl_xor_sync(0xffffffffu, best, o));
-        if (lane == 0) sm.best[warp] = best;
-        __syncthreads();
-        unsigned long long b = sm.best[0];
-#pragma unroll
-        for (int w = 1; w < kWarps; ++w) b = min(b, sm.best[w]);
-        rep.best_index = (int)(b & 0xffffffffu);
-        qp.scale = scale_of(clip_candidate(make_clip_grid(absmax, p.Nc), rep.best_index), L);
-      }
-    } else {
-      degenerate = (absmax != absmax) || isinf(absmax);
-      qp = params_from_minmax(p.scheme, p.bits, tmin, tmax, L);
+    QParams qp = pj.qp;
+    if (p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC && !pj.degenerate) {
+      smem_candidate_sums(sm, n, [&](int e) { return sub_rn(sm.Hls[e], sm.U[e]); }, pj.absmax, p.Nc, 0, p.Nc, L, p.bits);
+      rep.best_index = cta_best_candidate<false>(sm.acc, p.Nc, pj.absmax, (double)n, sm.best);
+      qp.scale = clip_scale(pj.absmax, p.Nc, rep.best_index, L);
     }
     rep.scale = qp.scale;
-    lap(1);
+    rb.lap(1);
     // ---------------- P3: H = Q(V), U += H - H_ls, residual sums, next RHS
     __syncthreads();  // everyone is done with X as the sorted array
-    float f0 = 0.0f, f1 = 0.0f, f2 = 0.0f, f3 = 0.0f;
-    double sums[4] = {0.0, 0.0, 0.0, 0.0};
-    int cnt = 0;
+    ResidualSums res;
     for (int e0 = t; e0 < n; e0 += kThreads * 4) {
       float hp[4], fv[4];
 #pragma unroll
@@ -389,46 +159,23 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_resident(const Reside
       for (int b = 0; b < 4; ++b) {
         const int e = e0 + b * kThreads;
         if (e < n) {
-          const float hls = sm.Hls[e], u = sm.U[e];
-          const float v = sub_rn(hls, u);
-          float code = 0.0f;
-          const float hq = degenerate ? qnan : quantize_value(v, qp, L, code);   // H = Q(H_ls - U)   (:59)
-          const float d1 = sub_rn(hq, hls);
-          const float un = add_rn(u, d1);                                        // U += H - H_ls     (:60)
-          const float d2 = sub_rn(hq, hp[b]);
-          f0 = fmaf(d1, d1, f0);  // sum (H - H_ls)^2     (:62)
-          f1 = fmaf(hq, hq, f1);  // sum H^2
-          f2 = fmaf(d2, d2, f2);  // sum (H - H_prev)^2   (:63)
-          f3 = fmaf(un, un, f3);  // sum U^2
-          p.H[e] = hq;
-          sm.U[e] = un;
-          sm.X[e] = add_rn(fv[b], mul_rn(rho, add_rn(hq, un)));
-          if (p.codes != nullptr) p.codes[e] = (int8_t)code;
-          if (++cnt == 16) {
-            sums[0] += (double)f0;
-            sums[1] += (double)f1;
-            sums[2] += (double)f2;
-            sums[3] += (double)f3;
-            f0 = f1 = f2 = f3 = 0.0f;
-            cnt = 0;
-          }
+          const ElementStep o = p3_element(sm.Hls[e], sm.U[e], hp[b], fv[b], rho, qp, L, pj.degenerate, res);
+          p.H[e] = o.hq;
+          sm.U[e] = o.un;
+          sm.X[e] = o.rhs_next;
+          if (p.codes != nullptr) p.codes[e] = (int8_t)o.code;
         }
       }
     }
-    sums[0] += (double)f0;
-    sums[1] += (double)f1;
-    sums[2] += (double)f2;
-    sums[3] += (double)f3;
-    if (degenerate) {  // uniform: the reference would carry NaN through every remaining iteration
-      rep.status |= ADMMQ_ST_NONFINITE;
-      rep.r = qnan;
-      rep.s = qnan;
+    res.flush();
+    if (pj.degenerate) {  // uniform
+      rb.nonfinite();
       break;
     }
-    res_sum4(sums, sm);  // (contains the barriers that publish U and X for the next iteration)
-    rep.r = div_rn((float)sums[0], (float)sums[1]);
-    rep.s = div_rn((float)sums[2], (float)sums[3]);
-    lap(2);
+    cta_sum4(res.sums, sm);  // (contains the barriers that publish U and X for the next iteration)
+    rep.r = div_rn((float)res.sums[0], (float)res.sums[1]);
+    rep.s = div_rn((float)res.sums[2], (float)res.sums[3]);
+    rb.lap(2);
     if (rep.r < p.eps && rep.s < p.eps) {
       rep.status |= ADMMQ_ST_CONVERGED;
       break;
@@ -436,8 +183,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_resident(const Reside
   }
   __syncthreads();
   for (int e = t; e < n; e += kThreads) p.U[e] = sm.U[e];
-  rep.phase_ns[3] = global_ns() - t_begin;
-  if (t == 0) *p.report = rep;
+  rb.finish(p.report, t == 0);
 }
 
 inline bool resident_fits(int I, int R, int Rp, int num_attempts) {

@@ -18,6 +18,7 @@
 // Same float32 recipe as the general kernel's column-strip product up to the order of the k-slices.
 #pragma once
 #include <cstddef>
+#include "admm_loop_common.cuh"
 #include "admm_loop_cluster.cuh"
 
 namespace admmq {
@@ -61,31 +62,13 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_tap(const ResidentPar
   const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
   const int I = p.I, R = p.R, Rp = p.Rp, n = I * R;
   const int rank = (int)cl_rank(), C = (int)cl_size();
-  admmq_loop_report rep;
-  rep.iterations = 0;
-  rep.status = 0;
-  rep.rho = *p.rho;
-  rep.scale = 0.0f;
-  rep.r = 0.0f;
-  rep.s = 0.0f;
-  rep.best_index = -1;
-  rep.absmax = 0.0f;
-  rep.phase_ns[0] = rep.phase_ns[1] = rep.phase_ns[2] = rep.phase_ns[3] = 0ull;
-  if (p.inv_status != nullptr && *p.inv_status != 0) {  // uniform over the cluster: nobody reaches a barrier
-    rep.status = *p.inv_status;
-    if (rank == 0 && t == 0) *p.report = rep;
-    return;
-  }
-  const unsigned long long t_begin = global_ns();
-  unsigned long long t_mark = t_begin;
-  auto lap = [&](int phase) {
-    const unsigned long long now = global_ns();
-    rep.phase_ns[phase] += now - t_mark;
-    t_mark = now;
-  };
+  LoopReport rb;
+  admmq_loop_report& rep = rb.rep;
+  // inv_status is uniform over the cluster: nobody reaches a barrier
+  if (!rb.begin(p.rho, p.inv_status, p.report, rank == 0 && t == 0)) return;
+  rb.start();
   const float rho = rep.rho;
   const Levels L = make_levels(p.bits);
-  const float qnan = __int_as_float(0x7fc00000);
   // own columns [n0, n1) (a multiple of four per CTA) and own candidates [c0, c1)
   const int cps = ((R + C - 1) / C + 3) / 4 * 4;
   const int n0 = min(R, rank * cps), n1 = min(R, n0 + cps), w = n1 - n0;
@@ -95,7 +78,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_tap(const ResidentPar
   // ---- the whole right-hand side F + rho (H + U) for the first iteration (:56), own U
   for (int e = t; e < I * Rp; e += kThreads) {
     const int i = e / Rp, c = e - i * Rp;
-    sm.rhs[e] = (c < R) ? add_rn(p.F[i * R + c], mul_rn(rho, add_rn(p.H[i * R + c], p.U[i * R + c]))) : 0.0f;
+    sm.rhs[e] = (c < R) ? rhs_of(p.F[i * R + c], rho, p.H[i * R + c], p.U[i * R + c]) : 0.0f;
   }
   for (int e = t; e < own; e += kThreads) {
     const int i = e / w, c = e - i * w;
@@ -197,122 +180,52 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_tap(const ResidentPar
       kmax = max(kmax, sm.keys[rk][0]);
       kinv = max(kinv, sm.keys[rk][1]);
     }
-    lap(0);
+    rb.lap(0);
     // ---------------- P2
-    const float tmax = key_float(kmax), tmin = key_float(~kinv);
-    float absmax = fmaxf(fabsf(tmin), fabsf(tmax));
-    if (tmin != tmin || tmax != tmax) absmax = qnan;
-    rep.absmax = absmax;
+    const Projection pj = projection_from_keys(kmax, kinv, p.scheme, p.bits, L);
+    rep.absmax = pj.absmax;
     rep.iterations = j;
     done = j;
-    QParams qp;
-    qp.scheme = p.scheme;
-    qp.bits = p.bits;
-    qp.aux = 0.0f;
-    qp.n = 0.0f;
-    qp.scale = 0.0f;
-    bool degenerate = false;
-    if (p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) {
-      degenerate = !(absmax > 0.0f) || isinf(absmax);
-      if (!degenerate) {
-        if (binned_range_ok(absmax)) {
-          cl_candidate_sums(sm, n, absmax, p.Nc, c0, c1, L, p.bits);
-        } else {
-          const ClipGrid g = make_clip_grid(absmax, p.Nc);
-          const double unit_inv = fixed_point_unit_inv((double)n, absmax);
-          for (int c = c0 + t; c < c1; c += kThreads) {
-            const float s = scale_of(clip_candidate(g, c), L);
-            double tot = 0.0;
-            for (int e = 0; e < n; ++e) tot += (double)sqerr_exact(sm.Vall[e], s, L);
-            sm.acc[c] = (unsigned long long)__double2ll_rn(tot * unit_inv);
-          }
-          __syncthreads();
-        }
-        for (int c = c0 + t; c < c1; c += kThreads) {
-          const unsigned long long v = sm.acc[c];
-          for (int rk = 0; rk < C; ++rk) cl_store(cl_map(&sm.cand[c], (unsigned int)rk), v);
-        }
+    QParams qp = pj.qp;
+    const bool search = p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC && !pj.degenerate;
+    if (search) {
+      smem_candidate_sums(sm, n, [&](int e) { return sm.Vall[e]; }, pj.absmax, p.Nc, c0, c1, L, p.bits);
+      for (int c = c0 + t; c < c1; c += kThreads) {
+        const unsigned long long v = sm.acc[c];
+        for (int rk = 0; rk < C; ++rk) cl_store(cl_map(&sm.cand[c], (unsigned int)rk), v);
       }
-    } else {
-      degenerate = (absmax != absmax) || isinf(absmax);
-      qp = params_from_minmax(p.scheme, p.bits, tmin, tmax, L);
     }
     cl_sync();   // ---- barrier 2: every candidate's sum is everywhere (nobody reads V / the sorted array any more)
-    if (p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC && !degenerate) {
-      const double unit = fixed_point_unit((double)n, absmax);
-      const float nf = (float)n;
-      unsigned long long best = ~0ull;
-      for (int c = t; c < p.Nc; c += kThreads) {
-        const float mse = mse_from_fixed((long long)sm.cand[c], unit, nf);
-        best = min(best, ((unsigned long long)float_key(mse) << 32) | (unsigned int)c);
-      }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) best = min(best, __shfl_xor_sync(0xffffffffu, best, o));
-      if (lane == 0) sm.best[warp] = best;
-      __syncthreads();
-      unsigned long long b = sm.best[0];
-#pragma unroll
-      for (int wq = 1; wq < kWarps; ++wq) b = min(b, sm.best[wq]);
-      rep.best_index = (int)(b & 0xffffffffu);
-      qp.scale = scale_of(clip_candidate(make_clip_grid(absmax, p.Nc), rep.best_index), L);
+    if (search) {
+      rep.best_index = cta_best_candidate<false>(sm.cand, p.Nc, pj.absmax, (double)n, sm.best);
+      qp.scale = clip_scale(pj.absmax, p.Nc, rep.best_index, L);
     }
     rep.scale = qp.scale;
-    lap(1);
+    rb.lap(1);
     // ---------------- P3: H = Q(V), U += H - H_ls, residual sums, next RHS (to every CTA) - own columns
-    float f0 = 0.0f, f1 = 0.0f, f2 = 0.0f, f3 = 0.0f;
-    double sums[4] = {0.0, 0.0, 0.0, 0.0};
-    int cnt = 0;
+    ResidualSums res;
     for (int o = t; o < own; o += kThreads) {
       const int i = o / w, nn = o - i * w;
       const int e = i * R + n0 + nn;
       const float hp = p.H[e];
       const float fv = __ldg(p.F + e);
-      const float hls = sm.Hls[o], u = sm.U[o];
-      const float v = sub_rn(hls, u);
-      float code = 0.0f;
-      const float hq = degenerate ? qnan : quantize_value(v, qp, L, code);   // H = Q(H_ls - U)   (:59)
-      const float d1 = sub_rn(hq, hls);
-      const float un = add_rn(u, d1);                                        // U += H - H_ls     (:60)
-      const float d2 = sub_rn(hq, hp);
-      f0 = fmaf(d1, d1, f0);  // sum (H - H_ls)^2     (:62)
-      f1 = fmaf(hq, hq, f1);  // sum H^2
-      f2 = fmaf(d2, d2, f2);  // sum (H - H_prev)^2   (:63)
-      f3 = fmaf(un, un, f3);  // sum U^2
-      p.H[e] = hq;
-      sm.U[o] = un;
-      const float rnew = add_rn(fv, mul_rn(rho, add_rn(hq, un)));
-      for (int rk = 0; rk < C; ++rk) cl_store(cl_map(&sm.rhs[i * Rp + n0 + nn], (unsigned int)rk), rnew);
-      if (p.codes != nullptr) p.codes[e] = (int8_t)code;
-      if (++cnt == 16) {
-        sums[0] += (double)f0;
-        sums[1] += (double)f1;
-        sums[2] += (double)f2;
-        sums[3] += (double)f3;
-        f0 = f1 = f2 = f3 = 0.0f;
-        cnt = 0;
-      }
+      const ElementStep s = p3_element(sm.Hls[o], sm.U[o], hp, fv, rho, qp, L, pj.degenerate, res);
+      p.H[e] = s.hq;
+      sm.U[o] = s.un;
+      for (int rk = 0; rk < C; ++rk) cl_store(cl_map(&sm.rhs[i * Rp + n0 + nn], (unsigned int)rk), s.rhs_next);
+      if (p.codes != nullptr) p.codes[e] = (int8_t)s.code;
     }
-    sums[0] += (double)f0;
-    sums[1] += (double)f1;
-    sums[2] += (double)f2;
-    sums[3] += (double)f3;
-    if (degenerate) {  // uniform: the reference would carry NaN through every remaining iteration
-      rep.status |= ADMMQ_ST_NONFINITE;
-      rep.r = qnan;
-      rep.s = qnan;
+    res.flush();
+    if (pj.degenerate) {  // uniform
+      rb.nonfinite();
       break;
     }
-    cl_sum4(sums, sm);
-    if (t < 4 * C) cl_store(cl_map(&sm.slots[rank][t & 3], (unsigned int)(t >> 2)), sums[t & 3]);
+    cta_sum4(res.sums, sm);
+    if (t < 4 * C) cl_store(cl_map(&sm.slots[rank][t & 3], (unsigned int)(t >> 2)), res.total(t & 3));
     cl_sync();   // ---- barrier 3: the next right-hand side and the residual sums are everywhere
-    double tot[4] = {0.0, 0.0, 0.0, 0.0};
-    for (int rk = 0; rk < C; ++rk)
-#pragma unroll
-      for (int q = 0; q < 4; ++q) tot[q] += sm.slots[rk][q];
-    rep.r = div_rn((float)tot[0], (float)tot[1]);
-    rep.s = div_rn((float)tot[2], (float)tot[3]);
-    lap(2);
-    if (rep.r < p.eps && rep.s < p.eps) {   // exit test (:62-65), evaluated identically by every CTA
+    const bool converged = cluster_converged(sm.slots, C, p.eps, rep);
+    rb.lap(2);
+    if (converged) {
       rep.status |= ADMMQ_ST_CONVERGED;
       break;
     }
@@ -323,8 +236,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_tap(const ResidentPar
     const int i = o / w, nn = o - i * w;
     p.U[i * R + n0 + nn] = sm.U[o];
   }
-  rep.phase_ns[3] = global_ns() - t_begin;
-  if (rank == 0 && t == 0) *p.report = rep;
+  rb.finish(p.report, rank == 0 && t == 0);
 }
 
 // Eligible: few rows, everything fits the shared-memory arrays, a budget of at least one cluster - and a rank up to

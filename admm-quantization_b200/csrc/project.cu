@@ -60,7 +60,7 @@ __global__ void __launch_bounds__(kThreads) k_apply(const float* x, long long n,
                                                    const ProjectHeader* hdr, const unsigned long long* cand_sums,
                                                    const float* tmin_in, const float* tmax_in, float* xq,
                                                    int8_t* codes, float* info) {
-  __shared__ BestSmem sm;
+  __shared__ unsigned long long wkey[kWarps];
   float tmin, tmax, absmax;
   read_minmax(hdr, tmin, tmax, absmax);
   const Levels L = make_levels(bits);
@@ -76,7 +76,7 @@ __global__ void __launch_bounds__(kThreads) k_apply(const float* x, long long n,
       nan_fill = true;  // reference: scale 0 or inf/NaN -> every output NaN (SURVEY App. A.3 item 6)
       p.scale = __int_as_float(0x7fc00000);
     } else {
-      best = cta_best_candidate(cand_sums, Nc, absmax, (double)n, sm);
+      best = cta_best_candidate<true>(cand_sums, Nc, absmax, (double)n, wkey);
       p.scale = scale_of(clip_candidate(make_clip_grid(absmax, Nc), best), L);
     }
   } else {

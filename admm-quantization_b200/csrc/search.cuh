@@ -550,31 +550,28 @@ __device__ inline void cta_candidate_sums(const float* __restrict__ v, long long
     cta_candidate_sums_direct(v, e0, e1, absmax, Nc, L, n_total, cand_sums, sm.direct, opaque_neg_zero);
 }
 
-// First index of the smallest MSE (torch.argmin, source/quantization.py:141), evaluated
-// redundantly by every CTA from the global fixed-point sums.  Returns the index to all threads.
-struct BestSmem {
-  unsigned long long key[kWarps];
-};
-template <class Smem>
-__device__ inline int cta_best_candidate(const unsigned long long* cand_sums, int Nc, float absmax,
-                                         double n_total, Smem& sm) {
+// First index of the smallest MSE (torch.argmin, source/quantization.py:141), evaluated redundantly by every CTA from
+// the fixed-point sums: global sums written by other CTAs are read with __ldcg (Ldcg), sums in shared memory with plain
+// loads.  wkey is kWarps words of shared scratch that no thread may still be reading.  Returns the index to all threads.
+template <bool Ldcg>
+__device__ inline int cta_best_candidate(const unsigned long long* cand_sums, int Nc, float absmax, double n_total,
+                                         unsigned long long* wkey) {
   const double unit = fixed_point_unit(n_total, absmax);
   const float nf = (float)n_total;
   unsigned long long best = ~0ull;
   for (int c = threadIdx.x; c < Nc; c += kThreads) {
-    const long long fx = (long long)__ldcg(cand_sums + c);
+    const long long fx = (long long)(Ldcg ? __ldcg(cand_sums + c) : cand_sums[c]);
     const float mse = mse_from_fixed(fx, unit, nf);
     const unsigned long long key = ((unsigned long long)float_key(mse) << 32) | (unsigned int)c;
     best = min(best, key);
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) best = min(best, __shfl_xor_sync(0xffffffffu, best, o));
+  if ((threadIdx.x & 31) == 0) wkey[threadIdx.x >> 5] = best;
   __syncthreads();
-  if ((threadIdx.x & 31) == 0) sm.key[threadIdx.x >> 5] = best;
-  __syncthreads();
-  unsigned long long b = sm.key[0];
+  unsigned long long b = wkey[0];
 #pragma unroll
-  for (int w = 1; w < kWarps; ++w) b = min(b, sm.key[w]);
+  for (int w = 1; w < kWarps; ++w) b = min(b, wkey[w]);
   return (int)(b & 0xffffffffu);
 }
 
