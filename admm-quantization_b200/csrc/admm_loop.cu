@@ -530,8 +530,9 @@ __device__ __forceinline__ void slot_totals(const double* slots, int ctas, doubl
 // TCBN = 0: P1 as float32 FFMA tiles (BM x BN, TM x TN per thread); TCBN = 16 / 32 / 64: P1 on the tensor cores;
 // TCBN = -MI: P1 for factors with at most MI rows (gemm_phase_skinny); TCBN = kDiagP1: elementwise P1 of the
 // two-block splitting (elementwise_phase); TCBN = kF64P1: float64-accumulating tiles against the float64 inverse
-// (parity mode, gemm_phase_f64).
-template <int BM, int BN, int TM, int TN, int TCBN>
+// (parity mode, gemm_phase_f64).  FP4: the E2M1 grid (tensor_mseminmax_e2m1, numerics.cuh); its instantiations run no
+// other scheme.
+template <int BM, int BN, int TM, int TN, int TCBN, bool FP4>
 __global__ void __launch_bounds__(kThreads, 1) k_admm_loop(const __grid_constant__ LoopParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   LoopSmem<BM, BN, TCBN>& sm = *reinterpret_cast<LoopSmem<BM, BN, TCBN>*>(smem_raw);
@@ -694,16 +695,16 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop(const __grid_constant
     qp.n = 0.0f;
     qp.scale = 0.0f;
     bool degenerate = false;
-    if (p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) {
+    if (clip_search_scheme<FP4>(p.scheme)) {
       degenerate = !(absmax > 0.0f) || isinf(absmax);
       if (!degenerate) {
         unsigned long long* cand = p.cand + (size_t)slot * kMaxCandidates;
-        cta_candidate_sums(p.V, e0, e1, absmax, p.Nc, L, p.bits, (double)N, cand, sm.search, p.neg_zero, kFormAuto, p.direct_below);
+        cta_candidate_sums<FP4>(p.V, e0, e1, absmax, p.Nc, L, p.bits, (double)N, cand, sm.search, p.neg_zero, kFormAuto, p.direct_below);
         bar.sync();
         lap(1);
         // ---------------- P3
         rep.best_index = cta_best_candidate<true>(cand, p.Nc, absmax, (double)N, sm.search.direct.key);
-        qp.scale = clip_scale(absmax, p.Nc, rep.best_index, L);
+        qp.scale = clip_scale<FP4>(absmax, p.Nc, rep.best_index, L);
       }
     } else {
       degenerate = (absmax != absmax) || isinf(absmax);
@@ -712,8 +713,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop(const __grid_constant
     rep.scale = qp.scale;
     // clip-search scheme: the code comes from x * (1 / scale) + magic-number rounding (numerics.cuh dev_fast, the
     // shortcut the direct search uses); the rare quotient too close to a rounding boundary is redone with the exact
-    // division, so the codes stay those of rint(fl(x / scale))
-    const bool fast_code = p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC && !degenerate;
+    // division, so the codes stay those of rint(fl(x / scale)).  The E2M1 grid takes the exact division throughout.
+    const bool fast_code = !FP4 && p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC && !degenerate;
     const float rcp_scale = fast_code ? div_rn(1.0f, qp.scale) : 0.0f;
     double sums[4] = {0.0, 0.0, 0.0, 0.0};
     {
@@ -825,6 +826,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop(const __grid_constant
                 code = copysignf(code, tq);  // rint keeps the sign of a quotient in (-0.5, 0); the magic sum returns +0
                 if (near_tie) code = code_exact(v, qp.scale, L);
                 hq = mul_rn(code, qp.scale);
+              } else if constexpr (FP4) {
+                hq = degenerate ? qnan : e2m1_quantize(v, qp.scale, code);
               } else {
                 hq = degenerate ? qnan : quantize_value(v, qp, L, code);
               }
@@ -1025,8 +1028,10 @@ static int check_loop_args(const char* who, const void* H, const void* U, const 
   if (H == nullptr || U == nullptr || F == nullptr || M == nullptr || report == nullptr || I <= 0 || R <= 0)
     return fail(ADMMQ_E_BADARG, "%s: null pointer or empty shape", who);
   if (bits < 1 || bits > 8) return fail(ADMMQ_E_BADARG, "%s: bits must be in 1..8, got %d", who, bits);
-  if (qscheme < 0 || qscheme > 3) return fail(ADMMQ_E_BADARG, "%s: unknown qscheme %d", who, qscheme);
-  if (qscheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC && (num_attempts < 1 || num_attempts > kMaxCandidates))
+  if (qscheme < 0 || qscheme > 4) return fail(ADMMQ_E_BADARG, "%s: unknown qscheme %d", who, qscheme);
+  if (qscheme == ADMMQ_Q_MSEMINMAX_E2M1 && bits != 4)
+    return fail(ADMMQ_E_BADARG, "%s: tensor_mseminmax_e2m1 needs bits = 4, got %d", who, bits);
+  if (clip_search_scheme(qscheme) && (num_attempts < 1 || num_attempts > kMaxCandidates))
     return fail(ADMMQ_E_BADARG, "%s: num_attempts must be in 1..%d", who, kMaxCandidates);
   if ((long long)I * ((R + 3) / 4 * 4) >= (1ll << 31)) return fail(ADMMQ_E_UNSUPPORTED, "%s: I * (R rounded up to 4) must be < 2^31", who);
   return ADMMQ_OK;
@@ -1079,6 +1084,39 @@ static int select_loop_kernel(int I, int R, int num_attempts, int precision, int
   }
 }
 
+// kernel function and dynamic shared memory of a general loop kernel id (not the shared-memory kernels)
+template <bool FP4>
+static void general_kernel(int kid, const void** fn, size_t* smem) {
+  switch (kid) {
+    case ADMMQ_LOOP_F64_64: *fn = (const void*)k_admm_loop<64, 64, 4, 4, kF64P1, FP4>; *smem = sizeof(LoopSmem<64, 64, kF64P1>); break;
+    case ADMMQ_LOOP_F64_32: *fn = (const void*)k_admm_loop<32, 32, 2, 2, kF64P1, FP4>; *smem = sizeof(LoopSmem<32, 32, kF64P1>); break;
+    case ADMMQ_LOOP_SKINNY9: *fn = (const void*)k_admm_loop<16, 32, 1, 2, -9, FP4>; *smem = sizeof(LoopSmem<16, 32, -9>); break;
+    case ADMMQ_LOOP_SKINNY16: *fn = (const void*)k_admm_loop<16, 32, 1, 2, -16, FP4>; *smem = sizeof(LoopSmem<16, 32, -16>); break;
+    case ADMMQ_LOOP_FFMA64: *fn = (const void*)k_admm_loop<64, 64, 4, 4, 0, FP4>; *smem = sizeof(LoopSmem<64, 64, 0>); break;
+    case ADMMQ_LOOP_FFMA32: *fn = (const void*)k_admm_loop<32, 32, 2, 2, 0, FP4>; *smem = sizeof(LoopSmem<32, 32, 0>); break;
+    case ADMMQ_LOOP_FFMA16: *fn = (const void*)k_admm_loop<16, 32, 1, 2, 0, FP4>; *smem = sizeof(LoopSmem<16, 32, 0>); break;
+    default: {  // ADMMQ_LOOP_TC + tile width
+      const int tcbn = kid - ADMMQ_LOOP_TC;
+      if (tcbn > 128) {
+        *fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 160 : 64), FP4>;
+        *smem = sizeof(LoopSmem<16, 32, (kLoopPS ? 160 : 64)>);
+      } else if (tcbn > 64) {
+        *fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 128 : 64), FP4>;
+        *smem = sizeof(LoopSmem<16, 32, (kLoopPS ? 128 : 64)>);
+      } else if (tcbn > 32) {
+        *fn = (const void*)k_admm_loop<16, 32, 1, 2, 64, FP4>;
+        *smem = sizeof(LoopSmem<16, 32, 64>);
+      } else if (tcbn > 16) {
+        *fn = (const void*)k_admm_loop<16, 32, 1, 2, 32, FP4>;
+        *smem = sizeof(LoopSmem<16, 32, 32>);
+      } else {
+        *fn = (const void*)k_admm_loop<16, 32, 1, 2, 16, FP4>;
+        *smem = sizeof(LoopSmem<16, 32, 16>);
+      }
+    }
+  }
+}
+
 // one launch of a shared-memory loop kernel on a thread-block cluster of `ctas` CTAs (the whole grid)
 static int launch_cluster(void (*kernel)(ResidentParams), int ctas, size_t smem, const ResidentParams& rp, cudaStream_t stream) {
   ADMMQ_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1105,6 +1143,7 @@ static int launch_loop(float* H, float* U, const float* F, const float* Minv, co
                        int8_t* codes, admmq_loop_report* report, char* ws, int grid, cudaStream_t stream) {
   const LoopLayout l = loop_layout(I, R, grid);
   const int kid = select_loop_kernel(I, R, num_attempts, precision, grid);
+  const bool fp4 = qscheme == ADMMQ_Q_MSEMINMAX_E2M1;
   if (kid == ADMMQ_LOOP_RESIDENT || kid == ADMMQ_LOOP_CLUSTER4 || kid == ADMMQ_LOOP_CLUSTER8 || kid == ADMMQ_LOOP_TAP) {
     ResidentParams rp;
     rp.H = H;
@@ -1120,14 +1159,18 @@ static int launch_loop(float* H, float* U, const float* F, const float* Minv, co
     rp.eps = eps;
     rp.bits = bits;
     rp.scheme = qscheme;
-    rp.Nc = (qscheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) ? num_attempts : 0;
+    rp.Nc = clip_search_scheme(qscheme) ? num_attempts : 0;
     rp.codes = codes;
     rp.report = report;
-    if (kid == ADMMQ_LOOP_TAP) return launch_cluster(k_admm_loop_tap<kTapMaxRows>, kTapCtas, sizeof(TapSmem), rp, stream);
+    if (kid == ADMMQ_LOOP_TAP)
+      return launch_cluster(fp4 ? k_admm_loop_tap<kTapMaxRows, true> : k_admm_loop_tap<kTapMaxRows, false>, kTapCtas,
+                            sizeof(TapSmem), rp, stream);
     if (kid != ADMMQ_LOOP_RESIDENT)
-      return launch_cluster(k_admm_loop_cluster, kid == ADMMQ_LOOP_CLUSTER8 ? 8 : 4, sizeof(ClusterSmem), rp, stream);
-    ADMMQ_CUDA_OK(cudaFuncSetAttribute(k_admm_loop_resident, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ResidentSmem)));
-    k_admm_loop_resident<<<1, kThreads, sizeof(ResidentSmem), stream>>>(rp);
+      return launch_cluster(fp4 ? k_admm_loop_cluster<true> : k_admm_loop_cluster<false>, kid == ADMMQ_LOOP_CLUSTER8 ? 8 : 4,
+                            sizeof(ClusterSmem), rp, stream);
+    void (*resident)(ResidentParams) = fp4 ? k_admm_loop_resident<true> : k_admm_loop_resident<false>;
+    ADMMQ_CUDA_OK(cudaFuncSetAttribute(resident, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ResidentSmem)));
+    resident<<<1, kThreads, sizeof(ResidentSmem), stream>>>(rp);
     ADMMQ_CUDA_OK(cudaGetLastError());
     count_launches(1);
     return ADMMQ_OK;
@@ -1145,7 +1188,7 @@ static int launch_loop(float* H, float* U, const float* F, const float* Minv, co
   p.eps = eps;
   p.bits = bits;
   p.scheme = qscheme;
-  p.Nc = (qscheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) ? num_attempts : 0;
+  p.Nc = clip_search_scheme(qscheme) ? num_attempts : 0;
   p.neg_zero = -0.0f;
   p.direct_below = direct_below_default();
   p.codes = codes;
@@ -1174,38 +1217,15 @@ static int launch_loop(float* H, float* U, const float* F, const float* Minv, co
     memset(&p.tm_minv_hi, 0, sizeof(CUtensorMap));
     memset(&p.tm_minv_lo, 0, sizeof(CUtensorMap));
   }
-  switch (kid) {
-    case ADMMQ_LOOP_F64_64: fn = (const void*)k_admm_loop<64, 64, 4, 4, kF64P1>; smem = sizeof(LoopSmem<64, 64, kF64P1>); break;
-    case ADMMQ_LOOP_F64_32: fn = (const void*)k_admm_loop<32, 32, 2, 2, kF64P1>; smem = sizeof(LoopSmem<32, 32, kF64P1>); break;
-    case ADMMQ_LOOP_SKINNY9: fn = (const void*)k_admm_loop<16, 32, 1, 2, -9>; smem = sizeof(LoopSmem<16, 32, -9>); break;
-    case ADMMQ_LOOP_SKINNY16: fn = (const void*)k_admm_loop<16, 32, 1, 2, -16>; smem = sizeof(LoopSmem<16, 32, -16>); break;
-    case ADMMQ_LOOP_FFMA64: fn = (const void*)k_admm_loop<64, 64, 4, 4, 0>; smem = sizeof(LoopSmem<64, 64, 0>); break;
-    case ADMMQ_LOOP_FFMA32: fn = (const void*)k_admm_loop<32, 32, 2, 2, 0>; smem = sizeof(LoopSmem<32, 32, 0>); break;
-    case ADMMQ_LOOP_FFMA16: fn = (const void*)k_admm_loop<16, 32, 1, 2, 0>; smem = sizeof(LoopSmem<16, 32, 0>); break;
-    default: {  // ADMMQ_LOOP_TC + tile width
-      const int tcbn = kid - ADMMQ_LOOP_TC;
-      p.tc_bn = tcbn;
-      if (int e = tc::make_operand_tmap(&p.tm_rhs, p.RHS, I, R, l.Rp, tc::kTileM)) return e;
-      if (int e = tc::make_operand_tmap(&p.tm_minv_hi, kLoopPS ? p.MinvHi : Minv, R, R, l.Rp, tcbn)) return e;
-      if (int e = tc::make_operand_tmap(&p.tm_minv_lo, kLoopPS ? p.MinvLo : Minv, R, R, l.Rp, tcbn)) return e;
-      if (tcbn > 128) {
-        fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 160 : 64)>;
-        smem = sizeof(LoopSmem<16, 32, (kLoopPS ? 160 : 64)>);
-      } else if (tcbn > 64) {
-        fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 128 : 64)>;
-        smem = sizeof(LoopSmem<16, 32, (kLoopPS ? 128 : 64)>);
-      } else if (tcbn > 32) {
-        fn = (const void*)k_admm_loop<16, 32, 1, 2, 64>;
-        smem = sizeof(LoopSmem<16, 32, 64>);
-      } else if (tcbn > 16) {
-        fn = (const void*)k_admm_loop<16, 32, 1, 2, 32>;
-        smem = sizeof(LoopSmem<16, 32, 32>);
-      } else {
-        fn = (const void*)k_admm_loop<16, 32, 1, 2, 16>;
-        smem = sizeof(LoopSmem<16, 32, 16>);
-      }
-    }
+  if (kid > ADMMQ_LOOP_TC) {
+    const int tcbn = kid - ADMMQ_LOOP_TC;
+    p.tc_bn = tcbn;
+    if (int e = tc::make_operand_tmap(&p.tm_rhs, p.RHS, I, R, l.Rp, tc::kTileM)) return e;
+    if (int e = tc::make_operand_tmap(&p.tm_minv_hi, kLoopPS ? p.MinvHi : Minv, R, R, l.Rp, tcbn)) return e;
+    if (int e = tc::make_operand_tmap(&p.tm_minv_lo, kLoopPS ? p.MinvLo : Minv, R, R, l.Rp, tcbn)) return e;
   }
+  if (fp4) general_kernel<true>(kid, &fn, &smem);
+  else general_kernel<false>(kid, &fn, &smem);
   ADMMQ_CUDA_OK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   ADMMQ_CUDA_OK(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, smem, stream));
   count_launches(1);
@@ -1315,7 +1335,7 @@ extern "C" int admmq_split_loop(float* H, float* U, const float* W, const float*
   p.eps = eps;
   p.bits = bits;
   p.scheme = qscheme;
-  p.Nc = (qscheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) ? num_attempts : 0;
+  p.Nc = clip_search_scheme(qscheme) ? num_attempts : 0;
   p.neg_zero = -0.0f;
   p.codes = codes;
   p.report = report;
@@ -1332,7 +1352,8 @@ extern "C" int admmq_split_loop(float* H, float* U, const float* W, const float*
   p.RHS = nullptr;
   p.Minv = nullptr;
   void* args[] = {&p};
-  const void* fn = (const void*)k_admm_loop<16, 32, 1, 2, kDiagP1>;
+  const void* fn = qscheme == ADMMQ_Q_MSEMINMAX_E2M1 ? (const void*)k_admm_loop<16, 32, 1, 2, kDiagP1, true>
+                                                    : (const void*)k_admm_loop<16, 32, 1, 2, kDiagP1, false>;
   const size_t smem = sizeof(LoopSmem<16, 32, kDiagP1>);
   ADMMQ_CUDA_OK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   ADMMQ_CUDA_OK(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, smem, stream));

@@ -57,12 +57,13 @@ struct LoopReport {
   }
 };
 
-// ---- projection parameters of an iteration from the min / max keys of V
+// ---- projection parameters of an iteration from the min / max keys of V (FP4: the E2M1 grid's instantiation)
 struct Projection {
   float tmin, tmax, absmax;
   QParams qp;       // scale still 0 for the clip search: it comes from the argmin (clip_scale)
   bool degenerate;  // no finite, non-zero range: H becomes NaN (every scheme follows the reference's NaN propagation)
 };
+template <bool FP4>
 __device__ __forceinline__ Projection projection_from_keys(unsigned int kmax, unsigned int kinv, int scheme, int bits,
                                                            const Levels& L) {
   Projection pj;
@@ -70,7 +71,7 @@ __device__ __forceinline__ Projection projection_from_keys(unsigned int kmax, un
   pj.tmin = key_float(~kinv);
   pj.absmax = fmaxf(fabsf(pj.tmin), fabsf(pj.tmax));
   if (pj.tmin != pj.tmin || pj.tmax != pj.tmax) pj.absmax = __int_as_float(0x7fc00000);
-  if (scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) {
+  if (clip_search_scheme<FP4>(scheme)) {
     pj.qp.scheme = scheme;
     pj.qp.bits = bits;
     pj.qp.aux = 0.0f;
@@ -82,11 +83,6 @@ __device__ __forceinline__ Projection projection_from_keys(unsigned int kmax, un
     pj.qp = params_from_minmax(scheme, bits, pj.tmin, pj.tmax, L);
   }
   return pj;
-}
-
-// scale of clip candidate `best` (source/quantization.py:141-144)
-__device__ __forceinline__ float clip_scale(float absmax, int Nc, int best, const Levels& L) {
-  return scale_of(clip_candidate(make_clip_grid(absmax, Nc), best), L);
 }
 
 // ---- sum over the CTA of four per-thread doubles (fixed order), result valid in every thread; sm.red is [4][kWarps]
@@ -158,12 +154,16 @@ struct ResidualSums {
 struct ElementStep {
   float hq, un, code, rhs_next;
 };
+template <bool FP4>
 __device__ __forceinline__ ElementStep p3_element(float hls, float u, float hp, float fv, float rho, const QParams& qp,
                                                   const Levels& L, bool degenerate, ResidualSums& res) {
   ElementStep o;
   const float v = sub_rn(hls, u);
   o.code = 0.0f;
-  o.hq = degenerate ? __int_as_float(0x7fc00000) : quantize_value(v, qp, L, o.code);   // H = Q(H_ls - U)   (:59)
+  if constexpr (FP4)
+    o.hq = degenerate ? __int_as_float(0x7fc00000) : e2m1_quantize(v, qp.scale, o.code);
+  else
+    o.hq = degenerate ? __int_as_float(0x7fc00000) : quantize_value(v, qp, L, o.code);   // H = Q(H_ls - U)   (:59)
   const float d1 = sub_rn(o.hq, hls);
   o.un = add_rn(u, d1);                                                                // U += H - H_ls     (:60)
   res.add(d1, o.hq, sub_rn(o.hq, hp), o.un);
@@ -176,7 +176,7 @@ __device__ __forceinline__ ElementStep p3_element(float hls, float u, float hp, 
 // one thread per (candidate, threshold) pair) or, for abs-max outside [2^-40, 2^40], the plain evaluation of every
 // (element, candidate) pair.  The per-candidate sums are integers over a fixed element order: the same bits whatever
 // the thread that adds a term.
-template <class Smem, class Value>
+template <bool FP4, class Smem, class Value>
 __device__ inline void smem_candidate_sums(Smem& sm, int n, Value value, float absmax, int Nc, int c0, int c1,
                                            const Levels L, int bits) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -184,9 +184,12 @@ __device__ inline void smem_candidate_sums(Smem& sm, int n, Value value, float a
   const double unit_inv = fixed_point_unit_inv((double)n, absmax);
   if (!binned_range_ok(absmax)) {
     for (int c = c0 + tid; c < c1; c += kThreads) {
-      const float s = scale_of(clip_candidate(g, c), L);
+      const float s = SearchGrid<FP4>::scale(clip_candidate(g, c), L);
       double tot = 0.0;
-      for (int e = 0; e < n; ++e) tot += (double)sqerr_exact(value(e), s, L);
+      for (int e = 0; e < n; ++e) {
+        const float d = SearchGrid<FP4>::dev(value(e), s, L);
+        tot += (double)mul_rn(d, d);
+      }
       sm.acc[c] = (unsigned long long)__double2ll_rn(tot * unit_inv);
     }
     __syncthreads();
@@ -194,11 +197,11 @@ __device__ inline void smem_candidate_sums(Smem& sm, int n, Value value, float a
   }
   const FixX fx = make_fix_x(absmax);
   const float bmul = div_rn((float)(kResBins / 2), absmax);
-  const int nthr = (1 << bits) - 1;
+  const int nthr = SearchGrid<FP4>::thresholds(bits);
   const int ncand = c1 - c0;
   const int npairs = ncand * nthr;
   for (int c = c0 + tid; c < c1; c += kThreads) {
-    sm.scale[c] = scale_of(clip_candidate(g, c), L);
+    sm.scale[c] = SearchGrid<FP4>::scale(clip_candidate(g, c), L);
     sm.acc[c] = 0ull;
   }
   float* sorted = sm.X;
@@ -288,8 +291,7 @@ __device__ inline void smem_candidate_sums(Smem& sm, int n, Value value, float a
     for (int p = tid; p < npairs; p += kThreads) {
       const int j = p / ncand, c = c0 + (p - j * ncand);
       const float s = sm.scale[c];
-      const float level = L.lo + (float)j;
-      const float theta = code_threshold(s, level);
+      const float theta = SearchGrid<FP4>::threshold(s, j, L);
       const int b = res_bin_of(theta, bmul);
       const unsigned int beg = b ? sm.cnt[b - 1] : 0u, end = sm.cnt[b];
       long long ps = (long long)(((unsigned long long)sm.shi[b] << 32) | sm.slo[b]);
@@ -301,8 +303,8 @@ __device__ inline void smem_candidate_sums(Smem& sm, int n, Value value, float a
           ps += fix_x(x, fx);
         }
       }
-      double term = threshold_term(s, level, cn, ps, fx.unit);
-      if (j == nthr - 1) term += closing_term(s, L.hi, (long long)n, ptot, fx.unit);
+      double term = SearchGrid<FP4>::term(s, j, L, cn, ps, fx.unit);
+      if (j == nthr - 1) term += closing_term(s, SearchGrid<FP4>::top(L), (long long)n, ptot, fx.unit);
       atomicAdd(&sm.acc[c], (unsigned long long)__double2ll_rn(term * unit_inv));
     }
   }

@@ -336,17 +336,148 @@ ADMMQ_HD float sumsq4(float a, float b, float c, float d) {
 }
 
 // contribution of threshold j of one candidate to the per-candidate sum, in float64:
-//   C (y_lo^2 - y_hi^2) - 2 P unit (y_lo - y_hi),   y_lo = fl32(level * s), y_hi = fl32((level + 1) * s)
-ADMMQ_HD double threshold_term(float scale, float level, long long count, long long psum, double xunit) {
-  const double ylo = (double)mul_rn(level, scale), yhi = (double)mul_rn(level + 1.0f, scale);
+//   C (y_lo^2 - y_hi^2) - 2 P unit (y_lo - y_hi),   y_lo = fl32(lo_level * s), y_hi = fl32(hi_level * s)
+// for the two neighbouring levels of the grid that the threshold separates
+ADMMQ_HD double threshold_term(float scale, float lo_level, float hi_level, long long count, long long psum, double xunit) {
+  const double ylo = (double)mul_rn(lo_level, scale), yhi = (double)mul_rn(hi_level, scale);
   const double d1 = ylo - yhi;
   return (double)count * (d1 * (ylo + yhi)) - 2.0 * ((double)psum * xunit) * d1;
+}
+// the integer grid: levels `level` and `level + 1`
+ADMMQ_HD double threshold_term(float scale, float level, long long count, long long psum, double xunit) {
+  return threshold_term(scale, level, level + 1.0f, count, psum, xunit);
 }
 // closing term n y_top^2 - 2 P_tot unit y_top, y_top = fl32((q - 1) * s)
 ADMMQ_HD double closing_term(float scale, float top_level, long long n, long long ptot, double xunit) {
   const double y = (double)mul_rn(top_level, scale);
   return (double)n * (y * y) - 2.0 * ((double)ptot * xunit) * y;
 }
+
+// --- the FP4 E2M1 grid (tensor_mseminmax_e2m1, ADMMQ_Q_MSEMINMAX_E2M1) ---------------------------
+// The reference has no such scheme; this is its definition (DESIGN.md 2b).  bits = 4 only.
+//   candidates  the clip grid of quantize_tensor_mse, make_clip_grid(absmax, num_attempts); scale s_c = fl(clip_c / 6)
+//   element     t = fl(x / s); the level is t rounded to the nearest of +-{0, 0.5, 1, 1.5, 2, 3, 4, 6}, ties to the
+//               even mantissa, saturating at +-6 - what cvt.rn.satfinite.e2m1x2.f32 does to t; the value is
+//               fl(level * s), -0 for a small negative t
+//   code        the 4-bit E2M1 encoding 0 .. 15: bit 3 sign, bits 2-1 exponent, bit 0 mantissa
+//   choice      the first minimum of the candidate MSEs, with the sums of the uniform search (fixed point, same argmin)
+// The 15 distinct values -6 .. 6 have 14 boundaries; their thresholds come in closed form (e2m1_threshold_mid).
+constexpr float kE2M1Magnitude[8] = {0.0f, 0.5f, 1.0f, 1.5f, 2.0f, 3.0f, 4.0f, 6.0f};   // by code & 7
+constexpr int kE2M1Thresholds = 14;
+constexpr float kE2M1Max = 6.0f;
+
+// value of a code, from its bits (no table lookup on the device): magnitude 2^(e-1) (1 + m/2) for e > 0, m/2 for e = 0
+ADMMQ_HD float e2m1_value(unsigned int code) {
+  const unsigned int i = code & 7u;
+  const unsigned int mag = i == 0u ? 0u : (i + (i == 1u ? 251u : 252u)) << 22;
+  return bits_f32(mag | ((code & 8u) << 28));
+}
+
+// round-to-nearest-even onto E2M1 with saturation, in software (the host's form of the hardware conversion; t not NaN)
+ADMMQ_HD unsigned int e2m1_round_sw(float t) {
+  const float a = fabsf(t);
+  // the boundaries are midpoints of neighbouring magnitudes; a tie goes to the even mantissa (even index)
+  unsigned int i;
+  if (a <= 0.25f) i = 0u;
+  else if (a < 0.75f) i = 1u;
+  else if (a <= 1.25f) i = 2u;
+  else if (a < 1.75f) i = 3u;
+  else if (a <= 2.5f) i = 4u;
+  else if (a < 3.5f) i = 5u;
+  else if (a <= 5.0f) i = 6u;
+  else i = 7u;
+  return i | ((f32_bits(t) >> 28) & 8u);
+}
+
+// code of a quotient t: cvt.rn.satfinite.e2m1x2.f32 on the device, e2m1_round_sw on the host
+ADMMQ_HD unsigned int e2m1_code(float t) {
+#if defined(__CUDA_ARCH__)
+  unsigned int r;
+  asm("{\n\t.reg .b8 b;\n\tcvt.rn.satfinite.e2m1x2.f32 b, %1, %1;\n\tmov.b32 %0, {b, b, b, b};\n\t}" : "=r"(r) : "f"(t));
+  return r & 15u;
+#else
+  return e2m1_round_sw(t);
+#endif
+}
+
+ADMMQ_HD float e2m1_scale_of(float clip) { return div_rn(clip, kE2M1Max); }
+
+// the element step of the definition: code and value of x on the grid of scale s (exact division)
+ADMMQ_HD float e2m1_quantize(float x, float scale, float& code) {
+  const unsigned int c = e2m1_code(div_rn(x, scale));
+  code = (float)c;
+  return mul_rn(e2m1_value(c), scale);
+}
+ADMMQ_HD float e2m1_dev(float x, float scale) {
+  float code;
+  return sub_rn(x, e2m1_quantize(x, scale, code));
+}
+
+// the 15 distinct values in ascending order, j = 0 .. 14 (-6 .. 6; j = 7 is +0), and the code of each
+ADMMQ_HD unsigned int e2m1_grid_code(int j) { return j < 7 ? (unsigned int)(15 - j) : (unsigned int)(j - 7); }
+ADMMQ_HD float e2m1_grid_level(int j) { return e2m1_value(e2m1_grid_code(j)); }
+
+// threshold j (j = 0 .. 13) separates grid values j and j + 1: the smallest float32 x with level(fl(x / s)) >= value
+// j + 1.  The boundary b = (value j + value j+1) / 2 is exact in float32; rounding onto E2M1 reaches value j + 1 for
+// t >= y*, y* = b when the tie goes up (value j + 1 has the even mantissa), else the next float above b.  From y* the
+// midpoint machinery of the integer grid applies unchanged (code_threshold_from_mid).
+ADMMQ_HD ThresholdMid e2m1_threshold_mid(int j) {
+  const float b = mul_rn(0.5f, add_rn(e2m1_grid_level(j), e2m1_grid_level(j + 1)));
+  const bool tie_up = (e2m1_grid_code(j + 1) & 1u) == 0u;
+  const float ystar = tie_up ? b : ordered_float(ordered_key(b) + 1u);
+  const float pred = ordered_float(ordered_key(ystar) - 1u);
+  ThresholdMid m;
+  m.mid = 0.5 * ((double)pred + (double)ystar);
+  m.odd = (f32_bits(ystar) & 1u) != 0u;
+  return m;
+}
+ADMMQ_HD float e2m1_threshold(float scale, int j) {
+  const ThresholdMid m = e2m1_threshold_mid(j);
+  return code_threshold_from_mid(scale, m.mid, m.odd);
+}
+// the same threshold by stepping through neighbouring floats with the exact division (reference of the definition;
+// used by the host tests)
+ADMMQ_HD bool e2m1_reaches(float x, float scale, float level) { return e2m1_value(e2m1_code(div_rn(x, scale))) >= level; }
+ADMMQ_HD float e2m1_threshold_search(float scale, int j) {
+  const float target = e2m1_grid_level(j + 1);
+  const float b = mul_rn(0.5f, add_rn(e2m1_grid_level(j), target));
+  unsigned int key = ordered_key(mul_rn(b, scale));
+  if (e2m1_reaches(ordered_float(key), scale, target)) {
+    for (int it = 0; it < 64 && e2m1_reaches(ordered_float(key - 1u), scale, target); ++it) --key;
+  } else {
+    for (int it = 0; it < 64; ++it) {
+      ++key;
+      if (e2m1_reaches(ordered_float(key), scale, target)) break;
+    }
+  }
+  return ordered_float(key);
+}
+
+// --- the grid of a clip search, a compile-time choice: the integer grid of quantize_tensor_mse (false) or E2M1 (true).
+// Threshold j separates grid levels j and j + 1; the last level closes the sum by parts.
+template <bool FP4> struct SearchGrid;
+template <> struct SearchGrid<false> {
+  static ADMMQ_HD float scale(float clip, const Levels& L) { return scale_of(clip, L); }
+  static ADMMQ_HD int thresholds(int bits) { return (1 << bits) - 1; }
+  static ADMMQ_HD ThresholdMid mid(int j, const Levels& L) { return threshold_mid(L.lo + (float)j); }
+  static ADMMQ_HD float threshold(float scale, int j, const Levels& L) { return code_threshold(scale, L.lo + (float)j); }
+  static ADMMQ_HD double term(float scale, int j, const Levels& L, long long count, long long psum, double xunit) {
+    return threshold_term(scale, L.lo + (float)j, count, psum, xunit);
+  }
+  static ADMMQ_HD float top(const Levels& L) { return L.hi; }
+  static ADMMQ_HD float dev(float x, float scale, const Levels& L) { return dev_exact(x, scale, L); }
+};
+template <> struct SearchGrid<true> {
+  static ADMMQ_HD float scale(float clip, const Levels&) { return e2m1_scale_of(clip); }
+  static ADMMQ_HD int thresholds(int) { return kE2M1Thresholds; }
+  static ADMMQ_HD ThresholdMid mid(int j, const Levels&) { return e2m1_threshold_mid(j); }
+  static ADMMQ_HD float threshold(float scale, int j, const Levels&) { return e2m1_threshold(scale, j); }
+  static ADMMQ_HD double term(float scale, int j, const Levels&, long long count, long long psum, double xunit) {
+    return threshold_term(scale, e2m1_grid_level(j), e2m1_grid_level(j + 1), count, psum, xunit);
+  }
+  static ADMMQ_HD float top(const Levels&) { return kE2M1Max; }
+  static ADMMQ_HD float dev(float x, float scale, const Levels&) { return e2m1_dev(x, scale); }
+};
 
 // --- the other tensor_* schemes ---------------------------------------------------------
 struct QParams {

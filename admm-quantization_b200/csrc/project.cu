@@ -4,7 +4,8 @@
 //
 // Three launches on the caller's stream:
 //   k_minmax_keys   min and max of x as order-preserving integer keys (atomicMax)
-//   k_mse_sums      per-candidate squared-error sums (only for tensor_mseminmax_symmetric)
+//   k_mse_sums      per-candidate squared-error sums (only for the clip-search schemes: tensor_mseminmax_symmetric and
+//                   tensor_mseminmax_e2m1)
 //   k_apply         argmin (redundantly per CTA) + quantize + codes
 // HBM traffic: x is read 2x (4x for the clip search), xq written once: 12-20 B/element.  The clip search runs in its
 // threshold form (search.cuh / numerics.cuh): O(1) work per element plus (2^bits - 1) * num_attempts thresholds per
@@ -42,6 +43,7 @@ __device__ __forceinline__ void read_minmax(const ProjectHeader* hdr, float& tmi
   if (tmin != tmin || tmax != tmax) absmax = __int_as_float(0x7fc00000);
 }
 
+template <bool FP4>
 __global__ void __launch_bounds__(kThreads) k_mse_sums(const float* x, long long n, int bits, int Nc,
                                                       const ProjectHeader* hdr, unsigned long long* cand_sums,
                                                       float neg_zero, int form) {
@@ -53,7 +55,7 @@ __global__ void __launch_bounds__(kThreads) k_mse_sums(const float* x, long long
   const Levels L = make_levels(bits);
   const long long cs = chunk_size(n, gridDim.x);
   const long long e0 = min(n, (long long)blockIdx.x * cs), e1 = min(n, e0 + cs);
-  cta_candidate_sums(x, e0, e1, absmax, Nc, L, bits, (double)n, cand_sums, sm, neg_zero, form);
+  cta_candidate_sums<FP4>(x, e0, e1, absmax, Nc, L, bits, (double)n, cand_sums, sm, neg_zero, form);
 }
 
 __global__ void __launch_bounds__(kThreads) k_apply(const float* x, long long n, int bits, int scheme, int Nc,
@@ -67,7 +69,8 @@ __global__ void __launch_bounds__(kThreads) k_apply(const float* x, long long n,
   QParams p;
   int best = -1;
   bool nan_fill = false;
-  if (scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) {
+  const bool fp4 = scheme == ADMMQ_Q_MSEMINMAX_E2M1;
+  if (clip_search_scheme(scheme)) {
     p.scheme = scheme;
     p.bits = bits;
     p.aux = 0.0f;
@@ -77,7 +80,7 @@ __global__ void __launch_bounds__(kThreads) k_apply(const float* x, long long n,
       p.scale = __int_as_float(0x7fc00000);
     } else {
       best = cta_best_candidate<true>(cand_sums, Nc, absmax, (double)n, wkey);
-      p.scale = scale_of(clip_candidate(make_clip_grid(absmax, Nc), best), L);
+      p.scale = fp4 ? clip_scale<true>(absmax, Nc, best, L) : clip_scale<false>(absmax, Nc, best, L);
     }
   } else {
     if (scheme == ADMMQ_Q_AFFINE && tmin_in != nullptr && tmax_in != nullptr) {
@@ -97,6 +100,8 @@ __global__ void __launch_bounds__(kThreads) k_apply(const float* x, long long n,
     float v;
     if (nan_fill) {
       v = __int_as_float(0x7fc00000);
+    } else if (fp4) {
+      v = e2m1_quantize(x[i], p.scale, code);
     } else {
       v = quantize_value(x[i], p, L, code);
     }
@@ -115,6 +120,12 @@ __global__ void k_sums_to_double(const unsigned long long* cand_sums, const Proj
     out[c] = (double)(long long)cand_sums[c] * unit;
 }
 
+// E2M1 codes of t by the hardware conversion (admmq_e2m1_encode)
+__global__ void k_e2m1_encode(const float* t, long long n, int8_t* codes) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+    codes[i] = (int8_t)e2m1_code(t[i]);
+}
+
 }  // namespace admmq
 
 using namespace admmq;
@@ -125,22 +136,27 @@ extern "C" size_t admmq_project_workspace_bytes(int64_t n, int num_attempts) {
   return align_up(sizeof(ProjectHeader), 256) + align_up((size_t)nc * sizeof(unsigned long long), 256);
 }
 
-static int launch_mse_sums(const float* x, int64_t n, int bits, int num_attempts, ProjectHeader* hdr,
+static int launch_mse_sums(const float* x, int64_t n, int bits, int qscheme, int num_attempts, ProjectHeader* hdr,
                            unsigned long long* cand, int form, int max_ctas, const DeviceProps& dp, cudaStream_t stream) {
   // one chunk of >= 512 elements per CTA, at most one CTA per SM
   const long long want = (n + 511) / 512;
   int g = (int)std::max<long long>(1, std::min<long long>((long long)dp.sm_count, want));
   if (max_ctas > 0) g = std::min(g, max_ctas);
-  ADMMQ_CUDA_OK(cudaFuncSetAttribute(k_mse_sums, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SearchSmem)));
-  k_mse_sums<<<g, kThreads, sizeof(SearchSmem), stream>>>(x, n, bits, num_attempts, hdr, cand, -0.0f, form);
+  auto kernel = qscheme == ADMMQ_Q_MSEMINMAX_E2M1 ? k_mse_sums<true> : k_mse_sums<false>;
+  ADMMQ_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SearchSmem)));
+  kernel<<<g, kThreads, sizeof(SearchSmem), stream>>>(x, n, bits, num_attempts, hdr, cand, -0.0f, form);
   return ADMMQ_OK;
 }
 
-extern "C" int admmq_clip_search_sums(const float* x, int64_t n, int bits, int num_attempts, int method, int max_ctas,
-                                      double* sums, void* workspace, size_t workspace_bytes, void* stream_) {
+extern "C" int admmq_clip_search_sums_scheme(const float* x, int64_t n, int bits, int qscheme, int num_attempts, int method,
+                                             int max_ctas, double* sums, void* workspace, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   if (x == nullptr || sums == nullptr || n <= 0) return fail(ADMMQ_E_BADARG, "admmq_clip_search_sums: null pointer or n <= 0");
   if (bits < 1 || bits > 8) return fail(ADMMQ_E_BADARG, "admmq_clip_search_sums: bits must be in 1..8, got %d", bits);
+  if (qscheme != ADMMQ_Q_MSEMINMAX_SYMMETRIC && qscheme != ADMMQ_Q_MSEMINMAX_E2M1)
+    return fail(ADMMQ_E_BADARG, "admmq_clip_search_sums: qscheme %d has no clip search", qscheme);
+  if (qscheme == ADMMQ_Q_MSEMINMAX_E2M1 && bits != 4)
+    return fail(ADMMQ_E_BADARG, "admmq_clip_search_sums: tensor_mseminmax_e2m1 needs bits = 4, got %d", bits);
   if (num_attempts < 1 || num_attempts > kMaxCandidates)
     return fail(ADMMQ_E_BADARG, "admmq_clip_search_sums: num_attempts must be in 1..%d", kMaxCandidates);
   if (method != 0 && method != 1) return fail(ADMMQ_E_BADARG, "admmq_clip_search_sums: method must be 0 (direct) or 1 (thresholds)");
@@ -154,10 +170,29 @@ extern "C" int admmq_clip_search_sums(const float* x, int64_t n, int bits, int n
   ADMMQ_CUDA_OK(cudaMemsetAsync(workspace, 0, admmq_project_workspace_bytes(n, num_attempts), stream));
   const int g_stream = (int)std::min<long long>((long long)dp.sm_count * 4, (n + kThreads * 4 - 1) / (kThreads * 4));
   k_minmax_keys<<<std::max(g_stream, 1), kThreads, 0, stream>>>(x, n, hdr);
-  if (int e = launch_mse_sums(x, n, bits, num_attempts, hdr, cand, method == 0 ? kFormDirect : kFormThresholds, max_ctas, dp, stream)) return e;
+  if (int e = launch_mse_sums(x, n, bits, qscheme, num_attempts, hdr, cand, method == 0 ? kFormDirect : kFormThresholds,
+                              max_ctas, dp, stream))
+    return e;
   k_sums_to_double<<<(num_attempts + 255) / 256, 256, 0, stream>>>(cand, hdr, n, num_attempts, sums);
   ADMMQ_CUDA_OK(cudaGetLastError());
   count_launches(3);
+  return ADMMQ_OK;
+}
+
+extern "C" int admmq_clip_search_sums(const float* x, int64_t n, int bits, int num_attempts, int method, int max_ctas,
+                                      double* sums, void* workspace, size_t workspace_bytes, void* stream) {
+  return admmq_clip_search_sums_scheme(x, n, bits, ADMMQ_Q_MSEMINMAX_SYMMETRIC, num_attempts, method, max_ctas, sums,
+                                       workspace, workspace_bytes, stream);
+}
+
+extern "C" int admmq_e2m1_encode(const float* t, int64_t n, int8_t* codes, void* stream_) {
+  if (t == nullptr || codes == nullptr || n <= 0) return fail(ADMMQ_E_BADARG, "admmq_e2m1_encode: null pointer or n <= 0");
+  DeviceProps dp;
+  if (int e = device_props(&dp)) return e;
+  const int g = (int)std::max<long long>(1, std::min<long long>((long long)dp.sm_count * 4, (n + 255) / 256));
+  k_e2m1_encode<<<g, 256, 0, (cudaStream_t)stream_>>>(t, n, codes);
+  ADMMQ_CUDA_OK(cudaGetLastError());
+  count_launches(1);
   return ADMMQ_OK;
 }
 
@@ -167,8 +202,10 @@ extern "C" int admmq_project(const float* x, int64_t n, int bits, int qscheme, i
   cudaStream_t stream = (cudaStream_t)stream_;
   if (x == nullptr || xq == nullptr || n <= 0) return fail(ADMMQ_E_BADARG, "admmq_project: null pointer or n <= 0");
   if (bits < 1 || bits > 8) return fail(ADMMQ_E_BADARG, "admmq_project: bits must be in 1..8, got %d", bits);
-  if (qscheme < 0 || qscheme > 3) return fail(ADMMQ_E_BADARG, "admmq_project: unknown qscheme %d", qscheme);
-  if (qscheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC && (num_attempts < 1 || num_attempts > kMaxCandidates))
+  if (qscheme < 0 || qscheme > 4) return fail(ADMMQ_E_BADARG, "admmq_project: unknown qscheme %d", qscheme);
+  if (qscheme == ADMMQ_Q_MSEMINMAX_E2M1 && bits != 4)
+    return fail(ADMMQ_E_BADARG, "admmq_project: tensor_mseminmax_e2m1 needs bits = 4, got %d", bits);
+  if (clip_search_scheme(qscheme) && (num_attempts < 1 || num_attempts > kMaxCandidates))
     return fail(ADMMQ_E_BADARG, "admmq_project: num_attempts must be in 1..%d, got %d", kMaxCandidates, num_attempts);
   if (workspace == nullptr || workspace_bytes < admmq_project_workspace_bytes(n, num_attempts) ||
       ((uintptr_t)workspace & 15) != 0)
@@ -181,12 +218,12 @@ extern "C" int admmq_project(const float* x, int64_t n, int bits, int qscheme, i
   const long long max_ctas = (long long)dp.sm_count * 4;
   const int g_stream = (int)std::min<long long>(max_ctas, (n + kThreads * 4 - 1) / (kThreads * 4));
   k_minmax_keys<<<std::max(g_stream, 1), kThreads, 0, stream>>>(x, n, hdr);
-  if (qscheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC) {
-    if (int e = launch_mse_sums(x, n, bits, num_attempts, hdr, cand, kFormAuto, 0, dp, stream)) return e;
+  if (clip_search_scheme(qscheme)) {
+    if (int e = launch_mse_sums(x, n, bits, qscheme, num_attempts, hdr, cand, kFormAuto, 0, dp, stream)) return e;
   }
   k_apply<<<std::max(g_stream, 1), kThreads, 0, stream>>>(x, n, bits, qscheme, num_attempts, hdr, cand, tmin, tmax,
                                                             xq, codes, info);
   ADMMQ_CUDA_OK(cudaGetLastError());
-  count_launches(qscheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC ? 3 : 2);
+  count_launches(clip_search_scheme(qscheme) ? 3 : 2);
   return ADMMQ_OK;
 }

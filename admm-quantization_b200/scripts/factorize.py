@@ -55,7 +55,7 @@ def parse_args(argv=None):
     parser.add_argument("--max_iter_admm", required=False, default=1000, type=int)
     parser.add_argument("--max_iter_epc", required=False, default=5000, type=int)
     parser.add_argument("--seed", required=True, type=int, help="Random seed.")
-    parser.add_argument("--qscheme", required=True, type=str, help="[tensor_mseminmax_symmetric, tensor_minmax]")
+    parser.add_argument("--qscheme", required=True, type=str, help="[tensor_mseminmax_symmetric, tensor_minmax, tensor_mseminmax_e2m1 (bits 4)]")
     # additions (defaults reproduce the reference's hard-coded values)
     parser.add_argument("--weights", default="pretrained", choices=["pretrained", "random"],
                         help="pretrained (default, what the reference loads: `resnet18(pretrained=True)`): fails loudly when the "

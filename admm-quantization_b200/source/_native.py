@@ -14,7 +14,9 @@ QSCHEME_IDS = {
     "tensor_minmax": 1,
     "tensor_symmetric": 2,
     "tensor_affine": 3,
+    "tensor_mseminmax_e2m1": 4,   # FP4 E2M1 grid, bits = 4 (include/admmq.h)
 }
+CLIP_SEARCH_SCHEMES = ("tensor_mseminmax_symmetric", "tensor_mseminmax_e2m1")   # scale from the clip search
 
 E_BADARG, E_WORKSPACE, E_CUDA, E_NOT_PD, E_UNSUPPORTED = -1, -2, -3, -4, -5
 ST_CONVERGED, ST_NONFINITE = 1, 2
@@ -56,6 +58,8 @@ def _load():
         "admmq_project_workspace_bytes": (c_sz, [c_i64, c_int]),
         "admmq_project": (c_int, [vp, c_i64, c_int, c_int, c_int, vp, vp, vp, vp, vp, vp, c_sz, vp]),
         "admmq_clip_search_sums": (c_int, [vp, c_i64, c_int, c_int, c_int, c_int, vp, vp, c_sz, vp]),
+        "admmq_clip_search_sums_scheme": (c_int, [vp, c_i64, c_int, c_int, c_int, c_int, c_int, vp, vp, c_sz, vp]),
+        "admmq_e2m1_encode": (c_int, [vp, c_i64, vp, vp]),
         "admmq_gram_hadamard": (c_int, [vp, c_int, vp, c_int, c_int, vp, vp]),
         "admmq_unfold3": (c_int, [vp, c_int, c_int, c_int, c_int, vp, vp]),
         "admmq_mttkrp_workspace_bytes": (c_sz, [c_int, c_int, c_int, c_int, c_int]),
@@ -100,7 +104,7 @@ def _load():
 
 lib = _load()
 EXPORTS = ("admmq_version admmq_last_error admmq_device_info admmq_launch_count admmq_project_workspace_bytes "
-           "admmq_project admmq_clip_search_sums admmq_admm_loop_kernel admmq_admm_loop_workspace_bytes admmq_admm_loop admmq_gemm_nt "
+           "admmq_project admmq_clip_search_sums admmq_clip_search_sums_scheme admmq_e2m1_encode admmq_admm_loop_kernel admmq_admm_loop_workspace_bytes admmq_admm_loop admmq_gemm_nt "
            "admmq_gram_hadamard admmq_unfold3 admmq_mttkrp_workspace_bytes admmq_mttkrp admmq_permute_myx "
            "admmq_mttkrp_tc_workspace_bytes admmq_mttkrp_tc admmq_mttkrp_kernel admmq_mttkrp_f64_workspace_bytes "
            "admmq_mttkrp_f64 "
@@ -228,16 +232,26 @@ def project(x, bits, qscheme, num_attempts=200, tmin=None, tmax=None, want_codes
     return out, codes, info
 
 
-def clip_search_sums(x, bits, num_attempts=200, method=1, max_ctas=0):
-    """Per-candidate sum((x - Q_c(x))**2) as float64: method 0 = direct evaluation, 1 = threshold form (parity tests)."""
+def clip_search_sums(x, bits, num_attempts=200, method=1, max_ctas=0, qscheme="tensor_mseminmax_symmetric"):
+    """Per-candidate sum((x - Q_c(x))**2) as float64: method 0 = direct evaluation, 1 = threshold form (parity tests),
+    for either clip-search scheme."""
     require_cuda(x)
     xc = f32c(x)
     n = xc.numel()
     sums = torch.empty(int(num_attempts), dtype=torch.float64, device=xc.device)
     ws = _ws(project_workspace_bytes(n, num_attempts), xc.device, None)
-    call(xc.device, lib.admmq_clip_search_sums, ptr(xc), n, int(bits), int(num_attempts), int(method), int(max_ctas), ptr(sums),
-                                     ptr(ws), ws.numel(), stream_ptr(xc.device))
+    call(xc.device, lib.admmq_clip_search_sums_scheme, ptr(xc), n, int(bits), qscheme_id(qscheme), int(num_attempts),
+         int(method), int(max_ctas), ptr(sums), ptr(ws), ws.numel(), stream_ptr(xc.device))
     return sums
+
+
+def e2m1_encode(t):
+    """E2M1 codes (int8, 0 .. 15) of float32 t by the hardware conversion cvt.rn.satfinite.e2m1x2.f32."""
+    require_cuda(t)
+    tc = f32c(t)
+    codes = torch.empty(tc.shape, dtype=torch.int8, device=tc.device)
+    call(tc.device, lib.admmq_e2m1_encode, ptr(tc), tc.numel(), ptr(codes), stream_ptr(tc.device))
+    return codes
 
 
 def gram_hadamard(U1, U2=None, out=None):

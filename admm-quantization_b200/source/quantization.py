@@ -30,13 +30,17 @@ def min_max_quantize(input, bits, min_val=None, max_val=None):
 
 def quantize_tensor(tensor, bits, qscheme, dim=None, **kwargs):
     """reference source/quantization.py:69-115: project `tensor` onto the `bits`-bit grid of `qscheme`.
-    kwargs: num_attempts (mseminmax), tmin/tmax (affine)."""
+    kwargs: num_attempts (mseminmax, mseminmax_e2m1), tmin/tmax (affine).  tensor_mseminmax_e2m1 is this project's
+    own scheme (no reference counterpart): the clip search onto the FP4 E2M1 grid, bits = 4."""
     if qscheme in _CHANNEL_SCHEMES:
         get_tensor_stats(tensor, qscheme, mode=dim)
     if qscheme not in _TENSOR_SCHEMES:
         raise NotImplementedError(qscheme)
     if qscheme == "tensor_mseminmax_symmetric":
         return quantize_tensor_mse(tensor, bits, **kwargs)
+    if qscheme == "tensor_mseminmax_e2m1":
+        out, _, _ = _native.project(tensor, bits, qscheme, num_attempts=kwargs.get("num_attempts", 200))
+        return out.reshape(tensor.shape)
     out, _, _ = _native.project(tensor, bits, qscheme, tmin=kwargs.get("tmin"), tmax=kwargs.get("tmax"))
     return out.reshape(tensor.shape)
 

@@ -252,7 +252,7 @@ class LayerSolver:
 
     def candidate_evaluations_per_sweep(self):
         it = max(self.max_iter_admm - 1, 0)
-        nc = self.num_attempts if self.qscheme == "tensor_mseminmax_symmetric" else 0
+        nc = self.num_attempts if self.qscheme in _native.CLIP_SEARCH_SCHEMES else 0
         return sum(it * nc * f.shape[0] * self.R for f in self.factors)
 
     def solve_flops_per_sweep(self):

@@ -50,6 +50,10 @@ extern "C" {
 #define ADMMQ_Q_MINMAX 1              /* 'tensor_minmax'              :110-111, :48-66  */
 #define ADMMQ_Q_SYMMETRIC 2           /* 'tensor_symmetric'           :91-95           */
 #define ADMMQ_Q_AFFINE 3              /* 'tensor_affine'              :97-106          */
+/* 'tensor_mseminmax_e2m1' (no counterpart in the reference; bits must be 4): the clip search of :118-144 onto the FP4
+ * E2M1 grid s * {+-0, 0.5, 1, 1.5, 2, 3, 4, 6}, s = clip / 6; codes are the 4-bit E2M1 encodings 0 .. 15 (bit 3 sign,
+ * bits 2-1 exponent, bit 0 mantissa), ready to pack into FP4 tensor-core operands.  Definition: DESIGN.md 2b. */
+#define ADMMQ_Q_MSEMINMAX_E2M1 4
 
 /* status bits written by the ADMM loop into admmq_loop_report.status */
 #define ADMMQ_ST_CONVERGED 1 /* r < eps and s < eps fired (source/admm.py:64-65) */
@@ -68,7 +72,7 @@ ADMMQ_API uint64_t admmq_launch_count(void);
  * and quantize_tensor_mse(x, bits, num_attempts)          source/quantization.py:118-144.
  *   x, xq       n floats (xq may alias x)
  *   codes       n int8 integer codes or NULL (mse/symmetric: clamp(rint(x/scale),-q,q-1);
- *               affine: code incl. zero point; minmax: level index - 2^(bits-1))
+ *               affine: code incl. zero point; minmax: level index - 2^(bits-1); e2m1: the E2M1 encoding 0 .. 15)
  *   info        device float[4] or NULL: {scale, zero_point or min, chosen candidate index, abs-max}
  *   tmin,tmax   only for ADMMQ_Q_AFFINE: device float scalars or NULL (= tensor min/max) (:98-101)
  */
@@ -83,6 +87,13 @@ ADMMQ_API int admmq_project(const float* x, int64_t n, int bits, int qscheme, in
  * limits the grid (the result must not depend on it).  Workspace: admmq_project_workspace_bytes(n, num_attempts). */
 ADMMQ_API int admmq_clip_search_sums(const float* x, int64_t n, int bits, int num_attempts, int method, int max_ctas,
                   double* sums, void* workspace, size_t workspace_bytes, void* stream);
+/* The same sums for either clip-search scheme: qscheme ADMMQ_Q_MSEMINMAX_SYMMETRIC (= admmq_clip_search_sums) or
+ * ADMMQ_Q_MSEMINMAX_E2M1 (bits 4; 14 thresholds per candidate in the threshold form). */
+ADMMQ_API int admmq_clip_search_sums_scheme(const float* x, int64_t n, int bits, int qscheme, int num_attempts, int method,
+                  int max_ctas, double* sums, void* workspace, size_t workspace_bytes, void* stream);
+/* E2M1 codes (0 .. 15) of n floats t by the hardware conversion cvt.rn.satfinite.e2m1x2.f32: round to nearest, ties
+ * to the even mantissa, saturating at +-6.  The projection's E2M1 codes are those of t = fl(x / scale). */
+ADMMQ_API int admmq_e2m1_encode(const float* t, int64_t n, int8_t* codes, void* stream);
 
 /* ------------------------------------------------------------------ per-sweep contractions
  * Gram-Hadamard  G = (U1^T U1) * (U2^T U2)   scripts/factorize.py:215,226,236 (3-D), :276,286 (2-D, U2 = NULL)
