@@ -530,9 +530,9 @@ __device__ __forceinline__ void slot_totals(const double* slots, int ctas, doubl
 // TCBN = 0: P1 as float32 FFMA tiles (BM x BN, TM x TN per thread); TCBN = 16 / 32 / 64: P1 on the tensor cores;
 // TCBN = -MI: P1 for factors with at most MI rows (gemm_phase_skinny); TCBN = kDiagP1: elementwise P1 of the
 // two-block splitting (elementwise_phase); TCBN = kF64P1: float64-accumulating tiles against the float64 inverse
-// (parity mode, gemm_phase_f64).  FP4: the E2M1 grid (tensor_mseminmax_e2m1, numerics.cuh); its instantiations run no
-// other scheme.
-template <int BM, int BN, int TM, int TN, int TCBN, bool FP4>
+// (parity mode, gemm_phase_f64).  G: the grid of the clip search (numerics.cuh SearchGrid); the E2M1 and FP8 / FP6
+// instantiations run no other scheme.
+template <int BM, int BN, int TM, int TN, int TCBN, Grid G>
 __global__ void __launch_bounds__(kThreads, 1) k_admm_loop(const __grid_constant__ LoopParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   LoopSmem<BM, BN, TCBN>& sm = *reinterpret_cast<LoopSmem<BM, BN, TCBN>*>(smem_raw);
@@ -577,7 +577,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop(const __grid_constant
   const long long N = (long long)p.I * R;
   const long long cs = chunk_size(N, gridDim.x);
   const long long e0 = min(N, (long long)blockIdx.x * cs), e1 = min(N, e0 + cs);
-  const Levels L = make_levels(p.bits);
+  const Levels L = make_levels(p.bits, G == kGridFP ? p.scheme : 0);
   const float qnan = __int_as_float(0x7fc00000);
   // P3 and the copies around the loop walk the working arrays (row pitch Rp) in aligned groups of four floats: groups
   // [g0, g1) belong to this CTA, thread t takes g0 + t, g0 + t + kThreads, ...  Only the last group of a row can hold
@@ -695,16 +695,16 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop(const __grid_constant
     qp.n = 0.0f;
     qp.scale = 0.0f;
     bool degenerate = false;
-    if (clip_search_scheme<FP4>(p.scheme)) {
+    if (clip_search_scheme<G>(p.scheme)) {
       degenerate = !(absmax > 0.0f) || isinf(absmax);
       if (!degenerate) {
         unsigned long long* cand = p.cand + (size_t)slot * kMaxCandidates;
-        cta_candidate_sums<FP4>(p.V, e0, e1, absmax, p.Nc, L, p.bits, (double)N, cand, sm.search, p.neg_zero, kFormAuto, p.direct_below);
+        cta_candidate_sums<G>(p.V, e0, e1, absmax, p.Nc, L, p.bits, (double)N, cand, sm.search, p.neg_zero, kFormAuto, p.direct_below);
         bar.sync();
         lap(1);
         // ---------------- P3
         rep.best_index = cta_best_candidate<true>(cand, p.Nc, absmax, (double)N, sm.search.direct.key);
-        qp.scale = clip_scale<FP4>(absmax, p.Nc, rep.best_index, L);
+        qp.scale = clip_scale<G>(absmax, p.Nc, rep.best_index, L);
       }
     } else {
       degenerate = (absmax != absmax) || isinf(absmax);
@@ -713,8 +713,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop(const __grid_constant
     rep.scale = qp.scale;
     // clip-search scheme: the code comes from x * (1 / scale) + magic-number rounding (numerics.cuh dev_fast, the
     // shortcut the direct search uses); the rare quotient too close to a rounding boundary is redone with the exact
-    // division, so the codes stay those of rint(fl(x / scale)).  The E2M1 grid takes the exact division throughout.
-    const bool fast_code = !FP4 && p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC && !degenerate;
+    // division, so the codes stay those of rint(fl(x / scale)).  The E2M1 and FP8 / FP6 grids take the exact division
+    // throughout.
+    const bool fast_code = G == kGridInt && p.scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC && !degenerate;
     const float rcp_scale = fast_code ? div_rn(1.0f, qp.scale) : 0.0f;
     double sums[4] = {0.0, 0.0, 0.0, 0.0};
     {
@@ -826,8 +827,10 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop(const __grid_constant
                 code = copysignf(code, tq);  // rint keeps the sign of a quotient in (-0.5, 0); the magic sum returns +0
                 if (near_tie) code = code_exact(v, qp.scale, L);
                 hq = mul_rn(code, qp.scale);
-              } else if constexpr (FP4) {
+              } else if constexpr (G == kGridE2M1) {
                 hq = degenerate ? qnan : e2m1_quantize(v, qp.scale, code);
+              } else if constexpr (G == kGridFP) {
+                hq = degenerate ? qnan : fp_quantize(v, qp.scale, L.fmt, code);
               } else {
                 hq = degenerate ? qnan : quantize_value(v, qp, L, code);
               }
@@ -1028,10 +1031,9 @@ static int check_loop_args(const char* who, const void* H, const void* U, const 
   if (H == nullptr || U == nullptr || F == nullptr || M == nullptr || report == nullptr || I <= 0 || R <= 0)
     return fail(ADMMQ_E_BADARG, "%s: null pointer or empty shape", who);
   if (bits < 1 || bits > 8) return fail(ADMMQ_E_BADARG, "%s: bits must be in 1..8, got %d", who, bits);
-  if (qscheme < 0 || qscheme > 4) return fail(ADMMQ_E_BADARG, "%s: unknown qscheme %d", who, qscheme);
-  if (qscheme == ADMMQ_Q_MSEMINMAX_E2M1 && bits != 4)
-    return fail(ADMMQ_E_BADARG, "%s: tensor_mseminmax_e2m1 needs bits = 4, got %d", who, bits);
-  if (clip_search_scheme(qscheme) && (num_attempts < 1 || num_attempts > kMaxCandidates))
+  if (!known_scheme(qscheme)) return fail(ADMMQ_E_BADARG, "%s: unknown qscheme %d", who, qscheme);
+  if (int e = check_scheme_bits(who, qscheme, bits)) return e;
+  if (has_clip_search(qscheme) && (num_attempts < 1 || num_attempts > kMaxCandidates))
     return fail(ADMMQ_E_BADARG, "%s: num_attempts must be in 1..%d", who, kMaxCandidates);
   if ((long long)I * ((R + 3) / 4 * 4) >= (1ll << 31)) return fail(ADMMQ_E_UNSUPPORTED, "%s: I * (R rounded up to 4) must be < 2^31", who);
   return ADMMQ_OK;
@@ -1084,33 +1086,39 @@ static int select_loop_kernel(int I, int R, int num_attempts, int precision, int
   }
 }
 
+// the instantiation of a kernel for a scheme's grid (grid_of)
+template <class F>
+static F by_grid(Grid g, F int_grid, F e2m1, F fp) {
+  return g == kGridE2M1 ? e2m1 : g == kGridFP ? fp : int_grid;
+}
+
 // kernel function and dynamic shared memory of a general loop kernel id (not the shared-memory kernels)
-template <bool FP4>
+template <Grid G>
 static void general_kernel(int kid, const void** fn, size_t* smem) {
   switch (kid) {
-    case ADMMQ_LOOP_F64_64: *fn = (const void*)k_admm_loop<64, 64, 4, 4, kF64P1, FP4>; *smem = sizeof(LoopSmem<64, 64, kF64P1>); break;
-    case ADMMQ_LOOP_F64_32: *fn = (const void*)k_admm_loop<32, 32, 2, 2, kF64P1, FP4>; *smem = sizeof(LoopSmem<32, 32, kF64P1>); break;
-    case ADMMQ_LOOP_SKINNY9: *fn = (const void*)k_admm_loop<16, 32, 1, 2, -9, FP4>; *smem = sizeof(LoopSmem<16, 32, -9>); break;
-    case ADMMQ_LOOP_SKINNY16: *fn = (const void*)k_admm_loop<16, 32, 1, 2, -16, FP4>; *smem = sizeof(LoopSmem<16, 32, -16>); break;
-    case ADMMQ_LOOP_FFMA64: *fn = (const void*)k_admm_loop<64, 64, 4, 4, 0, FP4>; *smem = sizeof(LoopSmem<64, 64, 0>); break;
-    case ADMMQ_LOOP_FFMA32: *fn = (const void*)k_admm_loop<32, 32, 2, 2, 0, FP4>; *smem = sizeof(LoopSmem<32, 32, 0>); break;
-    case ADMMQ_LOOP_FFMA16: *fn = (const void*)k_admm_loop<16, 32, 1, 2, 0, FP4>; *smem = sizeof(LoopSmem<16, 32, 0>); break;
+    case ADMMQ_LOOP_F64_64: *fn = (const void*)k_admm_loop<64, 64, 4, 4, kF64P1, G>; *smem = sizeof(LoopSmem<64, 64, kF64P1>); break;
+    case ADMMQ_LOOP_F64_32: *fn = (const void*)k_admm_loop<32, 32, 2, 2, kF64P1, G>; *smem = sizeof(LoopSmem<32, 32, kF64P1>); break;
+    case ADMMQ_LOOP_SKINNY9: *fn = (const void*)k_admm_loop<16, 32, 1, 2, -9, G>; *smem = sizeof(LoopSmem<16, 32, -9>); break;
+    case ADMMQ_LOOP_SKINNY16: *fn = (const void*)k_admm_loop<16, 32, 1, 2, -16, G>; *smem = sizeof(LoopSmem<16, 32, -16>); break;
+    case ADMMQ_LOOP_FFMA64: *fn = (const void*)k_admm_loop<64, 64, 4, 4, 0, G>; *smem = sizeof(LoopSmem<64, 64, 0>); break;
+    case ADMMQ_LOOP_FFMA32: *fn = (const void*)k_admm_loop<32, 32, 2, 2, 0, G>; *smem = sizeof(LoopSmem<32, 32, 0>); break;
+    case ADMMQ_LOOP_FFMA16: *fn = (const void*)k_admm_loop<16, 32, 1, 2, 0, G>; *smem = sizeof(LoopSmem<16, 32, 0>); break;
     default: {  // ADMMQ_LOOP_TC + tile width
       const int tcbn = kid - ADMMQ_LOOP_TC;
       if (tcbn > 128) {
-        *fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 160 : 64), FP4>;
+        *fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 160 : 64), G>;
         *smem = sizeof(LoopSmem<16, 32, (kLoopPS ? 160 : 64)>);
       } else if (tcbn > 64) {
-        *fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 128 : 64), FP4>;
+        *fn = (const void*)k_admm_loop<16, 32, 1, 2, (kLoopPS ? 128 : 64), G>;
         *smem = sizeof(LoopSmem<16, 32, (kLoopPS ? 128 : 64)>);
       } else if (tcbn > 32) {
-        *fn = (const void*)k_admm_loop<16, 32, 1, 2, 64, FP4>;
+        *fn = (const void*)k_admm_loop<16, 32, 1, 2, 64, G>;
         *smem = sizeof(LoopSmem<16, 32, 64>);
       } else if (tcbn > 16) {
-        *fn = (const void*)k_admm_loop<16, 32, 1, 2, 32, FP4>;
+        *fn = (const void*)k_admm_loop<16, 32, 1, 2, 32, G>;
         *smem = sizeof(LoopSmem<16, 32, 32>);
       } else {
-        *fn = (const void*)k_admm_loop<16, 32, 1, 2, 16, FP4>;
+        *fn = (const void*)k_admm_loop<16, 32, 1, 2, 16, G>;
         *smem = sizeof(LoopSmem<16, 32, 16>);
       }
     }
@@ -1143,7 +1151,7 @@ static int launch_loop(float* H, float* U, const float* F, const float* Minv, co
                        int8_t* codes, admmq_loop_report* report, char* ws, int grid, cudaStream_t stream) {
   const LoopLayout l = loop_layout(I, R, grid);
   const int kid = select_loop_kernel(I, R, num_attempts, precision, grid);
-  const bool fp4 = qscheme == ADMMQ_Q_MSEMINMAX_E2M1;
+  const Grid qgrid = grid_of(qscheme);
   if (kid == ADMMQ_LOOP_RESIDENT || kid == ADMMQ_LOOP_CLUSTER4 || kid == ADMMQ_LOOP_CLUSTER8 || kid == ADMMQ_LOOP_TAP) {
     ResidentParams rp;
     rp.H = H;
@@ -1159,16 +1167,18 @@ static int launch_loop(float* H, float* U, const float* F, const float* Minv, co
     rp.eps = eps;
     rp.bits = bits;
     rp.scheme = qscheme;
-    rp.Nc = clip_search_scheme(qscheme) ? num_attempts : 0;
+    rp.Nc = has_clip_search(qscheme) ? num_attempts : 0;
     rp.codes = codes;
     rp.report = report;
     if (kid == ADMMQ_LOOP_TAP)
-      return launch_cluster(fp4 ? k_admm_loop_tap<kTapMaxRows, true> : k_admm_loop_tap<kTapMaxRows, false>, kTapCtas,
-                            sizeof(TapSmem), rp, stream);
+      return launch_cluster(by_grid(qgrid, k_admm_loop_tap<kTapMaxRows, kGridInt>, k_admm_loop_tap<kTapMaxRows, kGridE2M1>,
+                                    k_admm_loop_tap<kTapMaxRows, kGridFP>),
+                            kTapCtas, sizeof(TapSmem), rp, stream);
     if (kid != ADMMQ_LOOP_RESIDENT)
-      return launch_cluster(fp4 ? k_admm_loop_cluster<true> : k_admm_loop_cluster<false>, kid == ADMMQ_LOOP_CLUSTER8 ? 8 : 4,
-                            sizeof(ClusterSmem), rp, stream);
-    void (*resident)(ResidentParams) = fp4 ? k_admm_loop_resident<true> : k_admm_loop_resident<false>;
+      return launch_cluster(by_grid(qgrid, k_admm_loop_cluster<kGridInt>, k_admm_loop_cluster<kGridE2M1>, k_admm_loop_cluster<kGridFP>),
+                            kid == ADMMQ_LOOP_CLUSTER8 ? 8 : 4, sizeof(ClusterSmem), rp, stream);
+    void (*resident)(ResidentParams) =
+        by_grid(qgrid, k_admm_loop_resident<kGridInt>, k_admm_loop_resident<kGridE2M1>, k_admm_loop_resident<kGridFP>);
     ADMMQ_CUDA_OK(cudaFuncSetAttribute(resident, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ResidentSmem)));
     resident<<<1, kThreads, sizeof(ResidentSmem), stream>>>(rp);
     ADMMQ_CUDA_OK(cudaGetLastError());
@@ -1188,7 +1198,7 @@ static int launch_loop(float* H, float* U, const float* F, const float* Minv, co
   p.eps = eps;
   p.bits = bits;
   p.scheme = qscheme;
-  p.Nc = clip_search_scheme(qscheme) ? num_attempts : 0;
+  p.Nc = has_clip_search(qscheme) ? num_attempts : 0;
   p.neg_zero = -0.0f;
   p.direct_below = direct_below_default();
   p.codes = codes;
@@ -1224,8 +1234,9 @@ static int launch_loop(float* H, float* U, const float* F, const float* Minv, co
     if (int e = tc::make_operand_tmap(&p.tm_minv_hi, kLoopPS ? p.MinvHi : Minv, R, R, l.Rp, tcbn)) return e;
     if (int e = tc::make_operand_tmap(&p.tm_minv_lo, kLoopPS ? p.MinvLo : Minv, R, R, l.Rp, tcbn)) return e;
   }
-  if (fp4) general_kernel<true>(kid, &fn, &smem);
-  else general_kernel<false>(kid, &fn, &smem);
+  if (qgrid == kGridE2M1) general_kernel<kGridE2M1>(kid, &fn, &smem);
+  else if (qgrid == kGridFP) general_kernel<kGridFP>(kid, &fn, &smem);
+  else general_kernel<kGridInt>(kid, &fn, &smem);
   ADMMQ_CUDA_OK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   ADMMQ_CUDA_OK(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, smem, stream));
   count_launches(1);
@@ -1335,7 +1346,7 @@ extern "C" int admmq_split_loop(float* H, float* U, const float* W, const float*
   p.eps = eps;
   p.bits = bits;
   p.scheme = qscheme;
-  p.Nc = clip_search_scheme(qscheme) ? num_attempts : 0;
+  p.Nc = has_clip_search(qscheme) ? num_attempts : 0;
   p.neg_zero = -0.0f;
   p.codes = codes;
   p.report = report;
@@ -1352,8 +1363,9 @@ extern "C" int admmq_split_loop(float* H, float* U, const float* W, const float*
   p.RHS = nullptr;
   p.Minv = nullptr;
   void* args[] = {&p};
-  const void* fn = qscheme == ADMMQ_Q_MSEMINMAX_E2M1 ? (const void*)k_admm_loop<16, 32, 1, 2, kDiagP1, true>
-                                                    : (const void*)k_admm_loop<16, 32, 1, 2, kDiagP1, false>;
+  const void* fn = by_grid(grid_of(qscheme), (const void*)k_admm_loop<16, 32, 1, 2, kDiagP1, kGridInt>,
+                           (const void*)k_admm_loop<16, 32, 1, 2, kDiagP1, kGridE2M1>,
+                           (const void*)k_admm_loop<16, 32, 1, 2, kDiagP1, kGridFP>);
   const size_t smem = sizeof(LoopSmem<16, 32, kDiagP1>);
   ADMMQ_CUDA_OK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   ADMMQ_CUDA_OK(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, smem, stream));

@@ -85,7 +85,7 @@ __device__ __forceinline__ void cl_store(unsigned int addr, double v) {
   asm volatile("st.shared::cluster.f64 [%0], %1;" ::"r"(addr), "d"(v) : "memory");
 }
 
-template <bool FP4>   // the E2M1 grid (tensor_mseminmax_e2m1), see numerics.cuh
+template <Grid G>   // G: the grid of the clip search (numerics.cuh SearchGrid)
 __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_cluster(const ResidentParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   ClusterSmem& sm = *reinterpret_cast<ClusterSmem*>(smem_raw);
@@ -98,7 +98,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_cluster(const Residen
   if (!rb.begin(p.rho, p.inv_status, p.report, rank == 0 && t == 0)) return;
   rb.start();
   const float rho = rep.rho;
-  const Levels L = make_levels(p.bits);
+  const Levels L = make_levels(p.bits, G == kGridFP ? p.scheme : 0);
   // own rows [i0, i1) and own candidates [c0, c1)
   const int rows_per = (I + C - 1) / C;
   const int i0 = min(I, rank * rows_per), i1 = min(I, i0 + rows_per);
@@ -181,14 +181,14 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_cluster(const Residen
     }
     rb.lap(0);
     // ---------------- P2
-    const Projection pj = projection_from_keys<FP4>(kmax, kinv, p.scheme, p.bits, L);
+    const Projection pj = projection_from_keys<G>(kmax, kinv, p.scheme, p.bits, L);
     rep.absmax = pj.absmax;
     rep.iterations = j;
     done = j;
     QParams qp = pj.qp;
-    const bool search = clip_search_scheme<FP4>(p.scheme) && !pj.degenerate;
+    const bool search = clip_search_scheme<G>(p.scheme) && !pj.degenerate;
     if (search) {
-      smem_candidate_sums<FP4>(sm, n, [&](int e) { return sm.Vall[e]; }, pj.absmax, p.Nc, c0, c1, L, p.bits);
+      smem_candidate_sums<G>(sm, n, [&](int e) { return sm.Vall[e]; }, pj.absmax, p.Nc, c0, c1, L, p.bits);
       for (int c = c0 + t; c < c1; c += kThreads) {
         const unsigned long long v = sm.acc[c];
         for (int rk = 0; rk < C; ++rk) cl_store(cl_map(&sm.cand[c], (unsigned int)rk), v);
@@ -197,7 +197,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_cluster(const Residen
     cl_sync();   // ---- barrier 2: every candidate's sum is everywhere (and nobody reads V / the sorted array any more)
     if (search) {
       rep.best_index = cta_best_candidate<false>(sm.cand, p.Nc, pj.absmax, (double)n, sm.best);
-      qp.scale = clip_scale<FP4>(pj.absmax, p.Nc, rep.best_index, L);
+      qp.scale = clip_scale<G>(pj.absmax, p.Nc, rep.best_index, L);
     }
     rep.scale = qp.scale;
     rb.lap(1);
@@ -207,7 +207,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_cluster(const Residen
       const int il = e / R, c = e - il * R;
       const float hp = p.H[e_base + e];
       const float fv = __ldg(p.F + e_base + e);
-      const ElementStep o = p3_element<FP4>(sm.Hls[e], sm.U[e], hp, fv, rho, qp, L, pj.degenerate, res);
+      const ElementStep o = p3_element<G>(sm.Hls[e], sm.U[e], hp, fv, rho, qp, L, pj.degenerate, res);
       p.H[e_base + e] = o.hq;
       sm.U[e] = o.un;
       rhs[il * Rp + c] = (double)o.rhs_next;

@@ -57,13 +57,13 @@ struct LoopReport {
   }
 };
 
-// ---- projection parameters of an iteration from the min / max keys of V (FP4: the E2M1 grid's instantiation)
+// ---- projection parameters of an iteration from the min / max keys of V (G: the grid of the instantiation)
 struct Projection {
   float tmin, tmax, absmax;
   QParams qp;       // scale still 0 for the clip search: it comes from the argmin (clip_scale)
   bool degenerate;  // no finite, non-zero range: H becomes NaN (every scheme follows the reference's NaN propagation)
 };
-template <bool FP4>
+template <Grid G>
 __device__ __forceinline__ Projection projection_from_keys(unsigned int kmax, unsigned int kinv, int scheme, int bits,
                                                            const Levels& L) {
   Projection pj;
@@ -71,7 +71,7 @@ __device__ __forceinline__ Projection projection_from_keys(unsigned int kmax, un
   pj.tmin = key_float(~kinv);
   pj.absmax = fmaxf(fabsf(pj.tmin), fabsf(pj.tmax));
   if (pj.tmin != pj.tmin || pj.tmax != pj.tmax) pj.absmax = __int_as_float(0x7fc00000);
-  if (clip_search_scheme<FP4>(scheme)) {
+  if (clip_search_scheme<G>(scheme)) {
     pj.qp.scheme = scheme;
     pj.qp.bits = bits;
     pj.qp.aux = 0.0f;
@@ -154,14 +154,16 @@ struct ResidualSums {
 struct ElementStep {
   float hq, un, code, rhs_next;
 };
-template <bool FP4>
+template <Grid G>
 __device__ __forceinline__ ElementStep p3_element(float hls, float u, float hp, float fv, float rho, const QParams& qp,
                                                   const Levels& L, bool degenerate, ResidualSums& res) {
   ElementStep o;
   const float v = sub_rn(hls, u);
   o.code = 0.0f;
-  if constexpr (FP4)
+  if constexpr (G == kGridE2M1)
     o.hq = degenerate ? __int_as_float(0x7fc00000) : e2m1_quantize(v, qp.scale, o.code);
+  else if constexpr (G == kGridFP)
+    o.hq = degenerate ? __int_as_float(0x7fc00000) : fp_quantize(v, qp.scale, L.fmt, o.code);
   else
     o.hq = degenerate ? __int_as_float(0x7fc00000) : quantize_value(v, qp, L, o.code);   // H = Q(H_ls - U)   (:59)
   const float d1 = sub_rn(o.hq, hls);
@@ -176,7 +178,7 @@ __device__ __forceinline__ ElementStep p3_element(float hls, float u, float hp, 
 // one thread per (candidate, threshold) pair) or, for abs-max outside [2^-40, 2^40], the plain evaluation of every
 // (element, candidate) pair.  The per-candidate sums are integers over a fixed element order: the same bits whatever
 // the thread that adds a term.
-template <bool FP4, class Smem, class Value>
+template <Grid G, class Smem, class Value>
 __device__ inline void smem_candidate_sums(Smem& sm, int n, Value value, float absmax, int Nc, int c0, int c1,
                                            const Levels L, int bits) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -184,10 +186,10 @@ __device__ inline void smem_candidate_sums(Smem& sm, int n, Value value, float a
   const double unit_inv = fixed_point_unit_inv((double)n, absmax);
   if (!binned_range_ok(absmax)) {
     for (int c = c0 + tid; c < c1; c += kThreads) {
-      const float s = SearchGrid<FP4>::scale(clip_candidate(g, c), L);
+      const float s = SearchGrid<G>::scale(clip_candidate(g, c), L);
       double tot = 0.0;
       for (int e = 0; e < n; ++e) {
-        const float d = SearchGrid<FP4>::dev(value(e), s, L);
+        const float d = SearchGrid<G>::dev(value(e), s, L);
         tot += (double)mul_rn(d, d);
       }
       sm.acc[c] = (unsigned long long)__double2ll_rn(tot * unit_inv);
@@ -197,11 +199,11 @@ __device__ inline void smem_candidate_sums(Smem& sm, int n, Value value, float a
   }
   const FixX fx = make_fix_x(absmax);
   const float bmul = div_rn((float)(kResBins / 2), absmax);
-  const int nthr = SearchGrid<FP4>::thresholds(bits);
+  const int nthr = SearchGrid<G>::thresholds(bits, L);
   const int ncand = c1 - c0;
   const int npairs = ncand * nthr;
   for (int c = c0 + tid; c < c1; c += kThreads) {
-    sm.scale[c] = SearchGrid<FP4>::scale(clip_candidate(g, c), L);
+    sm.scale[c] = SearchGrid<G>::scale(clip_candidate(g, c), L);
     sm.acc[c] = 0ull;
   }
   float* sorted = sm.X;
@@ -291,7 +293,7 @@ __device__ inline void smem_candidate_sums(Smem& sm, int n, Value value, float a
     for (int p = tid; p < npairs; p += kThreads) {
       const int j = p / ncand, c = c0 + (p - j * ncand);
       const float s = sm.scale[c];
-      const float theta = SearchGrid<FP4>::threshold(s, j, L);
+      const float theta = SearchGrid<G>::threshold(s, j, L);
       const int b = res_bin_of(theta, bmul);
       const unsigned int beg = b ? sm.cnt[b - 1] : 0u, end = sm.cnt[b];
       long long ps = (long long)(((unsigned long long)sm.shi[b] << 32) | sm.slo[b]);
@@ -303,8 +305,8 @@ __device__ inline void smem_candidate_sums(Smem& sm, int n, Value value, float a
           ps += fix_x(x, fx);
         }
       }
-      double term = SearchGrid<FP4>::term(s, j, L, cn, ps, fx.unit);
-      if (j == nthr - 1) term += closing_term(s, SearchGrid<FP4>::top(L), (long long)n, ptot, fx.unit);
+      double term = SearchGrid<G>::term(s, j, L, cn, ps, fx.unit);
+      if (j == nthr - 1) term += closing_term(s, SearchGrid<G>::top(L), (long long)n, ptot, fx.unit);
       atomicAdd(&sm.acc[c], (unsigned long long)__double2ll_rn(term * unit_inv));
     }
   }

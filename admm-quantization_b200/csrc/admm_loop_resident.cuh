@@ -51,7 +51,7 @@ struct __align__(16) ResidentSmem {
   unsigned long long best[kWarps];
 };
 
-template <bool FP4>   // the E2M1 grid (tensor_mseminmax_e2m1), see numerics.cuh
+template <Grid G>   // G: the grid of the clip search (numerics.cuh SearchGrid)
 __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_resident(const ResidentParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   ResidentSmem& sm = *reinterpret_cast<ResidentSmem*>(smem_raw);
@@ -62,7 +62,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_resident(const Reside
   if (!rb.begin(p.rho, p.inv_status, p.report, t == 0)) return;
   rb.start();
   const float rho = rep.rho;
-  const Levels L = make_levels(p.bits);
+  const Levels L = make_levels(p.bits, G == kGridFP ? p.scheme : 0);
   // ---- state into shared memory; RHS = F + rho (H + U) for the first iteration (:56)
   for (int e = t; e < R * Rp; e += kThreads) sm.Minv[e] = p.Minv[e];
   for (int e = t; e < n; e += kThreads) {
@@ -132,14 +132,14 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_resident(const Reside
     }
     rb.lap(0);
     // ---------------- P2
-    const Projection pj = projection_from_keys<FP4>(kmax, kinv, p.scheme, p.bits, L);
+    const Projection pj = projection_from_keys<G>(kmax, kinv, p.scheme, p.bits, L);
     rep.absmax = pj.absmax;
     rep.iterations = j;
     QParams qp = pj.qp;
-    if (clip_search_scheme<FP4>(p.scheme) && !pj.degenerate) {
-      smem_candidate_sums<FP4>(sm, n, [&](int e) { return sub_rn(sm.Hls[e], sm.U[e]); }, pj.absmax, p.Nc, 0, p.Nc, L, p.bits);
+    if (clip_search_scheme<G>(p.scheme) && !pj.degenerate) {
+      smem_candidate_sums<G>(sm, n, [&](int e) { return sub_rn(sm.Hls[e], sm.U[e]); }, pj.absmax, p.Nc, 0, p.Nc, L, p.bits);
       rep.best_index = cta_best_candidate<false>(sm.acc, p.Nc, pj.absmax, (double)n, sm.best);
-      qp.scale = clip_scale<FP4>(pj.absmax, p.Nc, rep.best_index, L);
+      qp.scale = clip_scale<G>(pj.absmax, p.Nc, rep.best_index, L);
     }
     rep.scale = qp.scale;
     rb.lap(1);
@@ -160,7 +160,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_resident(const Reside
       for (int b = 0; b < 4; ++b) {
         const int e = e0 + b * kThreads;
         if (e < n) {
-          const ElementStep o = p3_element<FP4>(sm.Hls[e], sm.U[e], hp[b], fv[b], rho, qp, L, pj.degenerate, res);
+          const ElementStep o = p3_element<G>(sm.Hls[e], sm.U[e], hp[b], fv[b], rho, qp, L, pj.degenerate, res);
           p.H[e] = o.hq;
           sm.U[e] = o.un;
           sm.X[e] = o.rhs_next;

@@ -55,7 +55,7 @@ static_assert((size_t)kThreads * kTapMaxRows * 4 * sizeof(float) <= sizeof(float
 static_assert(offsetof(TapSmem, cnt) == offsetof(TapSmem, X) + sizeof(float) * kTapMaxElems &&
               offsetof(TapSmem, shi) == offsetof(TapSmem, cnt) + 2 * sizeof(unsigned int) * kResBins, "X, cnt, slo, shi are contiguous");
 
-template <int MI, bool FP4>   // FP4: the E2M1 grid (tensor_mseminmax_e2m1), see numerics.cuh
+template <int MI, Grid G>   // G: the grid of the clip search (numerics.cuh SearchGrid)
 __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_tap(const ResidentParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   TapSmem& sm = *reinterpret_cast<TapSmem*>(smem_raw);
@@ -68,7 +68,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_tap(const ResidentPar
   if (!rb.begin(p.rho, p.inv_status, p.report, rank == 0 && t == 0)) return;
   rb.start();
   const float rho = rep.rho;
-  const Levels L = make_levels(p.bits);
+  const Levels L = make_levels(p.bits, G == kGridFP ? p.scheme : 0);
   // own columns [n0, n1) (a multiple of four per CTA) and own candidates [c0, c1)
   const int cps = ((R + C - 1) / C + 3) / 4 * 4;
   const int n0 = min(R, rank * cps), n1 = min(R, n0 + cps), w = n1 - n0;
@@ -182,14 +182,14 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_tap(const ResidentPar
     }
     rb.lap(0);
     // ---------------- P2
-    const Projection pj = projection_from_keys<FP4>(kmax, kinv, p.scheme, p.bits, L);
+    const Projection pj = projection_from_keys<G>(kmax, kinv, p.scheme, p.bits, L);
     rep.absmax = pj.absmax;
     rep.iterations = j;
     done = j;
     QParams qp = pj.qp;
-    const bool search = clip_search_scheme<FP4>(p.scheme) && !pj.degenerate;
+    const bool search = clip_search_scheme<G>(p.scheme) && !pj.degenerate;
     if (search) {
-      smem_candidate_sums<FP4>(sm, n, [&](int e) { return sm.Vall[e]; }, pj.absmax, p.Nc, c0, c1, L, p.bits);
+      smem_candidate_sums<G>(sm, n, [&](int e) { return sm.Vall[e]; }, pj.absmax, p.Nc, c0, c1, L, p.bits);
       for (int c = c0 + t; c < c1; c += kThreads) {
         const unsigned long long v = sm.acc[c];
         for (int rk = 0; rk < C; ++rk) cl_store(cl_map(&sm.cand[c], (unsigned int)rk), v);
@@ -198,7 +198,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_tap(const ResidentPar
     cl_sync();   // ---- barrier 2: every candidate's sum is everywhere (nobody reads V / the sorted array any more)
     if (search) {
       rep.best_index = cta_best_candidate<false>(sm.cand, p.Nc, pj.absmax, (double)n, sm.best);
-      qp.scale = clip_scale<FP4>(pj.absmax, p.Nc, rep.best_index, L);
+      qp.scale = clip_scale<G>(pj.absmax, p.Nc, rep.best_index, L);
     }
     rep.scale = qp.scale;
     rb.lap(1);
@@ -209,7 +209,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_admm_loop_tap(const ResidentPar
       const int e = i * R + n0 + nn;
       const float hp = p.H[e];
       const float fv = __ldg(p.F + e);
-      const ElementStep s = p3_element<FP4>(sm.Hls[o], sm.U[o], hp, fv, rho, qp, L, pj.degenerate, res);
+      const ElementStep s = p3_element<G>(sm.Hls[o], sm.U[o], hp, fv, rho, qp, L, pj.degenerate, res);
       p.H[e] = s.hq;
       sm.U[o] = s.un;
       for (int rk = 0; rk < C; ++rk) cl_store(cl_map(&sm.rhs[i * Rp + n0 + nn], (unsigned int)rk), s.rhs_next);

@@ -32,6 +32,35 @@ int device_props(DeviceProps* out);
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// ---- the quantization schemes as the entry points check them (include/admmq.h)
+// the width a scheme requires and its name: the E2M1 and FP8 / FP6 grids have one; 0 for the reference's schemes
+inline int scheme_bits(int scheme, const char** name) {
+  switch (scheme) {
+    case ADMMQ_Q_MSEMINMAX_E2M1: *name = "tensor_mseminmax_e2m1"; return 4;
+    case ADMMQ_Q_MSEMINMAX_E4M3: *name = "tensor_mseminmax_e4m3"; return 8;
+    case ADMMQ_Q_MSEMINMAX_E5M2: *name = "tensor_mseminmax_e5m2"; return 8;
+    case ADMMQ_Q_MSEMINMAX_E3M2: *name = "tensor_mseminmax_e3m2"; return 6;
+    case ADMMQ_Q_MSEMINMAX_E2M3: *name = "tensor_mseminmax_e2m3"; return 6;
+    default: *name = nullptr; return 0;
+  }
+}
+inline bool known_scheme(int scheme) {
+  const char* name;
+  return (scheme >= ADMMQ_Q_MSEMINMAX_SYMMETRIC && scheme <= ADMMQ_Q_AFFINE) || scheme_bits(scheme, &name) != 0;
+}
+// the scale comes from the clip search: tensor_mseminmax_symmetric and every fixed-width grid
+inline bool has_clip_search(int scheme) {
+  const char* name;
+  return scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC || scheme_bits(scheme, &name) != 0;
+}
+// ADMMQ_OK, or the failure for a width the scheme does not take
+inline int check_scheme_bits(const char* who, int scheme, int bits) {
+  const char* name;
+  const int want = scheme_bits(scheme, &name);
+  if (want != 0 && bits != want) return fail(ADMMQ_E_BADARG, "%s: %s needs bits = %d, got %d", who, name, want, bits);
+  return ADMMQ_OK;
+}
+
 #if defined(__CUDACC__)
 // ---- device-wide barrier for cooperative (co-resident) grids ----------------------------
 // Monotonic ticket counter in global memory: barrier k completes when the counter reaches

@@ -79,9 +79,8 @@ static int check_params(const char* who, int ndim, const int* shape, int R, cons
   if (R <= 0) return fail(ADMMQ_E_BADARG, "%s: rank must be positive", who);
   if (p->max_iter_als < 1 || p->max_iter_admm < 1) return fail(ADMMQ_E_BADARG, "%s: iteration budgets must be >= 1", who);
   if (p->bits < 1 || p->bits > 8) return fail(ADMMQ_E_BADARG, "%s: bits must be in 1..8", who);
-  if (p->qscheme < 0 || p->qscheme > 4) return fail(ADMMQ_E_BADARG, "%s: unknown qscheme %d", who, p->qscheme);
-  if (p->qscheme == ADMMQ_Q_MSEMINMAX_E2M1 && p->bits != 4)
-    return fail(ADMMQ_E_BADARG, "%s: tensor_mseminmax_e2m1 needs bits = 4, got %d", who, p->bits);
+  if (!known_scheme(p->qscheme)) return fail(ADMMQ_E_BADARG, "%s: unknown qscheme %d", who, p->qscheme);
+  if (int e = check_scheme_bits(who, p->qscheme, p->bits)) return e;
   if (p->solve_precision < 0 || p->solve_precision > 2 || p->mttkrp_precision < 0 || p->mttkrp_precision > 1)
     return fail(ADMMQ_E_BADARG, "%s: solve_precision must be 0..2, mttkrp_precision 0 or 1", who);
   return ADMMQ_OK;

@@ -72,10 +72,12 @@ struct Levels {
   float hi;     //  q-1
   float denom;  //  2q-1         (:89 scale_denom)
   float fast_lo, fast_hi, fast_thr;  // fast-path clamp window and "too close to .5" threshold
+  int fmt;      // the FP8 / FP6 format of the clip search (kFmtE4M3 .. kFmtE2M3), 0 on every other grid
 };
 
-ADMMQ_HD Levels make_levels(int bits) {
+ADMMQ_HD Levels make_levels(int bits, int fmt = 0) {
   Levels L;
+  L.fmt = fmt;
   const float q = (float)(1 << (bits - 1));
   L.lo = -q;
   L.hi = q - 1.0f;
@@ -453,12 +455,190 @@ ADMMQ_HD float e2m1_threshold_search(float scale, int j) {
   return ordered_float(key);
 }
 
-// --- the grid of a clip search, a compile-time choice: the integer grid of quantize_tensor_mse (false) or E2M1 (true).
-// Threshold j separates grid levels j and j + 1; the last level closes the sum by parts.
-template <bool FP4> struct SearchGrid;
-template <> struct SearchGrid<false> {
+// --- the FP8 (E4M3, E5M2) and FP6 (E3M2, E2M3) grids (tensor_mseminmax_e4m3 / _e5m2 / _e3m2 / _e2m3) ----------------
+// The reference has no such schemes; this is their definition (DESIGN.md 2c), the E2M1 definition with another value set:
+//   candidates  make_clip_grid(absmax, num_attempts); scale s_c = fl(clip_c / max)
+//   element     t = fl(x / s); the level is t rounded to the nearest value of the format, ties to the even mantissa,
+//               saturating at +-max, subnormals included - what cvt.rn.satfinite.<fmt>x2.f32 does to t; the value is
+//               fl(level * s), -0 for a small negative t
+//   code        the format's encoding: for FP8 the byte itself (int8 storage of float8_e4m3fn / float8_e5m2), for FP6
+//               0 .. 63 (bit 5 sign, then the exponent bits, then the mantissa bits)
+//   choice      the first minimum of the candidate MSEs, with the sums of the uniform search (fixed point, same argmin)
+// A non-finite abs-max takes the NONFINITE path first, as on the integer grid; a NaN element that still reaches the
+// element step takes -max, as on the integer grid (fp_quantize).
+// The format is a run-time value (the scheme id): one instantiation of every kernel serves all four.
+constexpr int kFmtE4M3 = 6, kFmtE5M2 = 7, kFmtE3M2 = 8, kFmtE2M3 = 9;   // = ADMMQ_Q_MSEMINMAX_E4M3 .. _E2M3
+ADMMQ_HD bool fp_format_id(int fmt) { return fmt >= kFmtE4M3 && fmt <= kFmtE2M3; }
+
+struct FpFormat {
+  int bits, ebits, mbits, bias;
+  bool nan_top;   // the all-ones magnitude is NaN and the one below it is max (E4M3); otherwise max is the all-ones
+                  // magnitude (FP6) or the last one below the IEEE infinities and NaNs (E5M2)
+  int top;        // magnitude code of max: the magnitudes 0 .. top ascend with their codes
+  float max;
+};
+ADMMQ_HD FpFormat fp_format(int fmt) {
+  switch (fmt) {
+    case kFmtE4M3: return {8, 4, 3, 7, true, 126, 448.0f};
+    case kFmtE5M2: return {8, 5, 2, 15, false, 123, 57344.0f};
+    case kFmtE3M2: return {6, 3, 2, 3, false, 31, 28.0f};
+    default: return {6, 2, 3, 1, false, 31, 7.5f};   // kFmtE2M3
+  }
+}
+// distinct values -max .. max (+-0 merged into one) and the thresholds between them: 2 top + 1 and 2 top
+ADMMQ_HD int fp_thresholds(int fmt) { return 2 * fp_format(fmt).top; }
+
+// value of a finite code from its bits: subnormal m 2^(1 - bias - mbits), normal (2^mbits + m) 2^(e - bias - mbits);
+// both exact in float32
+ADMMQ_HD float fp_value(int fmt, unsigned int code) {
+  const FpFormat f = fp_format(fmt);
+  const unsigned int sign = 1u << (f.bits - 1), k = code & (sign - 1u);
+  const unsigned int e = k >> f.mbits, m = k & ((1u << f.mbits) - 1u);
+  const float ulp = bits_f32((unsigned int)(127 + (e != 0u ? (int)e : 1) - f.bias - f.mbits) << 23);
+  const float mag = mul_rn((float)(e != 0u ? (m | (1u << f.mbits)) : m), ulp);
+  return bits_f32(f32_bits(mag) | ((code & sign) != 0u ? 0x80000000u : 0u));
+}
+
+// round-to-nearest-even onto the format with saturation, in software: the definition, and the host's form of the
+// hardware conversion (t not NaN).  Between neighbouring magnitudes the boundary is their midpoint (exact in float32);
+// a tie goes to the even mantissa, which is the even magnitude code.
+ADMMQ_HD unsigned int fp_round_sw(int fmt, float t) {
+  const FpFormat f = fp_format(fmt);
+  const float a = fabsf(t);
+  unsigned int lo = 0u, hi = (unsigned int)f.top;
+  if (a >= f.max) {
+    lo = hi;   // saturation, +-inf included
+  } else {     // value(lo) <= a < value(hi)
+    while (hi - lo > 1u) {
+      const unsigned int mid = (lo + hi) >> 1;
+      if (fp_value(fmt, mid) <= a) lo = mid;
+      else hi = mid;
+    }
+    const float b = mul_rn(0.5f, add_rn(fp_value(fmt, lo), fp_value(fmt, hi)));
+    if (a > b || (a == b && (hi & 1u) == 0u)) lo = hi;
+  }
+  return lo | ((f32_bits(t) >> 31) << (f.bits - 1));
+}
+
+#if defined(__CUDA_ARCH__)
+// code and value of a quotient t by the hardware: cvt.rn.satfinite.<fmt>x2.f32, and back by cvt.rn.f16x2.<fmt>x2
+// (exact: every value of the four formats is a float16).  fmt is uniform, so the switch does not diverge.
+__device__ __forceinline__ unsigned int fp_code_hw(int fmt, float t, float& value) {
+  unsigned short h;
+  unsigned int v;
+  switch (fmt) {
+    case kFmtE4M3:
+      asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %1;" : "=h"(h) : "f"(t));
+      asm("cvt.rn.f16x2.e4m3x2 %0, %1;" : "=r"(v) : "h"(h));
+      break;
+    case kFmtE5M2:
+      asm("cvt.rn.satfinite.e5m2x2.f32 %0, %1, %1;" : "=h"(h) : "f"(t));
+      asm("cvt.rn.f16x2.e5m2x2 %0, %1;" : "=r"(v) : "h"(h));
+      break;
+    case kFmtE3M2:
+      asm("cvt.rn.satfinite.e3m2x2.f32 %0, %1, %1;" : "=h"(h) : "f"(t));
+      asm("cvt.rn.f16x2.e3m2x2 %0, %1;" : "=r"(v) : "h"(h));
+      break;
+    default:   // kFmtE2M3
+      asm("cvt.rn.satfinite.e2m3x2.f32 %0, %1, %1;" : "=h"(h) : "f"(t));
+      asm("cvt.rn.f16x2.e2m3x2 %0, %1;" : "=r"(v) : "h"(h));
+      break;
+  }
+  asm("cvt.f32.f16 %0, %1;" : "=f"(value) : "h"((unsigned short)(v & 0xffffu)));
+  return (unsigned int)h & 0xffu;   // FP6: the 6-bit code in the low bits of its byte, the two above it zero
+}
+#endif
+
+// code of a quotient t: the hardware conversion on the device, fp_round_sw on the host
+ADMMQ_HD unsigned int fp_code(int fmt, float t) {
+#if defined(__CUDA_ARCH__)
+  float value;
+  return fp_code_hw(fmt, t, value);
+#else
+  return fp_round_sw(fmt, t);
+#endif
+}
+
+ADMMQ_HD float fp_scale_of(float clip, int fmt) { return div_rn(clip, fp_format(fmt).max); }
+
+// the element step of the definition: code and value of x on the grid of scale s (exact division).  The code is kept
+// as the signed value of its byte, so that the int8 store of the kernels writes the byte.  The quotient is clamped to
+// +-max first: for a finite or infinite t that is what the saturating conversion does anyway, and a NaN quotient becomes
+// -max, the level the integer grid's clamp gives it (code_exact).  A NaN that reaches the element step without making
+// the abs-max NaN (a NaN in the loop's input H does) so ends up in the same places on every grid, and the conversion of
+// a NaN, NaN for FP8 and some finite code for FP6, decides nothing.
+ADMMQ_HD float fp_quantize(float x, float scale, int fmt, float& code) {
+  const float max = fp_format(fmt).max;
+  const float t = fminf(fmaxf(div_rn(x, scale), -max), max);
+#if defined(__CUDA_ARCH__)
+  float level;
+  const unsigned int c = fp_code_hw(fmt, t, level);
+#else
+  const unsigned int c = fp_round_sw(fmt, t);
+  const float level = fp_value(fmt, c);
+#endif
+  code = (float)(int)(signed char)c;
+  return mul_rn(level, scale);
+}
+ADMMQ_HD float fp_dev(float x, float scale, int fmt) {
+  float code;
+  return sub_rn(x, fp_quantize(x, scale, fmt, code));
+}
+
+// the 2 top + 1 distinct values in ascending order, j = 0 .. 2 top (j = top is +0), and the code of each
+ADMMQ_HD unsigned int fp_grid_code(int fmt, int j) {
+  const FpFormat f = fp_format(fmt);
+  return j < f.top ? (1u << (f.bits - 1)) | (unsigned int)(f.top - j) : (unsigned int)(j - f.top);
+}
+ADMMQ_HD float fp_grid_level(int fmt, int j) { return fp_value(fmt, fp_grid_code(fmt, j)); }
+
+// threshold j (j = 0 .. 2 top - 1) separates grid values j and j + 1, exactly as for E2M1 (e2m1_threshold_mid): the
+// boundary b is their midpoint, exact in float32 (at most 3 mantissa bits); rounding reaches value j + 1 from y* = b
+// when the tie goes up (value j + 1 has the even mantissa, also across a binade, and 0 against the smallest
+// subnormal), else from the next float above b.
+ADMMQ_HD ThresholdMid fp_threshold_mid(int fmt, int j) {
+  const float b = mul_rn(0.5f, add_rn(fp_grid_level(fmt, j), fp_grid_level(fmt, j + 1)));
+  const bool tie_up = (fp_grid_code(fmt, j + 1) & 1u) == 0u;
+  const float ystar = tie_up ? b : ordered_float(ordered_key(b) + 1u);
+  const float pred = ordered_float(ordered_key(ystar) - 1u);
+  ThresholdMid m;
+  m.mid = 0.5 * ((double)pred + (double)ystar);
+  m.odd = (f32_bits(ystar) & 1u) != 0u;
+  return m;
+}
+ADMMQ_HD float fp_threshold(float scale, int fmt, int j) {
+  const ThresholdMid m = fp_threshold_mid(fmt, j);
+  return code_threshold_from_mid(scale, m.mid, m.odd);
+}
+// the same threshold by stepping through neighbouring floats with the exact division (reference of the definition;
+// used by the host tests)
+ADMMQ_HD bool fp_reaches(float x, float scale, int fmt, float level) {
+  return fp_value(fmt, fp_code(fmt, div_rn(x, scale))) >= level;
+}
+ADMMQ_HD float fp_threshold_search(float scale, int fmt, int j) {
+  const float target = fp_grid_level(fmt, j + 1);
+  const float b = mul_rn(0.5f, add_rn(fp_grid_level(fmt, j), target));
+  unsigned int key = ordered_key(mul_rn(b, scale));
+  if (fp_reaches(ordered_float(key), scale, fmt, target)) {
+    for (int it = 0; it < 64 && fp_reaches(ordered_float(key - 1u), scale, fmt, target); ++it) --key;
+  } else {
+    for (int it = 0; it < 64; ++it) {
+      ++key;
+      if (fp_reaches(ordered_float(key), scale, fmt, target)) break;
+    }
+  }
+  return ordered_float(key);
+}
+
+// --- the grid of a clip search, a compile-time choice: the integer grid of quantize_tensor_mse, E2M1, or the FP8 / FP6
+// grids (the format in Levels::fmt).  Threshold j separates grid levels j and j + 1; the last level closes the sum by
+// parts.
+// The parameter is an int so that false / true still name the integer and the E2M1 grid.
+enum Grid : int { kGridInt = 0, kGridE2M1 = 1, kGridFP = 2 };
+template <int G> struct SearchGrid;
+template <> struct SearchGrid<kGridInt> {
   static ADMMQ_HD float scale(float clip, const Levels& L) { return scale_of(clip, L); }
-  static ADMMQ_HD int thresholds(int bits) { return (1 << bits) - 1; }
+  static ADMMQ_HD int thresholds(int bits, const Levels&) { return (1 << bits) - 1; }
   static ADMMQ_HD ThresholdMid mid(int j, const Levels& L) { return threshold_mid(L.lo + (float)j); }
   static ADMMQ_HD float threshold(float scale, int j, const Levels& L) { return code_threshold(scale, L.lo + (float)j); }
   static ADMMQ_HD double term(float scale, int j, const Levels& L, long long count, long long psum, double xunit) {
@@ -467,9 +647,9 @@ template <> struct SearchGrid<false> {
   static ADMMQ_HD float top(const Levels& L) { return L.hi; }
   static ADMMQ_HD float dev(float x, float scale, const Levels& L) { return dev_exact(x, scale, L); }
 };
-template <> struct SearchGrid<true> {
+template <> struct SearchGrid<kGridE2M1> {
   static ADMMQ_HD float scale(float clip, const Levels&) { return e2m1_scale_of(clip); }
-  static ADMMQ_HD int thresholds(int) { return kE2M1Thresholds; }
+  static ADMMQ_HD int thresholds(int, const Levels&) { return kE2M1Thresholds; }
   static ADMMQ_HD ThresholdMid mid(int j, const Levels&) { return e2m1_threshold_mid(j); }
   static ADMMQ_HD float threshold(float scale, int j, const Levels&) { return e2m1_threshold(scale, j); }
   static ADMMQ_HD double term(float scale, int j, const Levels&, long long count, long long psum, double xunit) {
@@ -477,6 +657,17 @@ template <> struct SearchGrid<true> {
   }
   static ADMMQ_HD float top(const Levels&) { return kE2M1Max; }
   static ADMMQ_HD float dev(float x, float scale, const Levels&) { return e2m1_dev(x, scale); }
+};
+template <> struct SearchGrid<kGridFP> {
+  static ADMMQ_HD float scale(float clip, const Levels& L) { return fp_scale_of(clip, L.fmt); }
+  static ADMMQ_HD int thresholds(int, const Levels& L) { return fp_thresholds(L.fmt); }
+  static ADMMQ_HD ThresholdMid mid(int j, const Levels& L) { return fp_threshold_mid(L.fmt, j); }
+  static ADMMQ_HD float threshold(float scale, int j, const Levels& L) { return fp_threshold(scale, L.fmt, j); }
+  static ADMMQ_HD double term(float scale, int j, const Levels& L, long long count, long long psum, double xunit) {
+    return threshold_term(scale, fp_grid_level(L.fmt, j), fp_grid_level(L.fmt, j + 1), count, psum, xunit);
+  }
+  static ADMMQ_HD float top(const Levels& L) { return fp_format(L.fmt).max; }
+  static ADMMQ_HD float dev(float x, float scale, const Levels& L) { return fp_dev(x, scale, L.fmt); }
 };
 
 // --- the other tensor_* schemes ---------------------------------------------------------

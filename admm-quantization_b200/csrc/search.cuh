@@ -136,9 +136,9 @@ __device__ __forceinline__ void eval_pair(f32x2 x, f32x2 s, f32x2 rc, const Leve
 }
 
 // Adds this CTA's share of sum_e (x_e - Q_c(x_e))^2 for every candidate c < Nc into
-// cand_sums[c] (fixed point, see numerics.cuh).  The CTA's elements are v[e0 .. e1) (contiguous).  On the E2M1 grid
-// (FP4) every element takes the exact division; the summation recipe is the same.
-template <bool FP4 = false>
+// cand_sums[c] (fixed point, see numerics.cuh).  The CTA's elements are v[e0 .. e1) (contiguous).  On the E2M1 and the
+// FP8 / FP6 grids every element takes the exact division; the summation recipe is the same.
+template <Grid G = kGridInt>
 __device__ inline void cta_candidate_sums_direct(const float* __restrict__ v, long long e0, long long e1, float absmax,
                                                  int Nc, const Levels L, double n_total, unsigned long long* cand_sums,
                                                  DirectSmem& sm, float opaque_neg_zero) {
@@ -178,7 +178,7 @@ __device__ inline void cta_candidate_sums_direct(const float* __restrict__ v, lo
 #pragma unroll
     for (int j = 0; j < kCPL; ++j) {
       const int c = c0 + j * 32 + lane;
-      const float s = (c < Nc) ? SearchGrid<FP4>::scale(clip_candidate(g, c), L) : 1.0f;
+      const float s = (c < Nc) ? SearchGrid<G>::scale(clip_candidate(g, c), L) : 1.0f;
       const float r = (c < Nc) ? div_rn(1.0f, s) : 0.0f;
       sc[j] = pack2(s, s);
       rc[j] = pack2(r, r);
@@ -211,7 +211,7 @@ __device__ inline void cta_candidate_sums_direct(const float* __restrict__ v, lo
         const f32x2 xs[4] = {va.x, va.y, vb.x, vb.y};
         f32x2 acc[kCPL];
         float worst = 0.0f;
-        if constexpr (!FP4) {
+        if constexpr (G == kGridInt) {
 #pragma unroll
           for (int j = 0; j < kCPL; ++j) {
             acc[j] = 0ull;  // (+0.0f, +0.0f)
@@ -219,8 +219,8 @@ __device__ inline void cta_candidate_sums_direct(const float* __restrict__ v, lo
             for (int q = 0; q < 4; ++q) eval_pair(xs[q], sc[j], rc[j], L, magic, nmagic, nzero, acc[j], worst);
           }
         }
-        // integer grid, rare: a quotient too close to a rounding boundary (or non-finite); E2M1: always
-        if (FP4 || !(worst <= L.fast_thr)) {
+        // integer grid, rare: a quotient too close to a rounding boundary (or non-finite); the other grids: always
+        if (G != kGridInt || !(worst <= L.fast_thr)) {
 #pragma unroll
           for (int j = 0; j < kCPL; ++j) {
             float s0, s1, even = 0.0f, odd = 0.0f;
@@ -229,7 +229,7 @@ __device__ inline void cta_candidate_sums_direct(const float* __restrict__ v, lo
             for (int q = 0; q < 4; ++q) {
               float x0, x1;
               unpack2(xs[q], x0, x1);
-              const float d0 = SearchGrid<FP4>::dev(x0, s0, L), d1 = SearchGrid<FP4>::dev(x1, s0, L);
+              const float d0 = SearchGrid<G>::dev(x0, s0, L), d1 = SearchGrid<G>::dev(x1, s0, L);
               even = fma_rn(d0, d0, even);
               odd = fma_rn(d1, d1, odd);
             }
@@ -308,7 +308,7 @@ __device__ __forceinline__ float4 load_group4(const float* __restrict__ p, int g
   return x;
 }
 
-template <bool FP4 = false>
+template <Grid G = kGridInt>
 __device__ inline void cta_candidate_sums_binned(const float* __restrict__ v, long long e0, long long e1, float absmax,
                                                  int Nc, const Levels L, int bits, double n_total,
                                                  unsigned long long* cand_sums, BinnedSmem& sm) {
@@ -318,17 +318,17 @@ __device__ inline void cta_candidate_sums_binned(const float* __restrict__ v, lo
   const double unit_inv = fixed_point_unit_inv(n_total, absmax);
   const FixX fx = make_fix_x(absmax);
   const float bmul = div_rn((float)(kBins / 2), absmax);
-  const int nthr = SearchGrid<FP4>::thresholds(bits);  // thresholds per candidate
+  const int nthr = SearchGrid<G>::thresholds(bits, L);  // thresholds per candidate
   const int npairs = Nc * nthr;
   const bool vec_ok = ((reinterpret_cast<uintptr_t>(v + e0) & 15) == 0);
   __syncthreads();  // the previous phase is done with the shared memory
   for (int c = tid; c < Nc; c += kThreads) {
-    sm.scale[c] = SearchGrid<FP4>::scale(clip_candidate(g, c), L);
+    sm.scale[c] = SearchGrid<G>::scale(clip_candidate(g, c), L);
     sm.acc[c] = 0ull;
     sm.part[0][c] = sm.part[1][c] = sm.part[2][c] = 0u;
   }
   for (int j = tid; j < nthr; j += kThreads) {
-    const ThresholdMid tm = SearchGrid<FP4>::mid(j, L);
+    const ThresholdMid tm = SearchGrid<G>::mid(j, L);
     sm.mid[j] = tm.mid;
     sm.odd[j] = tm.odd ? 1u : 0u;
   }
@@ -504,8 +504,8 @@ __device__ inline void cta_candidate_sums_binned(const float* __restrict__ v, lo
           cn += below;
           ps += (long long)sth * 1048576ll + (long long)stl;
         }
-        double term = SearchGrid<FP4>::term(s, j, L, cn, ps, fx.unit);
-        if (j == nthr - 1) term += closing_term(s, SearchGrid<FP4>::top(L), (long long)cnt, ptot, fx.unit);
+        double term = SearchGrid<G>::term(s, j, L, cn, ps, fx.unit);
+        if (j == nthr - 1) term += closing_term(s, SearchGrid<G>::top(L), (long long)cnt, ptot, fx.unit);
         const long long f = __double2ll_rn(term * unit_inv);
         atomicAdd(&sm.part[0][c], (unsigned int)(f & 0x1fffffll));
         atomicAdd(&sm.part[1][c], (unsigned int)((f >> 21) & 0x1fffffll));
@@ -535,7 +535,7 @@ constexpr int kFormAuto = 0, kFormDirect = 1, kFormThresholds = 2;
 // ~69 ps on B200 (tools/time_search.py crossover: break-even near 5 k elements per CTA with 8 bits, 1.3 k with 6, and
 // no difference below 1 k with 4)
 constexpr int kPairsPerElement = 18;
-template <bool FP4 = false>
+template <Grid G = kGridInt>
 __device__ inline void cta_candidate_sums(const float* __restrict__ v, long long e0, long long e1, float absmax, int Nc,
                                           const Levels L, int bits, double n_total, unsigned long long* cand_sums,
                                           SearchSmem& sm, float opaque_neg_zero, int form = kFormAuto, int direct_below = 0) {
@@ -551,9 +551,9 @@ __device__ inline void cta_candidate_sums(const float* __restrict__ v, long long
   const bool direct_is_cheaper = (bits > 4 && (long long)((1 << bits) - 1) * stages * kPairsPerElement > elems) || elems <= direct_below;
   const bool want_direct = form == kFormDirect || (form == kFormAuto && direct_is_cheaper);
   if (!want_direct && binned_range_ok(absmax))
-    cta_candidate_sums_binned<FP4>(v, e0, e1, absmax, Nc, L, bits, n_total, cand_sums, sm.binned);
+    cta_candidate_sums_binned<G>(v, e0, e1, absmax, Nc, L, bits, n_total, cand_sums, sm.binned);
   else
-    cta_candidate_sums_direct<FP4>(v, e0, e1, absmax, Nc, L, n_total, cand_sums, sm.direct, opaque_neg_zero);
+    cta_candidate_sums_direct<G>(v, e0, e1, absmax, Nc, L, n_total, cand_sums, sm.direct, opaque_neg_zero);
 }
 
 // First index of the smallest MSE (torch.argmin, source/quantization.py:141), evaluated redundantly by every CTA from
@@ -581,17 +581,26 @@ __device__ inline int cta_best_candidate(const unsigned long long* cand_sums, in
   return (int)(b & 0xffffffffu);
 }
 
-// The scheme takes its scale from the clip search: quantize_tensor_mse on the integer grid or on the E2M1 grid.  A
-// kernel instantiated for the E2M1 grid (FP4) runs no other scheme.
-template <bool FP4 = false>
+static_assert(kFmtE4M3 == ADMMQ_Q_MSEMINMAX_E4M3 && kFmtE5M2 == ADMMQ_Q_MSEMINMAX_E5M2 &&
+              kFmtE3M2 == ADMMQ_Q_MSEMINMAX_E3M2 && kFmtE2M3 == ADMMQ_Q_MSEMINMAX_E2M3, "the FP format is the scheme id");
+
+// The scheme takes its scale from the clip search, in a kernel instantiated for grid G: quantize_tensor_mse on the
+// integer grid or on the E2M1 grid.  A kernel instantiated for the E2M1 or the FP8 / FP6 grids runs no other scheme;
+// the integer grid's instantiations never see an FP8 / FP6 scheme (grid_of).
+template <Grid G = kGridInt>
 __host__ __device__ __forceinline__ bool clip_search_scheme(int scheme) {
-  return FP4 || scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC || scheme == ADMMQ_Q_MSEMINMAX_E2M1;
+  return G != kGridInt || scheme == ADMMQ_Q_MSEMINMAX_SYMMETRIC || scheme == ADMMQ_Q_MSEMINMAX_E2M1;
+}
+
+// which instantiation runs a scheme (host side)
+inline Grid grid_of(int scheme) {
+  return scheme == ADMMQ_Q_MSEMINMAX_E2M1 ? kGridE2M1 : fp_format_id(scheme) ? kGridFP : kGridInt;
 }
 
 // scale of clip candidate `best` (source/quantization.py:141-144)
-template <bool FP4 = false>
+template <Grid G = kGridInt>
 __device__ __forceinline__ float clip_scale(float absmax, int Nc, int best, const Levels& L) {
-  return SearchGrid<FP4>::scale(clip_candidate(make_clip_grid(absmax, Nc), best), L);
+  return SearchGrid<G>::scale(clip_candidate(make_clip_grid(absmax, Nc), best), L);
 }
 
 // Parameters of the non-search schemes from the tensor's min / max (source/quantization.py:48-66, 91-106)

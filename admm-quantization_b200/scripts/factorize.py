@@ -55,7 +55,8 @@ def parse_args(argv=None):
     parser.add_argument("--max_iter_admm", required=False, default=1000, type=int)
     parser.add_argument("--max_iter_epc", required=False, default=5000, type=int)
     parser.add_argument("--seed", required=True, type=int, help="Random seed.")
-    parser.add_argument("--qscheme", required=True, type=str, help="[tensor_mseminmax_symmetric, tensor_minmax, tensor_mseminmax_e2m1 (bits 4)]")
+    parser.add_argument("--qscheme", required=True, type=str, help="[tensor_mseminmax_symmetric, tensor_minmax, tensor_mseminmax_e2m1 (bits 4), "
+                        "tensor_mseminmax_e4m3 / tensor_mseminmax_e5m2 (bits 8), tensor_mseminmax_e3m2 / tensor_mseminmax_e2m3 (bits 6)]")
     # additions (defaults reproduce the reference's hard-coded values)
     parser.add_argument("--weights", default="pretrained", choices=["pretrained", "random"],
                         help="pretrained (default, what the reference loads: `resnet18(pretrained=True)`): fails loudly when the "

@@ -33,7 +33,9 @@ def parse_args(argv=None):
     ap.add_argument("--model-name", default="resnet18", choices=["resnet18", "resnet50", "llama7b"])
     ap.add_argument("--bits", type=int, nargs="+", default=[4])
     ap.add_argument("--reduction-rate", type=float, nargs="+", default=[2.0])
-    ap.add_argument("--qscheme", default="tensor_mseminmax_symmetric")
+    ap.add_argument("--qscheme", default="tensor_mseminmax_symmetric",
+                    help="a tensor_* scheme; the clip search also onto FP4 (tensor_mseminmax_e2m1, bits 4), FP8 "
+                         "(tensor_mseminmax_e4m3 / _e5m2, bits 8) or FP6 (tensor_mseminmax_e3m2 / _e2m3, bits 6)")
     ap.add_argument("--init", default="random")
     ap.add_argument("--seed", type=int, default=42)
     ap.add_argument("--max_iter_als", type=int, default=5000)

@@ -15,8 +15,13 @@ QSCHEME_IDS = {
     "tensor_symmetric": 2,
     "tensor_affine": 3,
     "tensor_mseminmax_e2m1": 4,   # FP4 E2M1 grid, bits = 4 (include/admmq.h)
+    "tensor_mseminmax_e4m3": 6,   # FP8 E4M3 grid, bits = 8 (id 5 is unassigned)
+    "tensor_mseminmax_e5m2": 7,   # FP8 E5M2 grid, bits = 8
+    "tensor_mseminmax_e3m2": 8,   # FP6 E3M2 grid, bits = 6
+    "tensor_mseminmax_e2m3": 9,   # FP6 E2M3 grid, bits = 6
 }
-CLIP_SEARCH_SCHEMES = ("tensor_mseminmax_symmetric", "tensor_mseminmax_e2m1")   # scale from the clip search
+CLIP_SEARCH_SCHEMES = ("tensor_mseminmax_symmetric", "tensor_mseminmax_e2m1", "tensor_mseminmax_e4m3",
+                       "tensor_mseminmax_e5m2", "tensor_mseminmax_e3m2", "tensor_mseminmax_e2m3")   # scale from the clip search
 
 E_BADARG, E_WORKSPACE, E_CUDA, E_NOT_PD, E_UNSUPPORTED = -1, -2, -3, -4, -5
 ST_CONVERGED, ST_NONFINITE = 1, 2
@@ -60,6 +65,7 @@ def _load():
         "admmq_clip_search_sums": (c_int, [vp, c_i64, c_int, c_int, c_int, c_int, vp, vp, c_sz, vp]),
         "admmq_clip_search_sums_scheme": (c_int, [vp, c_i64, c_int, c_int, c_int, c_int, c_int, vp, vp, c_sz, vp]),
         "admmq_e2m1_encode": (c_int, [vp, c_i64, vp, vp]),
+        "admmq_fp_encode": (c_int, [vp, c_i64, c_int, vp, vp]),
         "admmq_gram_hadamard": (c_int, [vp, c_int, vp, c_int, c_int, vp, vp]),
         "admmq_unfold3": (c_int, [vp, c_int, c_int, c_int, c_int, vp, vp]),
         "admmq_mttkrp_workspace_bytes": (c_sz, [c_int, c_int, c_int, c_int, c_int]),
@@ -104,7 +110,7 @@ def _load():
 
 lib = _load()
 EXPORTS = ("admmq_version admmq_last_error admmq_device_info admmq_launch_count admmq_project_workspace_bytes "
-           "admmq_project admmq_clip_search_sums admmq_clip_search_sums_scheme admmq_e2m1_encode admmq_admm_loop_kernel admmq_admm_loop_workspace_bytes admmq_admm_loop admmq_gemm_nt "
+           "admmq_project admmq_clip_search_sums admmq_clip_search_sums_scheme admmq_e2m1_encode admmq_fp_encode admmq_admm_loop_kernel admmq_admm_loop_workspace_bytes admmq_admm_loop admmq_gemm_nt "
            "admmq_gram_hadamard admmq_unfold3 admmq_mttkrp_workspace_bytes admmq_mttkrp admmq_permute_myx "
            "admmq_mttkrp_tc_workspace_bytes admmq_mttkrp_tc admmq_mttkrp_kernel admmq_mttkrp_f64_workspace_bytes "
            "admmq_mttkrp_f64 "
@@ -234,7 +240,7 @@ def project(x, bits, qscheme, num_attempts=200, tmin=None, tmax=None, want_codes
 
 def clip_search_sums(x, bits, num_attempts=200, method=1, max_ctas=0, qscheme="tensor_mseminmax_symmetric"):
     """Per-candidate sum((x - Q_c(x))**2) as float64: method 0 = direct evaluation, 1 = threshold form (parity tests),
-    for either clip-search scheme."""
+    for any clip-search scheme."""
     require_cuda(x)
     xc = f32c(x)
     n = xc.numel()
@@ -251,6 +257,16 @@ def e2m1_encode(t):
     tc = f32c(t)
     codes = torch.empty(tc.shape, dtype=torch.int8, device=tc.device)
     call(tc.device, lib.admmq_e2m1_encode, ptr(tc), tc.numel(), ptr(codes), stream_ptr(tc.device))
+    return codes
+
+
+def fp_encode(t, qscheme):
+    """FP8 / FP6 codes (int8) of float32 t by the hardware conversion cvt.rn.satfinite.<fmt>x2.f32 for one of the
+    schemes tensor_mseminmax_e4m3 / _e5m2 / _e3m2 / _e2m3: the FP8 byte, or the FP6 encoding 0 .. 63."""
+    require_cuda(t)
+    tc = f32c(t)
+    codes = torch.empty(tc.shape, dtype=torch.int8, device=tc.device)
+    call(tc.device, lib.admmq_fp_encode, ptr(tc), tc.numel(), qscheme_id(qscheme), ptr(codes), stream_ptr(tc.device))
     return codes
 
 

@@ -54,6 +54,14 @@ extern "C" {
  * E2M1 grid s * {+-0, 0.5, 1, 1.5, 2, 3, 4, 6}, s = clip / 6; codes are the 4-bit E2M1 encodings 0 .. 15 (bit 3 sign,
  * bits 2-1 exponent, bit 0 mantissa), ready to pack into FP4 tensor-core operands.  Definition: DESIGN.md 2b. */
 #define ADMMQ_Q_MSEMINMAX_E2M1 4
+/* (id 5 is unassigned.)  The same clip search onto the FP8 and FP6 grids that tcgen05.mma kind::f8f6f4 reads, no
+ * counterpart in the reference either: s * (every finite value of the format), s = clip / max, each with a fixed width.
+ * Codes are the format's encodings: for FP8 the byte itself (a float8_e4m3fn / float8_e5m2 tensor viewed as int8), for
+ * FP6 0 .. 63 (bit 5 sign, then the exponent bits, then the mantissa bits).  Definition: DESIGN.md 2c. */
+#define ADMMQ_Q_MSEMINMAX_E4M3 6 /* 'tensor_mseminmax_e4m3'  bits 8, max 448   */
+#define ADMMQ_Q_MSEMINMAX_E5M2 7 /* 'tensor_mseminmax_e5m2'  bits 8, max 57344 */
+#define ADMMQ_Q_MSEMINMAX_E3M2 8 /* 'tensor_mseminmax_e3m2'  bits 6, max 28    */
+#define ADMMQ_Q_MSEMINMAX_E2M3 9 /* 'tensor_mseminmax_e2m3'  bits 6, max 7.5   */
 
 /* status bits written by the ADMM loop into admmq_loop_report.status */
 #define ADMMQ_ST_CONVERGED 1 /* r < eps and s < eps fired (source/admm.py:64-65) */
@@ -72,7 +80,8 @@ ADMMQ_API uint64_t admmq_launch_count(void);
  * and quantize_tensor_mse(x, bits, num_attempts)          source/quantization.py:118-144.
  *   x, xq       n floats (xq may alias x)
  *   codes       n int8 integer codes or NULL (mse/symmetric: clamp(rint(x/scale),-q,q-1);
- *               affine: code incl. zero point; minmax: level index - 2^(bits-1); e2m1: the E2M1 encoding 0 .. 15)
+ *               affine: code incl. zero point; minmax: level index - 2^(bits-1); e2m1: the E2M1 encoding 0 .. 15;
+ *               e4m3 / e5m2: the FP8 byte; e3m2 / e2m3: the FP6 encoding 0 .. 63)
  *   info        device float[4] or NULL: {scale, zero_point or min, chosen candidate index, abs-max}
  *   tmin,tmax   only for ADMMQ_Q_AFFINE: device float scalars or NULL (= tensor min/max) (:98-101)
  */
@@ -87,13 +96,18 @@ ADMMQ_API int admmq_project(const float* x, int64_t n, int bits, int qscheme, in
  * limits the grid (the result must not depend on it).  Workspace: admmq_project_workspace_bytes(n, num_attempts). */
 ADMMQ_API int admmq_clip_search_sums(const float* x, int64_t n, int bits, int num_attempts, int method, int max_ctas,
                   double* sums, void* workspace, size_t workspace_bytes, void* stream);
-/* The same sums for either clip-search scheme: qscheme ADMMQ_Q_MSEMINMAX_SYMMETRIC (= admmq_clip_search_sums) or
- * ADMMQ_Q_MSEMINMAX_E2M1 (bits 4; 14 thresholds per candidate in the threshold form). */
+/* The same sums for any clip-search scheme: qscheme ADMMQ_Q_MSEMINMAX_SYMMETRIC (= admmq_clip_search_sums),
+ * ADMMQ_Q_MSEMINMAX_E2M1 (bits 4; 14 thresholds per candidate in the threshold form) or ADMMQ_Q_MSEMINMAX_E4M3 / E5M2
+ * / E3M2 / E2M3 (bits 8 / 8 / 6 / 6; 252 / 246 / 62 / 62 thresholds). */
 ADMMQ_API int admmq_clip_search_sums_scheme(const float* x, int64_t n, int bits, int qscheme, int num_attempts, int method,
                   int max_ctas, double* sums, void* workspace, size_t workspace_bytes, void* stream);
 /* E2M1 codes (0 .. 15) of n floats t by the hardware conversion cvt.rn.satfinite.e2m1x2.f32: round to nearest, ties
  * to the even mantissa, saturating at +-6.  The projection's E2M1 codes are those of t = fl(x / scale). */
 ADMMQ_API int admmq_e2m1_encode(const float* t, int64_t n, int8_t* codes, void* stream);
+/* FP8 / FP6 codes of n floats t by the hardware conversion cvt.rn.satfinite.<fmt>x2.f32 for qscheme
+ * ADMMQ_Q_MSEMINMAX_E4M3 / E5M2 / E3M2 / E2M3: round to nearest, ties to the even mantissa, saturating at +-max.  The
+ * projection's codes are those of t = fl(x / scale). */
+ADMMQ_API int admmq_fp_encode(const float* t, int64_t n, int qscheme, int8_t* codes, void* stream);
 
 /* ------------------------------------------------------------------ per-sweep contractions
  * Gram-Hadamard  G = (U1^T U1) * (U2^T U2)   scripts/factorize.py:215,226,236 (3-D), :276,286 (2-D, U2 = NULL)
