@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.dirname(HERE)
 OUT_DIR = os.path.join(PKG, "lib")
 OBJ_DIR = os.path.join(PKG, "build")
-SOURCES = ["api.cu", "project.cu", "contract.cu", "admm_loop.cu", "mttkrp_tc.cu", "tc_gemm.cu", "factorize.cu"]
+SOURCES = ["api.cu", "project.cu", "contract.cu", "admm_loop.cu", "mttkrp_tc.cu", "tc_gemm.cu", "factorize.cu", "code_gemm.cu"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
          "-Xcompiler", "-fPIC,-fvisibility=hidden", "--fmad=true", "-Xptxas", "-v"]
 

@@ -630,6 +630,38 @@ ADMMQ_HD float fp_threshold_search(float scale, int fmt, int j) {
   return ordered_float(key);
 }
 
+// --- factor codes as FP8 tensor-core operands (DESIGN.md 2d) ---------------------------------------------------------
+// The code GEMM reads a factor's codes as FP8 bytes whose value IS the grid level: E4M3 and E5M2 codes as they are, every
+// other grid widened exactly into E4M3.  That needs each level to be an E4M3 value: E2M1 (+-{0 .. 6}), E3M2 (max 28,
+// subnormals 0.0625 m) and E2M3 (max 7.5, subnormals 0.125 m) are, and so is every integer code c with |c| <= 16, i.e.
+// the integer grids of at most 5 bits (c in [-16, 15]); 17 is not, and the offset grids of tensor_affine / tensor_minmax
+// are not levels times a scale at all.
+// The FP8 format of the operand (kFmtE4M3 / kFmtE5M2) for the codes of (scheme, bits), or -1 where no exact form exists.
+// The scheme ids are those of include/admmq.h (ADMMQ_Q_*).
+ADMMQ_HD int fp8_operand_format(int scheme, int bits) {
+  switch (scheme) {
+    case 0:  // ADMMQ_Q_MSEMINMAX_SYMMETRIC
+    case 2:  // ADMMQ_Q_SYMMETRIC
+      return (bits >= 1 && bits <= 5) ? kFmtE4M3 : -1;
+    case 4: return bits == 4 ? kFmtE4M3 : -1;   // ADMMQ_Q_MSEMINMAX_E2M1
+    case kFmtE4M3: return bits == 8 ? kFmtE4M3 : -1;
+    case kFmtE5M2: return bits == 8 ? kFmtE5M2 : -1;
+    case kFmtE3M2:
+    case kFmtE2M3: return bits == 6 ? kFmtE4M3 : -1;
+    default: return -1;
+  }
+}
+// The operand byte of one code (scheme and bits accepted by fp8_operand_format).  The level is decoded exactly and
+// rounded onto E4M3, which leaves it unchanged; the sign is kept, so -0 (E2M1 / FP6 codes) becomes 0x80.
+ADMMQ_HD unsigned int code_to_fp8(int scheme, int code) {
+  if (scheme == kFmtE4M3 || scheme == kFmtE5M2) return (unsigned int)code & 0xffu;
+  float level;
+  if (scheme == 4) level = e2m1_value((unsigned int)code & 15u);
+  else if (scheme == kFmtE3M2 || scheme == kFmtE2M3) level = fp_value(scheme, (unsigned int)code & 63u);
+  else level = (float)code;
+  return fp_round_sw(kFmtE4M3, level);
+}
+
 // --- the grid of a clip search, a compile-time choice: the integer grid of quantize_tensor_mse, E2M1, or the FP8 / FP6
 // grids (the format in Levels::fmt).  Threshold j separates grid levels j and j + 1; the last level closes the sum by
 // parts.

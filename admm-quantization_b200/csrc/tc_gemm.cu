@@ -7,7 +7,8 @@
 namespace admmq {
 
 namespace tc {
-int make_operand_tmap(CUtensorMap* out, const float* base, int rows, int cols, int ld, int box_rows) {
+int make_tmap_2d(CUtensorMap* out, CUtensorMapDataType dtype, const void* base, int rows, int cols, size_t ld_bytes,
+                 int box_cols, int box_rows) {
   typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -21,14 +22,18 @@ int make_operand_tmap(CUtensorMap* out, const float* base, int rows, int cols, i
     encode = (EncodeFn)fn;
   }
   const cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  const cuuint64_t gstride[1] = {(cuuint64_t)ld * sizeof(float)};
-  const cuuint32_t box[2] = {(cuuint32_t)kAtomK, (cuuint32_t)box_rows};
+  const cuuint64_t gstride[1] = {(cuuint64_t)ld_bytes};
+  const cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
   const cuuint32_t estr[2] = {1u, 1u};
-  const CUresult r = encode(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)base, gdim, gstride, box, estr,
+  const CUresult r = encode(out, dtype, 2, (void*)base, gdim, gstride, box, estr,
                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(ADMMQ_E_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
   return ADMMQ_OK;
+}
+
+int make_operand_tmap(CUtensorMap* out, const float* base, int rows, int cols, int ld, int box_rows) {
+  return make_tmap_2d(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, base, rows, cols, (size_t)ld * sizeof(float), kAtomK, box_rows);
 }
 }  // namespace tc
 
@@ -201,13 +206,6 @@ __global__ void __launch_bounds__(256) k_fold_partials(const double* __restrict_
 }
 
 // ---------------------------------------------------------------------------- launch choices
-// Tile widths come from a wave model: a tile costs a fixed part plus bn columns of tensor-core work, and the width
-// minimises waves * (fixed + bn); ties go to the wider tile (the candidates are tried widest first).
-static long long wave_cost(long long tilesM, int N, int w, int sms, int fixed) {
-  const long long tiles = tilesM * ((N + w - 1) / w);
-  return ((tiles + sms - 1) / sms) * (fixed + w);
-}
-
 // gemm_nt: measured 3.3 + 0.225 bn us at K = 1141, i.e. a fixed part of 16 columns; 128-wide tiles need the pre-split
 // B operand
 static int gemm_tile_width(int M, int N, int sms, bool presplit) {
@@ -216,7 +214,7 @@ static int gemm_tile_width(int M, int N, int sms, bool presplit) {
   long long best = -1;
   for (const int w : {128, 64, 32, 16}) {
     if (w == 128 && !presplit) continue;
-    const long long cost = wave_cost(tilesM, N, w, sms, 16);
+    const long long cost = tc::wave_cost(tilesM, N, w, sms, 16);
     if (best < 0 || cost < best) {
       best = cost;
       bn = w;
@@ -261,7 +259,7 @@ int select_mttkrp_kernel(int M, int nx, int ny, int R, int precision, int sms, i
     int bn = 128;
     long long best = -1;
     for (int w = 128; w >= (longf ? 80 : 16); w -= 16) {
-      const long long cost = wave_cost(tilesM, R, w, sms, 40);
+      const long long cost = tc::wave_cost(tilesM, R, w, sms, 40);
       if (best < 0 || cost < best) {
         best = cost;
         bn = w;

@@ -618,9 +618,20 @@ __device__ __forceinline__ const float* acc_to_smem(const Pipe& pipe, unsigned c
   return tile;
 }
 
-// Host: TMA descriptor of a row-major float32 matrix (rows x cols, leading dimension ld floats, ld % 4 == 0, base
-// 16-byte aligned) with box {32 columns, box_rows rows} and 128-byte swizzle.  Returns 0 or ADMMQ_E_CUDA.
+// Host: TMA descriptor of a row-major matrix of `dtype` elements (rows x cols, leading dimension ld_bytes, a multiple
+// of 16, base 16-byte aligned) with box {box_cols columns, box_rows rows} and 128-byte swizzle; rows and columns outside
+// the matrix read as zero.  Returns 0 or ADMMQ_E_CUDA.
+int make_tmap_2d(CUtensorMap* out, CUtensorMapDataType dtype, const void* base, int rows, int cols, size_t ld_bytes,
+                 int box_cols, int box_rows);
+// ... of a float32 matrix (ld floats, ld % 4 == 0) with box {32 columns, box_rows rows}
 int make_operand_tmap(CUtensorMap* out, const float* base, int rows, int cols, int ld, int box_rows);
+
+// Host: tile widths come from a wave model.  A tile costs a fixed part plus w columns of tensor-core work, and the width
+// minimises waves * (fixed + w); callers try the candidates widest first, so ties go to the wider tile.
+inline long long wave_cost(long long tilesM, int N, int w, int sms, int fixed) {
+  const long long tiles = tilesM * ((N + w - 1) / w);
+  return ((tiles + sms - 1) / sms) * (fixed + w);
+}
 
 }  // namespace tc
 }  // namespace admmq

@@ -5,7 +5,11 @@ pretrained checkpoints exist offline: the model is torchvision's architecture wi
 own predictions.
 
     python admm-quantization_b200/scripts/calibrate.py --model-name resnet18 --method admm --init random \
-        --reduction-rate 2 --bits 4 --qscheme tensor_mseminmax_symmetric --seed 42 [--layers layer1.0.conv1 ...]
+        --reduction-rate 2 --bits 4 --qscheme tensor_mseminmax_symmetric --seed 42 [--layers layer1.0.conv1 ...] \
+        [--execute fp8]
+
+`--execute fp32` (default) builds float32 CP layers from the factor values; `--execute fp8` re-projects every factor
+onto the `--bits/--qscheme` grid and runs the CP layers on the FP8 tensor cores from the codes (replace_with_cp_fp8).
 
 Factor files are read from `{bits}bit_{qscheme}/factors_{method}_seed{seed}/{layer}_{method}_{init}_rank_{rank}_mode_{m}.pt`
 (the naming of scripts/factorize.py:164-166, 345-347).
@@ -20,7 +24,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 
-from source.models import get_submodule, replace_with_cp  # noqa: E402
+from source.models import get_submodule, replace_with_cp, replace_with_cp_fp8  # noqa: E402
 from source.solver import layer_weight_as_tensor, rank_from_reduction_rate  # noqa: E402
 from source.utils import SyntheticImages, bncalibrate_model, top1_accuracy  # noqa: E402
 from source.workloads import resnet18_conv_layers  # noqa: E402
@@ -41,6 +45,8 @@ def parse_args(argv=None):
     ap.add_argument("--eval-batches", type=int, default=16)
     ap.add_argument("--batch-size", type=int, default=64)
     ap.add_argument("--image-size", type=int, default=64)
+    ap.add_argument("--execute", choices=("fp32", "fp8"), default="fp32",
+                    help="fp8: run the CP layers on the FP8 tensor cores from the factor codes")
     return ap.parse_args(argv)
 
 
@@ -65,7 +71,10 @@ def main(argv=None):
         prefix = os.path.join(fdir, f"{path}_{args.method}_{args.init}_rank_{rank}_")
         factors = [torch.load(prefix + f"mode_{m}.pt") for m in range(w.ndim)]
         assert all(f.dtype == torch.float32 for f in factors)
-        replace_with_cp(model, path, factors, rank)
+        if args.execute == "fp8":
+            replace_with_cp_fp8(model, path, factors, args.bits, args.qscheme)
+        else:
+            replace_with_cp(model, path, factors, rank)
     calib = SyntheticImages(args.calibration_samples // args.batch_size + 2, args.batch_size, args.image_size, seed=1, device=device)
     bncalibrate_model(model, calib, num_samples=args.calibration_samples, device=device)
     evalset = SyntheticImages(args.eval_batches, args.batch_size, args.image_size, seed=2, device=device, labels_from=teacher)

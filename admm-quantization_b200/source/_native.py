@@ -82,6 +82,11 @@ def _load():
         "admmq_recon_error_workspace_bytes": (c_sz, [c_int, c_int, c_int]),
         "admmq_recon_error": (c_int, [vp, c_int, vp, vp, c_int, vp, c_int, c_int, vp, vp, c_sz, vp]),
         "admmq_gemm_nt": (c_int, [vp, c_int, c_int, vp, c_int, c_int, c_int, vp, c_int, vp]),
+        "admmq_fp8_operand_format": (c_int, [c_int, c_int]),
+        "admmq_codes_to_fp8": (c_int, [vp, c_int, c_int, c_int, c_int, c_int, vp, c_int, vp]),
+        "admmq_fp8_quantize_rows": (c_int, [vp, c_int, c_int, c_int, vp, c_int, vp, vp]),
+        "admmq_code_gemm_kernel": (c_int, [c_int, c_int, c_int, c_int, ctypes.POINTER(c_int)]),
+        "admmq_code_gemm": (c_int, [vp, c_int, vp, c_int, vp, c_int, vp, c_int, c_int, c_int, vp, vp, c_int, vp]),
         "admmq_padded_ld": (c_int, [c_int]),
         "admmq_spd_inverse_workspace_bytes": (c_sz, [c_int]),
         "admmq_spd_inverse": (c_int, [vp, c_int, vp, vp, vp, vp, c_int, vp, c_sz, vp]),
@@ -118,7 +123,8 @@ EXPORTS = ("admmq_version admmq_last_error admmq_device_info admmq_launch_count 
            "admmq_recon_error_workspace_bytes admmq_recon_error admmq_padded_ld admmq_spd_inverse_workspace_bytes "
            "admmq_spd_inverse admmq_admm_iteration_workspace_bytes admmq_admm_iteration "
            "admmq_factorize_workspace_bytes admmq_factorize_cp3 admmq_factorize_mat admmq_factorize_batch "
-           "admmq_split_loop_workspace_bytes admmq_split_loop").split()
+           "admmq_split_loop_workspace_bytes admmq_split_loop "
+           "admmq_fp8_operand_format admmq_codes_to_fp8 admmq_fp8_quantize_rows admmq_code_gemm_kernel admmq_code_gemm").split()
 
 
 def last_error() -> str:
@@ -424,6 +430,75 @@ def gemm_nt(A, B, out=None):
     C = torch.empty(M, N, dtype=torch.float32, device=A.device) if out is None else out
     call(A.device, lib.admmq_gemm_nt, ptr(A), A.stride(0), M, ptr(B), B.stride(0), N, K, ptr(C), C.stride(0), stream_ptr(A.device))
     return C
+
+
+# ---- CP layers on the FP8 tensor cores (include/admmq.h, DESIGN.md 2d)
+FP8_DTYPES = {"tensor_mseminmax_e4m3": torch.float8_e4m3fn, "tensor_mseminmax_e5m2": torch.float8_e5m2}
+
+
+def ld16(n):
+    """Row stride (elements) of an FP8 operand with n columns: n rounded up to 16 bytes."""
+    return (int(n) + 15) // 16 * 16
+
+
+def fp8_operand_format(bits, qscheme):
+    """The FP8 format the codes of (bits, qscheme) run as: "tensor_mseminmax_e4m3" or "tensor_mseminmax_e5m2" (the scheme
+    whose torch dtype FP8_DTYPES gives).  ValueError, with the reason, for a grid without an exact FP8 form."""
+    rc = int(lib.admmq_fp8_operand_format(int(bits), qscheme_id(qscheme)))
+    check(min(rc, 0))
+    return "tensor_mseminmax_e5m2" if rc == QSCHEME_IDS["tensor_mseminmax_e5m2"] else "tensor_mseminmax_e4m3"
+
+
+def codes_to_fp8(codes, bits, qscheme, transpose=False):
+    """FP8 operand bytes (uint8) of a 2-D int8 code tensor: (rows, ld16(cols)), or with transpose=True
+    (cols, ld16(rows)) holding codes.T; pad columns zero.  View the result as FP8_DTYPES[fp8_operand_format(...)]."""
+    fp8_operand_format(bits, qscheme)
+    require_cuda(codes)
+    assert codes.dtype == torch.int8 and codes.dim() == 2
+    c = codes.contiguous()
+    rows, cols = c.shape
+    out_rows, out_cols = (cols, rows) if transpose else (rows, cols)
+    out = torch.empty(out_rows, ld16(out_cols), dtype=torch.uint8, device=c.device)
+    call(c.device, lib.admmq_codes_to_fp8, ptr(c), rows, cols, int(bits), qscheme_id(qscheme), 1 if transpose else 0,
+         ptr(out), out.shape[1], stream_ptr(c.device))
+    return out
+
+
+def fp8_quantize_rows(x, out=None, scale=None):
+    """Per-row dynamic E4M3 codes of a 2-D float32 tensor x (M, K) with unit column stride: (q uint8 (M, ld16(K)) with
+    zero pad columns, s float32 (M,)), s_m = fl(amax_m / 448), q = E4M3(fl(x / s_m))."""
+    require_cuda(x, out, scale)
+    assert x.dtype == torch.float32 and x.dim() == 2 and x.stride(1) == 1
+    M, K = x.shape
+    q = torch.empty(M, ld16(K), dtype=torch.uint8, device=x.device) if out is None else out
+    s = torch.empty(M, dtype=torch.float32, device=x.device) if scale is None else scale
+    call(x.device, lib.admmq_fp8_quantize_rows, ptr(x), x.stride(0), M, K, ptr(q), q.stride(0), ptr(s), stream_ptr(x.device))
+    return q, s
+
+
+def code_gemm(a8, a_scale, b8, b_scale, K, b_format="tensor_mseminmax_e4m3", bias=None, out=None):
+    """D (M, N) float32 = fl(acc * fl(a_scale[m] * b_scale[0])) (+ bias[n]) with acc = a8[:, :K] . b8[:, :K]^T summed on
+    the FP8 tensor cores: a8 (M, lda) E4M3 bytes, b8 (N, ldb) bytes of b_format, both uint8 with unit column stride;
+    a_scale (M,), b_scale (>= 1,) and bias (N,) float32 on the device."""
+    require_cuda(a8, a_scale, b8, b_scale, bias, out)
+    assert a8.dtype == torch.uint8 and b8.dtype == torch.uint8 and a8.stride(1) == 1 and b8.stride(1) == 1
+    for t in (a_scale, b_scale, bias):
+        assert t is None or (t.dtype == torch.float32 and t.is_contiguous())
+    M, N = a8.shape[0], b8.shape[0]
+    assert a_scale.numel() >= M and (bias is None or bias.numel() >= N)
+    D = torch.empty(M, N, dtype=torch.float32, device=a8.device) if out is None else out
+    assert D.dtype == torch.float32 and D.stride(1) == 1 and D.shape[0] >= M and D.shape[1] >= N
+    call(a8.device, lib.admmq_code_gemm, ptr(a8), a8.stride(0), ptr(a_scale), M, ptr(b8), b8.stride(0), ptr(b_scale),
+         qscheme_id(b_format), N, int(K), ptr(bias), ptr(D), D.stride(0), stream_ptr(a8.device))
+    return D
+
+
+def code_gemm_kernel(M, N, K, sm_count):
+    """(tile width, grid) a code_gemm of this shape runs on `sm_count` SMs."""
+    grid = ctypes.c_int(0)
+    rc = int(lib.admmq_code_gemm_kernel(int(M), int(N), int(K), int(sm_count), ctypes.byref(grid)))
+    check(min(rc, 0))
+    return rc, grid.value
 
 
 def spd_inverse_workspace_bytes(R):

@@ -183,6 +183,42 @@ ADMMQ_API int admmq_normalize_columns_f64(double* U, int n, int R, double* norms
 ADMMQ_API int admmq_gemm_nt(const float* A, int lda, int M, const float* B, int ldb, int N, int K, float* C, int ldc,
                   void* stream);
 
+/* ------------------------------------------------------------------ CP layers on the FP8 tensor cores (DESIGN.md 2d)
+ * A factor's codes (quantize_tensor_codes) run as FP8 tensor-core operands; every mapping is exact: the byte's value is
+ * the grid level, the factor's per-tensor scale s_w = info[0] stays on the device.
+ *   tensor_mseminmax_e4m3 / _e5m2 (bits 8)           E4M3 / E5M2, the byte as is
+ *   tensor_mseminmax_e2m1 (4), _e3m2 / _e2m3 (6)      E4M3 byte of the level (subnormals included), -0 -> 0x80
+ *   tensor_mseminmax_symmetric, tensor_symmetric      E4M3 byte of the integer code c in [-16, 15] (bits 1 .. 5)
+ * Anything else is ADMMQ_E_BADARG: integer grids of 6 bits or more (17 is not an E4M3 value) and tensor_affine /
+ * tensor_minmax (their levels are offset by a zero point / minimum).
+ *
+ * admmq_fp8_operand_format   pure host logic: the operand format of the codes of (bits, qscheme), ADMMQ_Q_MSEMINMAX_E4M3
+ *                            or ADMMQ_Q_MSEMINMAX_E5M2, or ADMMQ_E_BADARG with the reason.
+ * admmq_codes_to_fp8         codes (rows x cols int8, contiguous) -> out (uint8): transpose 0: rows x ldo, out[r, c] =
+ *                            byte(codes[r, c]); transpose 1: cols x ldo, out[c, r] = byte(codes[r, c]).  ldo a multiple
+ *                            of 16 and >= the output's columns; pad columns are zero.
+ * admmq_fp8_quantize_rows    per-row dynamic E4M3 activations of x (M x K, ld ldx): s_m = fl(amax_m / 448),
+ *                            q = cvt.rn.satfinite.e4m3x2.f32(fl(x / s_m)), M x ldq bytes (ldq a multiple of 16, >= K, q
+ *                            16-byte aligned), pad columns [K, ldq) zero; scale (M floats) = s_m.  amax_m == 0 or an s_m
+ *                            that underflows gives codes 0 and s_m = 0; a NaN or infinite amax_m gives s_m = NaN.
+ * admmq_code_gemm            D (M x N float32, ldd >= N) = fl(acc * fl(a_scale[m] * b_scale[0])) (+ bias[n] if bias is
+ *                            not NULL), acc[m, n] = sum_k A8[m, k] B8[n, k] as the tensor core's float32 sum over K in
+ *                            a fixed order (tcgen05.mma kind::f8f6f4, no split-K: the result does not depend on the grid
+ *                            or the tile width).  A8 (M x K, lda) E4M3, B8 (N x K, ldb) of b_format (ADMMQ_Q_MSEMINMAX_E4M3
+ *                            or _E5M2); lda, ldb multiples of 16 and >= K, A8 / B8 16-byte aligned.  Stores outside
+ *                            rows < M, columns < N never happen.
+ * admmq_code_gemm_kernel     pure host logic: the tile width (a multiple of 16 up to 256) a code GEMM of this shape runs
+ *                            on sm_count SMs, and its grid; honours ADMMQ_CODE_GEMM_BN (a forced width, read per call).
+ * Shapes with M * lda, N * ldb, M * ldd, M * ldx or rows * ldo >= 2^31 are ADMMQ_E_UNSUPPORTED; K <= 0 is ADMMQ_E_BADARG. */
+ADMMQ_API int admmq_fp8_operand_format(int bits, int qscheme);
+ADMMQ_API int admmq_codes_to_fp8(const int8_t* codes, int rows, int cols, int bits, int qscheme, int transpose,
+                  uint8_t* out, int ldo, void* stream);
+ADMMQ_API int admmq_fp8_quantize_rows(const float* x, int ldx, int M, int K, uint8_t* q, int ldq, float* scale,
+                  void* stream);
+ADMMQ_API int admmq_code_gemm_kernel(int M, int N, int K, int sm_count, int* grid);
+ADMMQ_API int admmq_code_gemm(const uint8_t* A8, int lda, const float* a_scale, int M, const uint8_t* B8, int ldb,
+                  const float* b_scale, int b_format, int N, int K, const float* bias, float* D, int ldd, void* stream);
+
 /* ------------------------------------------------------------------ ridge system
  * rho = trace(G)/R and Minv = (G + rho I)^-1  (replaces torch.linalg.cholesky at source/admm.py:52-54;
  * the per-iteration cholesky_solve of :56 becomes a product with Minv).  Blocked float64 Cholesky +
